@@ -24,6 +24,8 @@ rank.  pair-sites are counted nominally: pairs x n_eff x replicates.
           triangle tiles dealt to the ranks, and site shards with one NCCL reduce -- each with its collective's bytes and ms.
   --impl reference : the UNMODIFIED reference (oracle/_ref/ngsDist, built from /root/reference with the gsl_rng_taus
           shim) on the host cores, same flags, bounded sample of the C3 data set per step.
+  --dump-outputs DIR : after the timed steps, DIR/dist.npy holds the distance matrices of the last timed step (see
+          dump_outputs); inputs and bootstrap draws are seeded, so two builds run with the same arguments can be compared.
 """
 import argparse
 import json
@@ -50,10 +52,27 @@ UNIT = "pair-sites/s"
 WORKLOAD = ("C3: synthetic GL 2000 ind x 1M sites, 10% missing, --probs --indep_geno --pairwise_del, bootstrap block 1000 seed 12345, "
             "weighted contraction per replicate")
 REF_FLAGS = ["--probs", "--indep_geno", "--pairwise_del", "--boot_block_size", str(BLOCK), "--seed", str(BOOT_SEED)]
+DUMP_BYTES = 48 << 20       # --dump-outputs stays under 64 MB
+DUMP_SEED = 7
 
 
 def pairs(n):
     return n * (n - 1) // 2
+
+
+def dump_outputs(path, mats):
+    """Write mats [replicate][n_ind][n_ind] (float64, the matrices a caller of ngsd_distances_batch receives) to
+    path/dist.npy: whole when they fit DUMP_BYTES, otherwise as [replicate][k], the same k entries of every matrix,
+    drawn once with DUMP_SEED and kept in row-major order (the same entries on every run of the same shape)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    R, n, _ = mats.shape
+    flat = mats.reshape(R, n * n)
+    if flat.nbytes > DUMP_BYTES:
+        k = DUMP_BYTES // (8 * R)
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n * n, size=k, replace=False))
+        flat = flat[:, idx]
+    np.save(os.path.join(path, "dist.npy"), np.ascontiguousarray(flat, dtype=np.float64))
 
 
 class ClockSampler:
@@ -182,6 +201,7 @@ def main():
     ap.add_argument("--n-ind", type=int, default=N_IND)
     ap.add_argument("--n-sites", type=int, default=N_SITES)
     ap.add_argument("--reps", type=int, default=REPS_PER_STEP)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the distance matrices of the last timed step to DIR/dist.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -286,6 +306,8 @@ def main():
         sampler.start()
     ms_total = timed(step_resident, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out_pin.numpy())          # before the e2e steps below reuse out_pin
     n_launch = launches[0]
     res = dict(acc)
     tim = g.timing()

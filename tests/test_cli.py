@@ -1,7 +1,8 @@
 """The drop-in command line (ngsdist_b200/bin/ngsDist): same flags, inputs and .dist layout as the reference.
 
 CPU part: argument validation reproduces parse_args.cpp:203-220 (message + exit status 255) before any CUDA call.
-GPU part: every golden case is run through the binary and compared with the reference's own .dist text.
+GPU part: every golden case is run through the binary and compared with the reference's own .dist text; inputs made up
+inside a test are compared with the .dist text the reference writes for them, as the CPU oracle restates it.
 """
 import gzip
 import os
@@ -11,7 +12,7 @@ import numpy as np
 import pytest
 
 import oracle
-from util import GOLDEN, golden_text, manifest
+from util import GOLDEN, format_dist, golden_text, manifest, parse_flags
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CLI = os.path.join(ROOT, "ngsdist_b200", "bin", "ngsDist")
@@ -20,6 +21,14 @@ MAN = manifest()
 
 def run_cli(args, **kw):
     return subprocess.run([CLI] + args, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, **kw)
+
+
+def reference_text(data, flags, labels=None, **kw):
+    """The reference's .dist text for `data` run with the compute `flags`: the CPU oracle through the reference's writer,
+    which reproduces every .dist in tests/golden/ (written by the unmodified reference) byte for byte
+    (tests/test_oracle_golden.py).  kw: kind=1 for text input, genotypes=True for {-1,0,1,2} codes."""
+    okw, _ = parse_flags(flags)
+    return format_dist([r["dist"] for r in oracle.run_job(data, **okw, **kw)], labels)
 
 
 def test_cli_is_built():
@@ -133,13 +142,11 @@ def test_cli_labels_stdin_and_nan_spelling(tmp_path):
     flags = ["--probs", "--indep_geno", "--pairwise_del", "--evol_model", "0"]
     r = run_cli(["--geno", str(geno), "--n_ind", "5", "--n_sites", "64", "--labelsH", str(labels), "--out", str(out), "--verbose", "0"] + flags)
     assert r.returncode == 0, r.stderr
-    ref, ref_text = oracle.run_reference(None, flags + ["--labelsH", str(labels)], geno_path=str(geno), n_ind=n_ind, n_sites=n_sites) \
-        if oracle.have_ref() else (None, None)
+    ref_text = reference_text(raw, flags, labels=list("ABCDE"))
     text = out.read_text()
     assert text.split("\n")[2].startswith("A\t0.0000000000\t-nan\t")
-    if ref_text is not None:
-        assert [l.split("\t")[0] for l in text.split("\n")] == [l.split("\t")[0] for l in ref_text.split("\n")]
-        assert text.count("nan") == ref_text.count("nan") and text.count("-nan") == ref_text.count("-nan")
+    assert [l.split("\t")[0] for l in text.split("\n")] == [l.split("\t")[0] for l in ref_text.split("\n")]
+    assert text.count("nan") == ref_text.count("nan") and text.count("-nan") == ref_text.count("-nan")
     # binary from stdin ("-")
     out2 = tmp_path / "o2.dist"
     with open(geno, "rb") as fh:
@@ -154,19 +161,19 @@ def test_cli_c1_reference_test_script_matrix(tmp_path):
     """BASELINE configs[0] (C1): the 18 runs of the reference's own examples/test.sh (genotype text, BEAGLE-style text with
     header + 3 leading columns + --pos, binary, plain text posteriors; bootstrap, block size, --call_geno, thresholds) at
     its shape, 24 individuals x 10 000 sites with --labels, on synthetic data (the script's inputs are not shipped, SURVEY
-    D4).  Every run is executed by the drop-in CLI and by the unmodified reference binary and the .dist files are compared:
+    D4).  Every run is executed by the drop-in CLI and its .dist file is compared with the reference's (reference_text):
     same layout and labels, values within 1e-9 (default --probs rows run the per pair-site EM in both)."""
     import gzip
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref/ngsDist not built")
     n_ind, n_sites = 24, 10000
     raw = oracle.synth_raw(20251018, 0.05, n_ind, n_sites)
     P = raw / raw.sum(axis=2, keepdims=True)
     # keep 6-decimal text values off the --call_thresh 0.9 knife edge (a 1-ulp log/exp difference could flip a call there,
     # SURVEY App. E-7): no triple whose printed maximum is exactly 0.900000
     P[np.round(P, 6).max(axis=2) == 0.9] = (0.91, 0.05, 0.04)
+    P6 = np.array(["%.6f" % v for v in P.reshape(-1)]).astype(np.float64).reshape(P.shape)    # the values the text files hold
+    label_names = ["ind%02d_pop%d" % (i, i // 8) for i in range(n_ind)]
     labels = str(tmp_path / "testA.labels")
-    open(labels, "w").write("".join("ind%02d_pop%d\n" % (i, i // 8) for i in range(n_ind)))
+    open(labels, "w").write("".join(l + "\n" for l in label_names))
     # genotype text: chr, position, then one code per individual (-1 = missing where the synthetic triple is uniform)
     geno = np.argmax(raw, axis=2).astype(int)
     geno[(raw[..., 0] == raw[..., 1]) & (raw[..., 1] == raw[..., 2])] = -1
@@ -190,22 +197,22 @@ def test_cli_c1_reference_test_script_matrix(tmp_path):
     boot = [[], ["--n_boot_rep", "5"], ["--n_boot_rep", "5", "--boot_block_size", "10"]]
     call = [["--n_boot_rep", "5", "--boot_block_size", "10", "--call_geno"],
             ["--n_boot_rep", "5", "--boot_block_size", "10", "--call_geno", "--N_thresh", "0.3", "--call_thresh", "0.9"]]
-    runs = [("T%d" % k, f_geno, b) for k, b in enumerate(boot)]
-    runs += [("2_%d" % k, f_beagle, ["--probs", "--pos", f_pos] + b) for k, b in enumerate(boot + call)]
-    runs += [("32_%d" % k, f_bin, ["--probs"] + b) for k, b in enumerate(boot + call)]
-    runs += [("8_%d" % k, f_txt, ["--probs"] + b) for k, b in enumerate(boot + call)]
+    # name, file, CLI flags, the file's values and how the reference reads them
+    runs = [("T%d" % k, f_geno, b, geno, dict(genotypes=True)) for k, b in enumerate(boot)]
+    runs += [("2_%d" % k, f_beagle, ["--probs", "--pos", f_pos] + b, P6, dict(kind=1)) for k, b in enumerate(boot + call)]
+    runs += [("32_%d" % k, f_bin, ["--probs"] + b, P, dict(kind=0)) for k, b in enumerate(boot + call)]
+    runs += [("8_%d" % k, f_txt, ["--probs"] + b, P6, dict(kind=1)) for k, b in enumerate(boot + call)]
     assert len(runs) == 18
     threads = str(os.cpu_count() or 4)
     worst = 0.0
-    for name, path, extra in runs:
-        outs = []
-        for binary in (CLI, oracle.REF_BIN):
-            out = str(tmp_path / ("%s_%s.dist" % (name, "ref" if binary == oracle.REF_BIN else "b200")))
-            cmd = [binary, "--n_threads", threads, "--seed", "12345", "--verbose", "0", "--geno", path, "--n_ind", str(n_ind),
-                   "--n_sites", str(n_sites), "--labels", labels] + extra + ["--out", out]
-            r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True)
-            assert r.returncode == 0, (name, r.stderr[-1500:])
-            outs.append(out)
+    for name, path, extra, data, read in runs:
+        outs = [str(tmp_path / ("%s_b200.dist" % name)), str(tmp_path / ("%s_ref.dist" % name))]
+        cmd = [CLI, "--n_threads", threads, "--seed", "12345", "--verbose", "0", "--geno", path, "--n_ind", str(n_ind),
+               "--n_sites", str(n_sites), "--labels", labels] + extra + ["--out", outs[0]]
+        r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True)
+        assert r.returncode == 0, (name, r.stderr[-1500:])
+        compute = [f for f in extra if f not in ("--pos", f_pos)] + ["--seed", "12345"]
+        open(outs[1], "w").write(reference_text(data, compute, labels=label_names, **read))
         ta, tb = open(outs[0]).read(), open(outs[1]).read()
         la, lb = ta.split("\n"), tb.split("\n")
         assert len(la) == len(lb), name
@@ -247,9 +254,7 @@ def test_cli_plink_bed_input_matches_genotype_text(tmp_path):
         assert r.returncode == 0, r.stderr
         texts.append(open(out).read())
     assert texts[0] == texts[1] == texts[2]
-    if oracle.have_ref():
-        _, ref_text = oracle.run_reference(None, flags[6:], geno_path=txt, n_ind=n_ind, n_sites=n_sites)
-        assert texts[0] == ref_text
+    assert texts[0] == reference_text(geno, flags[6:], genotypes=True)
     # a truncated file and sample-major files are refused
     bad = str(tmp_path / "bad.bed")
     with open(bad, "wb") as fh:
@@ -274,6 +279,7 @@ def test_cli_vcf_likelihoods_are_the_log_scale_text_input(fmt, flags, tmp_path):
     rng = np.random.RandomState(1)
     vcf = tmp_path / "in.vcf.gz"
     txt = tmp_path / "in.txt.gz"
+    lik = []
     with gzip.open(vcf, "wt") as fv, gzip.open(txt, "wt") as ft:
         fv.write("##fileformat=VCFv4.2\n##FORMAT=<ID=GT,Number=1,Type=String,Description=\"g\">\n")
         fv.write("#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\t" + "\t".join("S%d" % i for i in range(n_ind)) + "\n")
@@ -294,6 +300,7 @@ def test_cli_vcf_likelihoods_are_the_log_scale_text_input(fmt, flags, tmp_path):
                 vals += [repr(v) for v in L]
             fv.write("chr1\t%d\t.\tA\tC\t.\tPASS\t.\tGT:%s:DP\t" % (s + 1, fmt) + "\t".join(cols) + "\n")
             ft.write("\t".join(vals) + "\n")
+            lik.append([float(v) for v in vals])
     outs = []
     for path, extra in ((vcf, []), (txt, ["--probs", "--log_scale"])):
         out = str(tmp_path / (os.path.basename(str(path)) + ".dist"))
@@ -302,10 +309,9 @@ def test_cli_vcf_likelihoods_are_the_log_scale_text_input(fmt, flags, tmp_path):
         assert r.returncode == 0, r.stderr[-2000:]
         outs.append(open(out).read())
     assert outs[0] == outs[1]
-    if oracle.have_ref():      # ... and that text file through the reference binary: the same bytes
-        _, ref_text = oracle.run_reference(None, ["--probs", "--log_scale", "--n_boot_rep", "2", "--boot_block_size", "7", "--seed", "12345"] + flags,
-                                           geno_path=str(txt), n_ind=n_ind, n_sites=n_sites)
-        assert outs[0] == ref_text
+    # ... and what the reference writes for that text file: the same bytes
+    assert outs[0] == reference_text(np.array(lik).reshape(n_sites, n_ind, 3),
+                                     ["--probs", "--log_scale", "--n_boot_rep", "2", "--boot_block_size", "7", "--seed", "12345"] + flags, kind=1)
 
 
 @pytest.mark.gpu
