@@ -112,7 +112,7 @@ typedef struct {
   int32_t dist_ctas;         /* grid size of the distance kernel                         */
   uint64_t dist_dmma;        /* warp-level DMMA.8x8x4 instructions the K2 launch issued  */
   uint64_t active_sites;     /* sites with non-zero weight in the call                   */
-  uint64_t dist_imma;        /* warp-level IMMA.16832 instructions of the K2c launch (called-genotype integer path) */
+  uint64_t dist_imma;        /* K2c work of the called-genotype integer path, in IMMA-equivalents of 4096 int8 MAC */
   int32_t block_cache;       /* bootstrap block cache: 0 not used, 1 built by this call, 2 reused (no contraction launched) */
   int32_t pad_;
 } ngsd_timing;

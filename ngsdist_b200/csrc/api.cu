@@ -26,13 +26,14 @@ cudaError_t dev_alloc(T **p, uint64_t count) {
   return cudaMalloc((void **) p, std::max<uint64_t>(count, 1) * sizeof(T));
 }
 
-int ensure_pinned(ngsd_ctx *ctx, uint64_t bytes) {
-  if (ctx->h_pin_bytes >= bytes) return NGSD_OK;
-  if (ctx->h_pin) cudaFreeHost(ctx->h_pin);
-  ctx->h_pin = nullptr;
-  ctx->h_pin_bytes = 0;
-  NGSD_CUDA(ctx, cudaHostAlloc(&ctx->h_pin, bytes, cudaHostAllocDefault));
-  ctx->h_pin_bytes = bytes;
+// grow-on-demand pinned scratch (ctx->h_pin or ctx->h_pin2)
+int ensure_pinned(ngsd_ctx *ctx, void **pin, uint64_t *pin_bytes, uint64_t bytes) {
+  if (*pin_bytes >= bytes) return NGSD_OK;
+  if (*pin) cudaFreeHost(*pin);
+  *pin = nullptr;
+  *pin_bytes = 0;
+  NGSD_CUDA(ctx, cudaHostAlloc(pin, bytes, cudaHostAllocDefault));
+  *pin_bytes = bytes;
   return NGSD_OK;
 }
 
@@ -63,9 +64,7 @@ std::vector<uint32_t> plan_splits(uint32_t n_chunks, uint32_t n_tiles, double co
     for (uint32_t k = 1; k <= s; k++) b.push_back((uint32_t) ((uint64_t) k * n_chunks / s));
     return b;
   }
-  // tuning knobs (development only): NGSD_TUNE="main_units_per_cta,tail_ratio,main_fraction"
-  double upc = 8.0, ratio = 4.0, frac = 0.84;
-  if (const char *t = getenv("NGSD_TUNE")) sscanf(t, "%lf,%lf,%lf", &upc, &ratio, &frac);
+  const double upc = 8.0, ratio = 4.0, frac = 0.84;   // main units per CTA, main / tail unit size, main fraction
   const uint32_t Lm = (uint32_t) (frac * n_chunks);
   uint64_t Sm = (uint64_t) llround(upc * grid / cost_tiles);
   Sm = std::max<uint64_t>(1, std::min<uint64_t>(Sm, Lm / 16));
@@ -100,6 +99,16 @@ cudaError_t dbg_sync(ngsd_ctx *ctx, const char *what) {
   if (e != cudaSuccess) fprintf(stderr, "NGSD_SYNC: %s failed: %s\n", what, cudaGetErrorString(e));
   (void) ctx;
   return e;
+}
+
+// Copy the matrices of the last ngsd_distances to the caller's buffers (each may be null) and wait for them.
+int copy_out(ngsd_ctx *ctx, double *out, double *num_opt, uint64_t *cnt_opt) {
+  const uint64_t n2 = ctx->n_ind * ctx->n_ind;
+  if (out) NGSD_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_out, n2 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  if (num_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(num_opt, ctx->d_num, n2 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  if (cnt_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(cnt_opt, ctx->d_cntout, n2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+  NGSD_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return NGSD_OK;
 }
 
 cudaError_t upload_tile_index(ngsd_ctx *ctx, const std::vector<ngsd_tile> &tiles) {
@@ -231,10 +240,10 @@ int ngsd_create(const ngsd_cfg *cfg, ngsd_ctx **out) {
   ctx->NC = ctx->planes == 3 ? ctx->NW * 8 : (ctx->NW * 16 + 2) / 3;
   ctx->pushed.assign(ctx->NW, 0);
   // Called genotypes (every triple one-hot or "missing"): exact integer contraction on the int8 tensor cores, 2 bits per
-  // individual-site in HBM instead of FP64 planes (dist_imma.cu).  --call_geno leaves soft triples between the two
+  // individual-site in HBM instead of FP64 planes (dist_umma.cu).  --call_geno leaves soft triples between the two
   // thresholds (gen_func.cpp:908), so it qualifies only when they coincide (the default 0 / 0).
   const bool hard_calls = cfg->input_kind == NGSD_INPUT_GENOTYPES || (cfg->call_geno && cfg->N_thresh == cfg->call_thresh);
-  ctx->int_path = hard_calls && cfg->indep_geno && !(cfg->reserved & 2) && !getenv("NGSD_NO_INT") &&
+  ctx->int_path = hard_calls && cfg->indep_geno && !(cfg->reserved & 2) &&
                   ngsd_int_lut(cfg->score, cfg->pairwise_del != 0, ctx->int_lut, &ctx->int_scale, &ctx->int_max_byte);
   if (ctx->int_path) {
     ctx->planes = 3;
@@ -685,35 +694,6 @@ int ngsd_get_posteriors(ngsd_ctx *ctx, double *P_host, uint8_t *miss_host) {
 
 // ---------------------------------------------------------------------------------------------- distances ----
 
-// Entry list of K3 (mask_count.cu): (64-site word, level mask) pairs.  Integer weights are decomposed into level masks
-// W_v = {s : w_s >= v}, so cnt = sum_v popc(m_i & m_j & W_v) stays exact for any block size; replicate 0 is every word
-// with an all-ones mask.
-static uint64_t build_count_entries(const ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_blocks, uint64_t block_size,
-                                    uint32_t maxw, uint32_t *h_ew, uint64_t *h_em) {
-  uint64_t n_entries = 0;
-  if (!block_counts) {
-    for (uint64_t w = 0; w < ctx->NW; w++) { h_ew[w] = (uint32_t) w; h_em[w] = ~0ull; }
-    return ctx->NW;
-  }
-  std::vector<uint64_t> level(ctx->NW);
-  for (uint32_t v = 1; v <= maxw; v++) {
-    std::fill(level.begin(), level.end(), 0ull);
-    for (uint64_t b = 0; b < n_blocks; b++) {
-      if (block_counts[b] < v) continue;
-      uint64_t s0 = b * block_size, s1 = s0 + block_size;
-      while (s0 < s1) {   // set bits [s0, s1) word by word
-        const uint64_t w = s0 >> 6, lo = s0 & 63, hi = std::min<uint64_t>(64, lo + (s1 - s0));
-        const uint64_t m = (hi == 64 ? ~0ull : ((1ull << hi) - 1)) & ~((1ull << lo) - 1);
-        level[w] |= m;
-        s0 += hi - lo;
-      }
-    }
-    for (uint64_t w = 0; w < ctx->NW; w++)
-      if (level[w]) { h_ew[n_entries] = (uint32_t) w; h_em[n_entries] = level[w]; n_entries++; }
-  }
-  return n_entries;
-}
-
 static int ensure_dist_buffers(ngsd_ctx *ctx, uint64_t slots);
 static int ensure_entries(ngsd_ctx *ctx, uint64_t n);
 
@@ -760,20 +740,111 @@ static int upload_deficit(ngsd_ctx *ctx) {
   return NGSD_OK;
 }
 
-// One matrix on the called-genotype integer path (K2c dist_imma.cu): same contract as ngsd_distances.
+// The input of k_dist_umma (K2c, dist_umma.cu), for the integer path's sums and for the tensor-core count pass of the
+// FP64 path:
+//  * per-site weight bytes in layers of at most `cap` each: the bootstrap multiplicities (ngsDist.cpp:416-437), 1 for
+//    replicate 0 (block_counts == nullptr), 0 beyond the sites in use and, with zero_blanks, at sites that were empty
+//    text lines;
+//  * the list of 64-site words to contract as (word id, layer | bit 31 when all 64 weights of the word are 1): every
+//    word with a non-zero weight or, with cache_words > 0, the first cache_words words in order (the K splits of the
+//    bootstrap block cache are the words of one block each).
+// Both are staged in the pinned scratch *pin, the device buffers d_wsite, d_word_ids and d_word_layer grow on demand and
+// the copies are queued on ctx->stream.  *n_words = length of the list.
+static int build_word_list(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_blocks, uint64_t block_size, uint32_t maxw,
+                           uint32_t cap, bool zero_blanks, uint64_t cache_words, void **pin, uint64_t *pin_bytes, uint64_t *n_words) {
+  const uint64_t NW = ctx->NW, nsp = NW * 64;
+  const uint32_t layers = (maxw + cap - 1) / cap;
+  const uint64_t bytes_w = (uint64_t) layers * nsp, n_list = (uint64_t) layers * NW, bytes_w64 = (bytes_w + 63) / 64 * 64;
+  int rc = ensure_pinned(ctx, pin, pin_bytes, bytes_w64 + 2 * n_list * sizeof(uint32_t) + 64);
+  if (rc) return rc;
+  uint8_t *h_w = (uint8_t *) *pin;
+  uint32_t *h_ids = (uint32_t *) (h_w + bytes_w64), *h_layer = h_ids + n_list;
+  memset(h_w, 0, bytes_w);
+  if (!block_counts) {
+    memset(h_w, 1, ctx->n_sites);
+  } else {
+    for (uint64_t b = 0; b < n_blocks; b++) {
+      uint32_t left = block_counts[b];
+      for (uint32_t l = 0; l < layers && left; l++) {
+        const uint32_t w = std::min(left, cap);
+        memset(h_w + (uint64_t) l * nsp + b * block_size, (int) w, block_size);
+        left -= w;
+      }
+    }
+  }
+  if (zero_blanks)
+    for (uint64_t w = 0; w < NW; w++)
+      for (uint64_t m = ctx->h_blank[w]; m; m &= m - 1)
+        for (uint32_t l = 0; l < layers; l++) h_w[(uint64_t) l * nsp + w * 64 + (uint64_t) __builtin_ctzll(m)] = 0;
+  const uint64_t scan = cache_words ? cache_words : NW;
+  uint64_t n = 0;
+  for (uint32_t l = 0; l < layers; l++)
+    for (uint64_t w = 0; w < scan; w++) {
+      const uint64_t *p8 = (const uint64_t *) (h_w + (uint64_t) l * nsp + w * 64);
+      if (cache_words || (p8[0] | p8[1] | p8[2] | p8[3] | p8[4] | p8[5] | p8[6] | p8[7])) {
+        const uint64_t one = 0x0101010101010101ull;
+        const bool unit = p8[0] == one && p8[1] == one && p8[2] == one && p8[3] == one && p8[4] == one && p8[5] == one && p8[6] == one && p8[7] == one;
+        h_ids[n] = (uint32_t) w;
+        h_layer[n] = l | (unit ? 0x80000000u : 0u);             // bit 31: the kernel may skip the weight bytes of this word
+        n++;
+      }
+    }
+  if (bytes_w > ctx->wsite_cap) {
+    cudaFree(ctx->d_wsite);
+    ctx->d_wsite = nullptr;
+    ctx->wsite_cap = 0;
+    NGSD_CUDA(ctx, dev_alloc(&ctx->d_wsite, bytes_w));
+    ctx->wsite_cap = bytes_w;
+  }
+  if (n_list > ctx->word_cap) {
+    cudaFree(ctx->d_word_ids);
+    cudaFree(ctx->d_word_layer);
+    ctx->d_word_ids = ctx->d_word_layer = nullptr;
+    ctx->word_cap = 0;
+    NGSD_CUDA(ctx, dev_alloc(&ctx->d_word_ids, n_list));
+    NGSD_CUDA(ctx, dev_alloc(&ctx->d_word_layer, n_list));
+    ctx->word_cap = n_list;
+  }
+  if (n) {
+    NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_wsite, h_w, bytes_w, cudaMemcpyHostToDevice, ctx->stream));
+    NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_word_ids, h_ids, n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_word_layer, h_layer, n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+  }
+  *n_words = n;
+  return NGSD_OK;
+}
+
+// Cut K splits (boundaries in the word list) so that none holds more than max_words words: the int32 accumulators of
+// k_dist_umma must not overflow.
+static void cap_splits(std::vector<uint32_t> &splits, uint32_t max_words) {
+  std::vector<uint32_t> cut(1, 0);
+  for (size_t k = 1; k < splits.size(); k++) {
+    while (splits[k] - cut.back() > max_words) cut.push_back(cut.back() + max_words);
+    if (splits[k] > cut.back()) cut.push_back(splits[k]);
+  }
+  if (cut.size() < 2) cut.push_back(0);
+  splits.swap(cut);
+}
+
+// One matrix on the called-genotype integer path (K2c dist_umma.cu): same contract as ngsd_distances.
 static int distances_int(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_blocks, uint64_t block_size, double *out,
                          double *num_opt, uint64_t *cnt_opt) {
   const bool weighted = block_counts != nullptr;
   const uint64_t n_eff = weighted ? n_blocks * block_size : ctx->n_sites;
-  const uint64_t NW = ctx->NW, nsp = NW * 64;
   uint32_t maxw = 1;
-  if (weighted)
-    for (uint64_t b = 0; b < n_blocks; b++) maxw = std::max(maxw, block_counts[b]);
+  uint64_t active_sites = n_eff;
+  if (weighted) {
+    active_sites = 0;
+    for (uint64_t b = 0; b < n_blocks; b++) {
+      maxw = std::max(maxw, block_counts[b]);
+      active_sites += block_counts[b] ? block_size : 0;
+    }
+  }
   const bool do_count = ctx->cfg.pairwise_del != 0;
   // ---- bootstrap block cache (see ngsd_distances): per-block int32 partials, blocks = whole 64-site words ----
   const uint64_t unit_ints = do_count ? 2 * NGSD_TILE_ELEMS : NGSD_TILE_ELEMS;
   bool use_cache = false, build_cache = false;
-  if (weighted && !(ctx->cfg.reserved & 4) && !getenv("NGSD_NO_BLOCK_CACHE") && block_size % 64 == 0 && n_blocks >= 2 &&
+  if (weighted && !(ctx->cfg.reserved & 4) && block_size % 64 == 0 && n_blocks >= 2 &&
       ctx->n_tiles > 0 && n_blocks < 0x7fffffffull / ctx->n_tiles &&
       (uint64_t) std::max(ctx->int_max_byte, 1) * block_size < 2147483647ull) {
     const uint64_t need = (n_blocks * (uint64_t) ctx->n_tiles * unit_ints + 1) / 2;   // in doubles
@@ -797,85 +868,31 @@ static int distances_int(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n
   }
   if (use_cache) maxw = 1;                                     // the contraction (if any) runs unweighted, K splits = blocks
   const uint32_t wcap = ngsd_int_weight_cap(ctx);              // site weights are int8 operand bytes: <= 127 (42) per layer
-  const uint32_t layers = (maxw + wcap - 1) / wcap;
-  const uint64_t ent_max = 0;   // the counts are a second int8 GEMM inside K2c: no K3 entry list
-  const uint64_t bytes_w = (uint64_t) layers * nsp, bytes_ids = (uint64_t) layers * NW * sizeof(uint32_t);
-  int rc = ensure_pinned(ctx, bytes_w + 2 * bytes_ids + ent_max * (sizeof(uint32_t) + sizeof(uint64_t)) + 256);
-  if (rc) return rc;
-  uint64_t *h_em = (uint64_t *) ctx->h_pin;
-  uint8_t *h_w = (uint8_t *) (h_em + ent_max);
-  uint32_t *h_ids = (uint32_t *) (h_w + ((bytes_w + 63) / 64) * 64);
-  uint32_t *h_layer = h_ids + (uint64_t) layers * NW;
-  uint32_t *h_ew = h_layer + (uint64_t) layers * NW;
-
-  // per-site weights (bootstrap multiplicities of ngsDist.cpp:416-437; 1 for replicate 0; 0 beyond the sites in use)
-  uint64_t active_sites = n_eff;
-  memset(h_w, 0, bytes_w);
-  if (!weighted || use_cache) {
-    memset(h_w, 1, ctx->n_sites);
-    if (weighted) {
-      active_sites = 0;
-      for (uint64_t b = 0; b < n_blocks; b++) active_sites += block_counts[b] ? block_size : 0;
-    }
-  } else {
-    active_sites = 0;
-    for (uint64_t b = 0; b < n_blocks; b++) {
-      uint32_t left = block_counts[b];
-      if (left) active_sites += block_size;
-      for (uint32_t l = 0; l < layers && left; l++) {
-        const uint32_t w = std::min<uint32_t>(left, wcap);
-        memset(h_w + (uint64_t) l * nsp + b * block_size, (int) w, block_size);
-        left -= w;
-      }
-    }
-  }
   // Sites that were empty text lines hold (0,0,0) in the reference (read_data.cpp:58-59): nothing to add for any pair,
   // but still counted without --pairwise_del.  A 2-bit code cannot say that, a site weight of 0 can.
   const bool blanks = ctx->any_blank && !ctx->cfg.pairwise_del;
-  if (blanks)
-    for (uint64_t w = 0; w < NW; w++)
-      for (uint64_t m = ctx->h_blank[w]; m; m &= m - 1)
-        for (uint32_t l = 0; l < layers; l++) h_w[(uint64_t) l * nsp + w * 64 + (uint64_t) __builtin_ctzll(m)] = 0;
-  uint64_t n_words = 0;
-  if (use_cache) {                                             // identity word list over the blocks in use
-    n_words = n_blocks * (block_size / 64);
-    for (uint64_t w = 0; w < n_words && build_cache; w++) {   // bit 31: all 64 weights are 1
-      h_ids[w] = (uint32_t) w;
-      h_layer[w] = (blanks && ctx->h_blank[w]) ? 0u : 0x80000000u;
-    }
-  }
-  for (uint32_t l = 0; l < layers && !use_cache; l++)
-    for (uint64_t w = 0; w < NW; w++) {
-      const uint64_t *p8 = (const uint64_t *) (h_w + (uint64_t) l * nsp + w * 64);
-      if (p8[0] | p8[1] | p8[2] | p8[3] | p8[4] | p8[5] | p8[6] | p8[7]) {
-        const uint64_t one = 0x0101010101010101ull;
-        const bool unit = p8[0] == one && p8[1] == one && p8[2] == one && p8[3] == one && p8[4] == one && p8[5] == one && p8[6] == one && p8[7] == one;
-        h_ids[n_words] = (uint32_t) w;
-        h_layer[n_words] = l | (unit ? 0x80000000u : 0u);      // bit 31: the kernels may skip the weight bytes of this word
-        n_words++;
-      }
-    }
-  (void) h_ew; (void) h_em;
-
-  const uint64_t n2 = ctx->n_ind * ctx->n_ind;
-  if (ctx->n_tiles == 0 || n_words == 0) {   // a tile shard that owns nothing (or no active site): all-zero sums
-    rc = ensure_dist_buffers(ctx, 1);
+  uint64_t n_words = use_cache ? n_blocks * (block_size / 64) : 0;
+  const bool contract = !use_cache || build_cache;            // (otherwise the cached partials of this geometry are resident)
+  if (contract) {
+    int rc = build_word_list(ctx, use_cache ? nullptr : block_counts, n_blocks, block_size, maxw, wcap, blanks, n_words, &ctx->h_pin,
+                             &ctx->h_pin_bytes, &n_words);
     if (rc) return rc;
+  }
+
+  if (ctx->n_tiles == 0 || n_words == 0) {   // a tile shard that owns nothing (or no active site): all-zero sums
+    int rc = ensure_dist_buffers(ctx, 1);
+    if (rc) return rc;
+    const uint64_t n2 = ctx->n_ind * ctx->n_ind;
     NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_out, 0, n2 * sizeof(double), ctx->stream));
     NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_num, 0, n2 * sizeof(double), ctx->stream));
     NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_cntout, 0, n2 * sizeof(uint64_t), ctx->stream));
     if (ctx->n_tiles == 0) {
-      if (out) NGSD_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_out, n2 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-      if (num_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(num_opt, ctx->d_num, n2 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-      if (cnt_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(cnt_opt, ctx->d_cntout, n2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
-      NGSD_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
       ctx->timing = ngsd_timing();
-      return NGSD_OK;
+      return copy_out(ctx, out, num_opt, cnt_opt);
     }
   }
 
   // K splits of the word list; an int32 accumulator must hold max_byte * weight * sites of one split
-  int grid = ctx->n_sm * ngsd_imma_ctas_per_sm();
   std::vector<uint32_t> splits;
   std::vector<double> scales;
   if (use_cache) {
@@ -884,41 +901,15 @@ static int distances_int(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n
     scales.resize(n_blocks);
     for (uint64_t b = 0; b < n_blocks; b++) scales[b] = (double) block_counts[b];
   } else {
-    splits = plan_splits((uint32_t) n_words, ctx->n_tiles, (double) ctx->n_tiles, grid);
-  }
-  if (!use_cache) {
+    splits = plan_splits((uint32_t) n_words, ctx->n_tiles, (double) ctx->n_tiles, ctx->n_sm);
     const uint64_t per_word = (uint64_t) std::max(ctx->int_max_byte, 1) * std::min<uint32_t>(maxw, wcap) * 64;
-    const uint32_t cap = (uint32_t) std::max<uint64_t>(1, 2147483647ull / per_word);
-    std::vector<uint32_t> cut;
-    cut.push_back(0);
-    for (size_t k = 1; k < splits.size(); k++) {
-      while (splits[k] - cut.back() > cap) cut.push_back(cut.back() + cap);
-      if (splits[k] > cut.back()) cut.push_back(splits[k]);
-    }
-    if (cut.size() < 2) cut.push_back(0);
-    splits.swap(cut);
+    cap_splits(splits, (uint32_t) std::max<uint64_t>(1, 2147483647ull / per_word));
   }
   const uint32_t n_splits = (uint32_t) splits.size() - 1;
   const uint64_t n_units = (uint64_t) n_splits * ctx->n_tiles;
-  grid = (int) std::min<uint64_t>(grid, std::max<uint64_t>(n_units, 1));
-  rc = ensure_dist_buffers(ctx, use_cache ? 1 : (do_count ? n_units + 1 : n_units / 2 + 1));   // int32 partials: sum tile (+ count tile) per unit
+  const int grid = (int) std::min<uint64_t>(ctx->n_sm, std::max<uint64_t>(n_units, 1));
+  int rc = ensure_dist_buffers(ctx, use_cache ? 1 : (do_count ? n_units + 1 : n_units / 2 + 1));   // int32 partials: sum tile (+ count tile) per unit
   if (rc) return rc;
-  if (bytes_w > ctx->wsite_cap) {
-    cudaFree(ctx->d_wsite);
-    ctx->d_wsite = nullptr;
-    ctx->wsite_cap = 0;
-    NGSD_CUDA(ctx, dev_alloc(&ctx->d_wsite, bytes_w));
-    ctx->wsite_cap = bytes_w;
-  }
-  if ((uint64_t) layers * NW > ctx->word_cap) {
-    cudaFree(ctx->d_word_ids);
-    cudaFree(ctx->d_word_layer);
-    ctx->d_word_ids = ctx->d_word_layer = nullptr;
-    ctx->word_cap = 0;
-    NGSD_CUDA(ctx, dev_alloc(&ctx->d_word_ids, (uint64_t) layers * NW));
-    NGSD_CUDA(ctx, dev_alloc(&ctx->d_word_layer, (uint64_t) layers * NW));
-    ctx->word_cap = (uint64_t) layers * NW;
-  }
   if (splits.size() > ctx->split_cap) {
     cudaFree(ctx->d_split_begin);
     ctx->d_split_begin = nullptr;
@@ -935,30 +926,26 @@ static int distances_int(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n
   ctx->timing = ngsd_timing();
   NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_split_begin, splits.data(), splits.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
   if (use_cache) NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_split_scale, scales.data(), scales.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-  const bool run_kernel = n_words && !(use_cache && !build_cache);
-  if (run_kernel) NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_wsite, h_w, bytes_w, cudaMemcpyHostToDevice, ctx->stream));
-  if (run_kernel) {
-    NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_word_ids, h_ids, n_words * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-    NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_word_layer, h_layer, n_words * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-  }
+  const bool run_kernel = n_words && contract;
   int launches = 0;
   tick(ctx, 2);
   tick(ctx, 3);
   if (run_kernel) {
-    NGSD_CUDA(ctx, ngsd_launch_dist_imma(ctx, (uint32_t) n_units, grid, do_count));
+    const uint32_t pstride = do_count ? 2 * NGSD_TILE_ELEMS : NGSD_TILE_ELEMS;
+    NGSD_CUDA(ctx, ngsd_launch_dist_umma(ctx, (uint32_t) n_units, grid, pstride, false));
+    // with --pairwise_del a second pass over the same units: the shared-site counts, as the second tile of each slot
+    if (do_count) NGSD_CUDA(ctx, ngsd_launch_dist_umma(ctx, (uint32_t) n_units, grid, pstride, true));
     launches += do_count ? 2 : 1;
   }
   tick(ctx, 4);
   tick(ctx, 8);
   if (n_words) {
-    NGSD_CUDA(ctx, ngsd_launch_epilogue_int(ctx, n_splits, n_eff, do_count, do_count));
+    NGSD_CUDA(ctx, ngsd_launch_epilogue_int(ctx, n_splits, n_eff, do_count));
     launches += 2;
   }
   tick(ctx, 5);
-  if (out) NGSD_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_out, n2 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-  if (num_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(num_opt, ctx->d_num, n2 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-  if (cnt_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(cnt_opt, ctx->d_cntout, n2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
-  NGSD_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  rc = copy_out(ctx, out, num_opt, cnt_opt);
+  if (rc) return rc;
   float ms;
   ctx->timing.count_ms = 0;                                  // part of dist_ms: the count GEMM runs inside K2c
   cudaEventElapsedTime(&ms, ctx->ev[3], ctx->ev[4]); ctx->timing.dist_ms = ms;
@@ -966,7 +953,9 @@ static int distances_int(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n
   cudaEventElapsedTime(&ms, ctx->ev[2], ctx->ev[5]); ctx->timing.total_ms = ms;
   ctx->timing.launches = launches;
   ctx->timing.dist_ctas = grid;
-  ctx->timing.dist_imma = run_kernel ? (uint64_t) n_words * ((ngsd_use_umma() ? 6 : 8) + (do_count ? 2 : 0)) * ctx->n_tiles * 128ull : 0;   // 8 (6 in three-plane form; +2 count) k-steps of 32 K bytes per word, 8 warps x 16 IMMA-equivalents per k-step
+  // IMMA-equivalents (4096 MAC each): 6 k-steps of 32 K bytes per word in the three-byte form (+2 for the count pass),
+  // 128 per k-step and tile
+  ctx->timing.dist_imma = run_kernel ? (uint64_t) n_words * (6 + (do_count ? 2 : 0)) * ctx->n_tiles * 128ull : 0;
   ctx->timing.active_sites = active_sites;
   ctx->timing.block_cache = use_cache ? (build_cache ? 1 : 2) : 0;
   if (use_cache) {
@@ -1016,80 +1005,19 @@ static int ensure_entries(ngsd_ctx *ctx, uint64_t n) {
 }
 
 // --pairwise_del counts of the FP64 path as an int8 GEMM on the tensor cores (north_star (3): "integer mask GEMM"):
-// per-site weight bytes (bootstrap multiplicities, layers of <= 127), the list of 64-site words with a non-zero weight,
-// K splits for load balance, then k_dist_umma<true> + k_cnt_reduce into ctx->d_cnt.  Queued on ctx->stream.
+// the word list of the per-site weights (build_word_list, layers of <= 127), K splits for load balance, then
+// k_dist_umma<true> + k_cnt_reduce into ctx->d_cnt.  Queued on ctx->stream.
 static int count_on_tensor_cores(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_blocks, uint64_t block_size, uint32_t maxw, int *launches) {
-  const bool weighted = block_counts != nullptr;
-  const uint64_t NW = ctx->NW, nsp = NW * 64;
-  const uint32_t layers = (maxw + 126) / 127;
-  const uint64_t bytes_w = (uint64_t) layers * nsp, n_list = (uint64_t) layers * NW;
-  const uint64_t need = ((bytes_w + 63) / 64) * 64 + 2 * n_list * sizeof(uint32_t) + 64;
-  if (ctx->h_pin2_bytes < need) {
-    if (ctx->h_pin2) cudaFreeHost(ctx->h_pin2);
-    ctx->h_pin2 = nullptr;
-    ctx->h_pin2_bytes = 0;
-    NGSD_CUDA(ctx, cudaHostAlloc(&ctx->h_pin2, need, cudaHostAllocDefault));
-    ctx->h_pin2_bytes = need;
-  }
-  uint8_t *h_w = (uint8_t *) ctx->h_pin2;
-  uint32_t *h_ids = (uint32_t *) (h_w + ((bytes_w + 63) / 64) * 64), *h_layer = h_ids + n_list;
-  memset(h_w, 0, bytes_w);
-  if (!weighted) {
-    memset(h_w, 1, ctx->n_sites);
-  } else {
-    for (uint64_t b = 0; b < n_blocks; b++) {
-      uint32_t left = block_counts[b];
-      for (uint32_t l = 0; l < layers && left; l++) {
-        const uint32_t w = std::min<uint32_t>(left, 127);
-        memset(h_w + (uint64_t) l * nsp + b * block_size, (int) w, block_size);
-        left -= w;
-      }
-    }
-  }
   uint64_t n_words = 0;
-  for (uint32_t l = 0; l < layers; l++)
-    for (uint64_t w = 0; w < NW; w++) {
-      const uint64_t *p8 = (const uint64_t *) (h_w + (uint64_t) l * nsp + w * 64);
-      if (p8[0] | p8[1] | p8[2] | p8[3] | p8[4] | p8[5] | p8[6] | p8[7]) {
-        const uint64_t one = 0x0101010101010101ull;
-        const bool unit = (p8[0] & p8[1] & p8[2] & p8[3] & p8[4] & p8[5] & p8[6] & p8[7]) == one && (p8[0] | p8[1] | p8[2] | p8[3] | p8[4] | p8[5] | p8[6] | p8[7]) == one;
-        h_ids[n_words] = (uint32_t) w;
-        h_layer[n_words] = l | (unit ? 0x80000000u : 0u);
-        n_words++;
-      }
-    }
+  int rc = build_word_list(ctx, block_counts, n_blocks, block_size, maxw, 127, false, 0, &ctx->h_pin2, &ctx->h_pin2_bytes, &n_words);
+  if (rc) return rc;
   if (n_words == 0) {
     NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_cnt, 0, ctx->n_pad * ctx->n_pad * sizeof(uint32_t), ctx->stream));
     return NGSD_OK;
   }
   std::vector<uint32_t> splits = plan_splits((uint32_t) n_words, ctx->n_tiles, (double) ctx->n_tiles, ctx->n_sm);
-  {   // an int32 accumulator holds 127 * 64 per word
-    const uint32_t cap = 2147483647u / (127u * 64u);
-    std::vector<uint32_t> cut;
-    cut.push_back(0);
-    for (size_t k = 1; k < splits.size(); k++) {
-      while (splits[k] - cut.back() > cap) cut.push_back(cut.back() + cap);
-      if (splits[k] > cut.back()) cut.push_back(splits[k]);
-    }
-    splits.swap(cut);
-  }
+  cap_splits(splits, 2147483647u / (127u * 64u));   // an int32 accumulator holds 127 * 64 per word
   const uint32_t n_splits = (uint32_t) splits.size() - 1;
-  if (bytes_w > ctx->wsite_cap) {
-    cudaFree(ctx->d_wsite);
-    ctx->d_wsite = nullptr;
-    ctx->wsite_cap = 0;
-    NGSD_CUDA(ctx, dev_alloc(&ctx->d_wsite, bytes_w));
-    ctx->wsite_cap = bytes_w;
-  }
-  if (n_list > ctx->word_cap) {
-    cudaFree(ctx->d_word_ids);
-    cudaFree(ctx->d_word_layer);
-    ctx->d_word_ids = ctx->d_word_layer = nullptr;
-    ctx->word_cap = 0;
-    NGSD_CUDA(ctx, dev_alloc(&ctx->d_word_ids, n_list));
-    NGSD_CUDA(ctx, dev_alloc(&ctx->d_word_layer, n_list));
-    ctx->word_cap = n_list;
-  }
   if (splits.size() > ctx->cs_cap) {
     cudaFree(ctx->d_cs_begin);
     ctx->d_cs_begin = nullptr;
@@ -1106,9 +1034,6 @@ static int count_on_tensor_cores(ngsd_ctx *ctx, const uint32_t *block_counts, ui
     ctx->cnt_part_ints = part;
   }
   NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_cs_begin, splits.data(), splits.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));   // pageable: staged before return
-  NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_wsite, h_w, bytes_w, cudaMemcpyHostToDevice, ctx->stream));
-  NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_word_ids, h_ids, n_words * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-  NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_word_layer, h_layer, n_words * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
   if (ctx->shard_world > 1) NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_cnt, 0, ctx->n_pad * ctx->n_pad * sizeof(uint32_t), ctx->stream));
   ngsd_count_umma_args ca{ctx->d_cs_begin, n_splits, ctx->d_cnt_part, ctx->d_wsite, ctx->d_word_ids, ctx->d_word_layer};
   NGSD_CUDA(ctx, ngsd_launch_count_umma(ctx, ca));
@@ -1144,10 +1069,8 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
       NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_num, 0, n2z * sizeof(double), ctx->stream));
       NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_cntout, 0, n2z * sizeof(uint64_t), ctx->stream));
       NGSD_CUDA(ctx, ngsd_launch_finish(ctx));
-      if (out) NGSD_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_out, n2z * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-      if (num_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(num_opt, ctx->d_num, n2z * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-      if (cnt_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(cnt_opt, ctx->d_cntout, n2z * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
-      NGSD_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+      rc0 = copy_out(ctx, out, num_opt, cnt_opt);
+      if (rc0) return rc0;
       ctx->timing = ngsd_timing();
       ctx->timing.launches = 1;
       return NGSD_OK;
@@ -1169,10 +1092,8 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
       const uint64_t n2z = ctx->n_ind * ctx->n_ind;
       NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_num, 0xFF, n2z * sizeof(double), ctx->stream));   // all-ones = the negative quiet NaN x86 gives 0/0
       NGSD_CUDA(ctx, ngsd_launch_finish(ctx, n_eff));
-      if (out) NGSD_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_out, n2z * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-      if (num_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(num_opt, ctx->d_num, n2z * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-      if (cnt_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(cnt_opt, ctx->d_cntout, n2z * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
-      NGSD_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+      rc0 = copy_out(ctx, out, num_opt, cnt_opt);
+      if (rc0) return rc0;
       ctx->timing = ngsd_timing();
       ctx->timing.launches = 1;
       return NGSD_OK;
@@ -1181,7 +1102,7 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
   const uint64_t SC = (uint64_t) ctx->sc;
   const uint64_t NCu = (ctx->n_sites + SC - 1) / SC;   // chunks that hold data
 
-  // ---- host-side bootstrap bookkeeping: per-site weights, active chunk list, level-mask entries ----
+  // ---- host-side bootstrap bookkeeping: per-site weights, active chunk list, K3 entries of the block cache ----
   uint64_t n_chunks = NCu, n_entries = 0, active_sites = n_eff;
   bool uniform_scale = false;
   std::vector<uint32_t> class_end;      // (uniform_scale) end position of each weight class in the sorted chunk list
@@ -1189,10 +1110,10 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
   uint32_t maxw = 1;
   if (weighted)
     for (uint64_t b = 0; b < n_blocks; b++) maxw = std::max(maxw, block_counts[b]);
-  const uint64_t ent_max = ctx->cfg.pairwise_del ? std::max<uint64_t>(ctx->NW * (weighted ? maxw : 1), ctx->NW + 2 * n_blocks + 2) : 0;
+  const uint64_t ent_max = ctx->cfg.pairwise_del ? ctx->NW + 2 * n_blocks + 2 : 0;   // a block touches <= block_size / 64 + 2 words
   const uint64_t bytes_w = ctx->NC * SC * sizeof(double), bytes_c = ctx->NC * sizeof(uint32_t);
   const uint64_t bytes_e = ent_max * (sizeof(uint32_t) + sizeof(uint64_t));
-  int rc = ensure_pinned(ctx, bytes_w + bytes_c + bytes_e + 64);
+  int rc = ensure_pinned(ctx, &ctx->h_pin, &ctx->h_pin_bytes, bytes_w + bytes_c + bytes_e + 64);
   if (rc) return rc;
   double *h_w = (double *) ctx->h_pin;
   uint64_t *h_em = (uint64_t *) ((char *) ctx->h_pin + bytes_w);
@@ -1206,7 +1127,7 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
   // bit 2, which benchmarks of the per-replicate weighted contraction set) the replicate is contracted directly.
   const uint64_t em_ld = em_path ? ngsd_em_ld(ctx) : 0;
   bool use_cache = false, build_cache = false;
-  if (weighted && !(ctx->cfg.reserved & 4) && !getenv("NGSD_NO_BLOCK_CACHE") && block_size % SC == 0 && n_blocks >= 2 &&
+  if (weighted && !(ctx->cfg.reserved & 4) && block_size % SC == 0 && n_blocks >= 2 &&
       n_blocks < 0x7fffffffull / std::max<uint32_t>(ctx->n_tiles, 1)) {
     const uint64_t need = em_path ? n_blocks * em_ld * em_ld : n_blocks * (uint64_t) ctx->n_tiles * NGSD_TILE_ELEMS;
     // with --pairwise_del the per-block shared-site counts are cached next to the sums (one K3 split per block)
@@ -1276,10 +1197,6 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
       memcpy(h_c, sorted.data(), n_chunks * sizeof(uint32_t));
     }
   }
-  const bool cnt_cacheable = use_cache && ctx->cfg.pairwise_del && n_blocks <= 65535 && ctx->d_cnt_cache != nullptr;
-  const bool tc_count_planned = ctx->cfg.pairwise_del && !cnt_cacheable && ngsd_use_umma() && !getenv("NGSD_COUNT_POPC");
-  if (ctx->cfg.pairwise_del && !cnt_cacheable && !tc_count_planned) n_entries = build_count_entries(ctx, block_counts, n_blocks, block_size, maxw, h_ew, h_em);
-
   if (ctx->n_tiles == 0) {   // a tile shard that owns nothing: all-zero contribution
     int rc0 = ensure_dist_buffers(ctx, 1);
     if (rc0) return rc0;
@@ -1287,40 +1204,36 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
     NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_out, 0, n2z * sizeof(double), ctx->stream));
     NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_num, 0, n2z * sizeof(double), ctx->stream));
     NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_cntout, 0, n2z * sizeof(uint64_t), ctx->stream));
-    if (out) NGSD_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_out, n2z * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    if (num_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(num_opt, ctx->d_num, n2z * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    if (cnt_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(cnt_opt, ctx->d_cntout, n2z * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    NGSD_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     ctx->timing = ngsd_timing();
-    return NGSD_OK;
+    return copy_out(ctx, out, num_opt, cnt_opt);
   }
-  // shared-site counts of the cached path: K3 with one split per source block, kept next to the per-block sums
-  const bool cnt_cached = use_cache && ctx->cfg.pairwise_del && n_blocks <= 65535 && ctx->d_cnt_cache != nullptr &&
-                          ctx->cnt_cache_elems >= n_blocks * (uint64_t) ctx->n_tiles * NGSD_TILE_ELEMS;
+  // The shared-site counts of --pairwise_del come from one of two sources: the per-block counts of the block cache
+  // (K3 builds them next to the per-block sums, one split per source block; the cache build above sized d_cnt_cache
+  // for this geometry), or the int8 count pass on the tensor cores.
+  const bool cnt_from_cache = use_cache && ctx->cfg.pairwise_del && n_blocks <= 65535 && ctx->d_cnt_cache != nullptr;
+  const bool cnt_on_tc = ctx->cfg.pairwise_del && !cnt_from_cache;
+  const bool run_k3 = cnt_from_cache && build_cache;
   std::vector<uint32_t> ent_begin;
-  if (cnt_cached) {
-    n_entries = 0;
-    if (build_cache) {
-      ent_begin.resize(n_blocks + 1);
-      for (uint64_t b = 0; b < n_blocks; b++) {
-        ent_begin[b] = (uint32_t) n_entries;
-        uint64_t s0 = b * block_size, s1 = s0 + block_size;
-        while (s0 < s1) {   // the block's bits, word by word
-          const uint64_t w = s0 >> 6, lo = s0 & 63, hi = std::min<uint64_t>(64, lo + (s1 - s0));
-          h_ew[n_entries] = (uint32_t) w;
-          h_em[n_entries] = (hi == 64 ? ~0ull : ((1ull << hi) - 1)) & ~((1ull << lo) - 1);
-          n_entries++;
-          s0 += hi - lo;
-        }
+  if (run_k3) {   // K3 entries: the sites of every block as (word, mask) pairs
+    ent_begin.resize(n_blocks + 1);
+    for (uint64_t b = 0; b < n_blocks; b++) {
+      ent_begin[b] = (uint32_t) n_entries;
+      uint64_t s0 = b * block_size, s1 = s0 + block_size;
+      while (s0 < s1) {   // the block's bits, word by word
+        const uint64_t w = s0 >> 6, lo = s0 & 63, hi = std::min<uint64_t>(64, lo + (s1 - s0));
+        h_ew[n_entries] = (uint32_t) w;
+        h_em[n_entries] = (hi == 64 ? ~0ull : ((1ull << hi) - 1)) & ~((1ull << lo) - 1);
+        n_entries++;
+        s0 += hi - lo;
       }
-      ent_begin[n_blocks] = (uint32_t) n_entries;
-      if (n_blocks + 1 > ctx->ent_begin_cap) {
-        cudaFree(ctx->d_ent_begin);
-        ctx->d_ent_begin = nullptr;
-        ctx->ent_begin_cap = 0;
-        NGSD_CUDA(ctx, dev_alloc(&ctx->d_ent_begin, n_blocks + 1));
-        ctx->ent_begin_cap = n_blocks + 1;
-      }
+    }
+    ent_begin[n_blocks] = (uint32_t) n_entries;
+    if (n_blocks + 1 > ctx->ent_begin_cap) {
+      cudaFree(ctx->d_ent_begin);
+      ctx->d_ent_begin = nullptr;
+      ctx->ent_begin_cap = 0;
+      NGSD_CUDA(ctx, dev_alloc(&ctx->d_ent_begin, n_blocks + 1));
+      ctx->ent_begin_cap = n_blocks + 1;
     }
   }
 
@@ -1388,7 +1301,7 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
   }
   ctx->cur_partials = use_cache ? ctx->d_cache : ctx->d_partials;
   ctx->cur_split_w = use_cache ? ctx->d_split_scale : nullptr;
-  ctx->cur_cnt_cache = cnt_cached ? ctx->d_cnt_cache : nullptr;
+  ctx->cur_cnt_cache = cnt_from_cache ? ctx->d_cnt_cache : nullptr;
 
   ctx->timing = ngsd_timing();
   // (pageable source: the copy is staged before the call returns, so `splits` may go out of scope afterwards)
@@ -1404,24 +1317,21 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
     NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_ent_word, h_ew, n_entries * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
     NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_ent_mask, h_em, n_entries * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
   }
-  if (!ent_begin.empty())
+  if (run_k3)
     NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_ent_begin, ent_begin.data(), ent_begin.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
   int launches = 0;
   const bool do_count = ctx->cfg.pairwise_del != 0;
-  bool run_count = do_count && !(cnt_cached && !build_cache);   // cached counts of this geometry are resident
   tick(ctx, 2);
-  const bool tc_count = run_count && !cnt_cached && ngsd_use_umma() && !getenv("NGSD_COUNT_POPC");
-  if (tc_count) {   // counts on the int8 tensor cores, ahead of the contraction on the same stream (mask_count.cu stays for the block cache)
+  if (cnt_on_tc) {   // counts on the int8 tensor cores, ahead of the contraction on the same stream
     NGSD_CUDA(ctx, cudaEventRecord(ctx->ev[6], ctx->stream));
     int rcc = count_on_tensor_cores(ctx, block_counts, n_blocks, block_size, maxw, &launches);
     if (rcc) return rcc;
     NGSD_CUDA(ctx, cudaEventRecord(ctx->ev[7], ctx->stream));
-    run_count = false;
   }
-  if (run_count) NGSD_CUDA(ctx, cudaEventRecord(ctx->ev_fork, ctx->stream));   // entry lists are on the device
+  if (run_k3) NGSD_CUDA(ctx, cudaEventRecord(ctx->ev_fork, ctx->stream));   // K3 entry lists are on the device
   tick(ctx, 3);
-  // K2 / K2b first, so that its persistent CTAs own every SM; K3 is then launched on the auxiliary stream and its
-  // (small) CTAs co-reside with them: integer AND+POPC in the shadow of the FP64 contraction.
+  // K2 / K2b first, so that its persistent CTAs own every SM; K3 (building the block cache's counts) is then launched on
+  // the auxiliary stream and its (small) CTAs co-reside with them: integer AND+POPC in the shadow of the FP64 contraction.
   if (use_cache && !build_cache) {
     // the per-block partials of this geometry are resident: nothing to contract
   } else if (em_path) {
@@ -1435,14 +1345,14 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
   }
   NGSD_CUDA(ctx, dbg_sync(ctx, "contraction"));
   tick(ctx, 4);
-  if (run_count) {
+  if (run_k3) {
     NGSD_CUDA(ctx, cudaStreamWaitEvent(ctx->aux_stream, ctx->ev_fork, 0));
     NGSD_CUDA(ctx, cudaEventRecord(ctx->ev[6], ctx->aux_stream));
-    NGSD_CUDA(ctx, ngsd_launch_mask_count(ctx, n_entries, ctx->aux_stream, cnt_cached ? (uint32_t) n_blocks : 0u));
+    NGSD_CUDA(ctx, ngsd_launch_mask_count(ctx, (uint32_t) n_blocks, ctx->aux_stream));
     NGSD_CUDA(ctx, cudaEventRecord(ctx->ev[7], ctx->aux_stream));
     NGSD_CUDA(ctx, cudaEventRecord(ctx->ev_join, ctx->aux_stream));
     NGSD_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
-    launches += n_entries ? 1 : 0;
+    launches++;
   }
   NGSD_CUDA(ctx, dbg_sync(ctx, "mask count"));
   tick(ctx, 8);
@@ -1469,14 +1379,11 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
   }
   NGSD_CUDA(ctx, dbg_sync(ctx, "epilogue"));
   tick(ctx, 5);
-  const uint64_t n2 = ctx->n_ind * ctx->n_ind;
-  if (out) NGSD_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_out, n2 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-  if (num_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(num_opt, ctx->d_num, n2 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-  if (cnt_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(cnt_opt, ctx->d_cntout, n2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
-  NGSD_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  rc = copy_out(ctx, out, num_opt, cnt_opt);
+  if (rc) return rc;
   float ms;
   ctx->timing.count_ms = 0;
-  if (run_count || tc_count) { cudaEventElapsedTime(&ms, ctx->ev[6], ctx->ev[7]); ctx->timing.count_ms = ms; }   // K3 overlaps dist_ms; the tensor-core count precedes it
+  if (cnt_on_tc || run_k3) { cudaEventElapsedTime(&ms, ctx->ev[6], ctx->ev[7]); ctx->timing.count_ms = ms; }   // K3 overlaps dist_ms; the tensor-core count precedes it
   cudaEventElapsedTime(&ms, ctx->ev[3], ctx->ev[4]); ctx->timing.dist_ms = ms;
   cudaEventElapsedTime(&ms, ctx->ev[8], ctx->ev[5]); ctx->timing.epilogue_ms = ms;
   cudaEventElapsedTime(&ms, ctx->ev[2], ctx->ev[5]); ctx->timing.total_ms = ms;
@@ -1566,9 +1473,7 @@ int ngsd_finish(ngsd_ctx *ctx, double *out_host) {
   if (!ctx->d_out) { ngsd_set_error(ctx, "no results yet: call ngsd_distances first"); return NGSD_ERR_STATE; }
   NGSD_CUDA(ctx, cudaSetDevice(ctx->device));
   NGSD_CUDA(ctx, ngsd_launch_finish(ctx));
-  if (out_host) NGSD_CUDA(ctx, cudaMemcpyAsync(out_host, ctx->d_out, ctx->n_ind * ctx->n_ind * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-  NGSD_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  return NGSD_OK;
+  return copy_out(ctx, out_host, nullptr, nullptr);
 }
 
 // ------------------------------------------------------------------------------------------- bootstrap RNG ----

@@ -14,8 +14,6 @@
 // reduces the splits in a fixed order (deterministic) and applies the normalisation + evolutionary model.
 // Bootstrap replicates (ngsDist.cpp:235-238,416-437) run as block-multiplicity weights: the chunk list skips chunks whose
 // 8 weights are all zero and B fragments are scaled in registers (exact: weights are small integers).
-#include <stdlib.h>
-
 #include "ngsd_internal.h"
 
 namespace {
@@ -74,7 +72,6 @@ struct DistArgs {
   double *partials;             // [n_units][16384]
   uint64_t NC;                  // chunk stride of the packed planes
   uint32_t n_tiles, n_units;
-  uint32_t no_diag;             // development knob: run diagonal tiles through the full-tile path
 };
 
 enum : uint32_t { kFirst = 1u, kLast = 2u, kDiag = 4u, kExit = 8u };
@@ -155,7 +152,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_dmma(DistArgs a) {
         const uint32_t c0 = a.split_begin[q], c1 = a.split_begin[q + 1];
         const double *Ab = a.Apack + (uint64_t) tl.ti * a.NC * NGSD_TILE_DOUBLES;
         const double *Bb = a.Bpack + (uint64_t) tl.tj * a.NC * NGSD_TILE_DOUBLES;
-        const uint32_t fl = (tl.ti == tl.tj && !a.no_diag) ? kDiag : 0u;
+        const uint32_t fl = tl.ti == tl.tj ? kDiag : 0u;
         for (uint32_t c = c0; c < c1; c++) {
           const uint64_t chunk = a.chunk_ids ? a.chunk_ids[c] : c;
           mbar_wait(&empty[stage], phase ^ 1);
@@ -290,7 +287,6 @@ cudaError_t ngsd_launch_dist_dmma(ngsd_ctx *ctx, const ngsd_dist_plan &p) {
   a.NC = ctx->NC;
   a.n_tiles = ctx->n_tiles;
   a.n_units = p.n_units;
-  a.no_diag = getenv("NGSD_NODIAG") ? 1u : 0u;
   cudaError_t e = cudaMemsetAsync(ctx->d_sched, 0, sizeof(uint32_t), ctx->stream);
   if (e != cudaSuccess) return e;
   if (p.weighted && !p.uniform_scale) {

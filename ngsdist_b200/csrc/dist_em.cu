@@ -14,19 +14,19 @@
 //     ahat_x(t) = x^t / S_x(t)      the individual's factor of sfs_t
 // and the pair-site term is  ahat_i(T)^T . score . ahat_j(T)  with T = first t whose rho product is below e^0.001.
 //
-// Kernel structure: one CTA owns a 64 x 64 tile of pairs and a range of sites.  Per site it alternates
-//   build : 128 individual-sites x 50 EM steps -> shared-memory tables (rho for rows and columns; ahat for the rows;
-//           u = score . ahat folded with the sum-to-one identity for the columns), 2 threads per individual-site;
-//   pairs : every thread finds T for its 16 pairs by bisection on the rho tables -- valid because rho_i * rho_j is
-//           non-increasing beyond t* = the last step at which either sequence still rises (recorded by the build; the
-//           steps up to t* are scanned linearly, which is rare: t* = 0 for > 96 % of Dirichlet individual-sites) --
-//           and adds  u2 + ahat0 * (u0 - u2) + ahat1 * (u1 - u2)  (3 operands per side, 2 FMA).
+// Kernel structure (k_dist_em3): one CTA owns a 64 x 64 tile of pairs and a range of 8-site chunks.  Per TWO sites it
+// alternates
+//   build : 2 sites x 128 individual-sites x EM steps 1..26 -> shared-memory tables (rho and ahat for rows and columns),
+//           one thread per (site, individual, half of the steps); each individual-site also records t* (the last step
+//           at which rho still rises), the search interval [lo, hi] of the stop and its state at step 27;
+//   pairs : every thread finds T for its 8 pairs per site by bisection on the rho tables -- valid because rho_i * rho_j
+//           is non-increasing beyond max(t*_i, t*_j) (the steps up to it are scanned linearly, which is rare: t* = 0
+//           for > 96 % of Dirichlet individual-sites) -- and adds the pair term of the ahat factors at T (8 FMA).
+//           A pair that has not stopped by step 26 continues by direct iteration from the saved state at step 27.
 // A warp works on ONE row and 32 columns at a time, so row-table reads are broadcasts / few distinct addresses and
 // column-table reads ([t][column] layout) are conflict-free whatever t each lane is at.  ~50 FP64 instructions per
 // pair-site instead of ~200 for the direct iteration, and no data-dependent trip counts in the common case.
 // Powers are taken of x / max(x) so nothing underflows; rho and ahat are scale invariant.
-#include <stdlib.h>
-
 #include <algorithm>
 
 #include "ngsd_internal.h"
@@ -36,22 +36,10 @@ namespace {
 constexpr int kEdge = 64;                       // pairs tile: 64 rows x 64 columns
 constexpr int kIter = 50;                       // maxIter of em2 (ngsDist.cpp:349)
 constexpr int kThreads = 512;                   // 16 warps: the kernel is bound by FP64 / shared-memory latency
-constexpr int kRowLd = 51;                      // row-table stride (odd: conflict-free build stores)
 constexpr double kExpTol = 1.0010005001667084;  // e^0.001 (tole of ngsDist.cpp:349)
 constexpr double kRise = 1e-13;                 // a rho step counts as "rising" above rounding noise only
-constexpr int kWin = 26;                        // k_dist_em3: EM steps held in the tables
-constexpr int kWLd = 27;                        // k_dist_em3: row-table stride (odd)
-
-// shared-memory layout (in doubles).  The bisection may probe up to index pos + 31 <= 81 of a rho table before the
-// result is masked; those reads stay inside this block (rho_row is followed by rho_col, rho_col by the factor tables).
-constexpr int kRhoRow = 0;                              // [64][51]     rho of row r at step t:    [r * 51 + t]          t = 1..49
-constexpr int kRhoCol = kRhoRow + kEdge * kRowLd;       // [50][64]     rho of column c at step t: [t * 64 + c]          t = 1..49
-constexpr int kFacRow = kRhoCol + kIter * kEdge;        // [2][64][51]  ahat_g of row r at step t: [(g * 64 + r) * 51 + t - 1]
-constexpr int kFacCol = kFacRow + 2 * kEdge * kRowLd;   // [50][2][64]  ahat_g of column c:        [((t - 1) * 2 + g) * 64 + c]
-constexpr int kRaw = kFacCol + kIter * 2 * kEdge;       // [2][6][256]  staged posteriors of one 8-site chunk (rows, columns)
-constexpr int kWgt = kRaw + 2 * 6 * 256;                // [8]          bootstrap weights of the chunk
-constexpr int kDoubles = kWgt + 8;
-constexpr size_t kSmemBytes = (size_t) kDoubles * 8 + 3 * 128 * sizeof(int);   // + tstar[2][128] (alternating) + valid[128]
+constexpr int kWin = 26;                        // EM steps held in the tables
+constexpr int kWLd = 27;                        // row-table stride (odd: conflict-free build stores)
 
 struct EmArgs {
   const double *Apack;          // packed posterior planes (A operand of dist_dmma, 3-plane layout)
@@ -86,215 +74,10 @@ __device__ __forceinline__ double pair_term(const double (&K)[9], double a0, dou
   return fma(a0, r0, fma(a1, r1, r2));
 }
 
-// EM steps of one quarter (qtr: t = 1..13, 14..26, 27..38, 39..50) of one individual-site.  SIDE 0 = row of the tile
-// (tables indexed [individual][t]), 1 = column ([t][individual]).  A rolled two-step loop keeps the kernel inside the
-// instruction cache (a fully unrolled, per-quarter specialised build thrashed it) without register moves.
-template <int SIDE, int LD = kRowLd>
-__device__ __forceinline__ int build_steps(const Pow3 &x, int qtr, double *rho_t, double *fac) {
-  constexpr int RS = SIDE == 0 ? 1 : kEdge;               // rho stride per step
-  constexpr int FS = SIDE == 0 ? 1 : 2 * kEdge;           // factor stride per step
-  constexpr int FG = SIDE == 0 ? kEdge * LD : kEdge;      // factor stride per genotype (LD = row-table stride)
-  // state at step t: p = x^t, Sc = S(t), Sp = S(t-1), rp = rho(t-1)
-  Pow3 p;
-  double Sp, Sc, rp;
-  int t, n_rho;                                   // first step, number of steps that store rho (t <= 49)
-  if (qtr == 0) {
-    p = x; Sp = 3.0; Sc = sum3(x); rp = INFINITY; t = 1; n_rho = 13;
-  } else {
-    // x^(t0-2) by square-and-multiply (t0 - 2 = 12 = 8+4, 25 = 16+8+1, 37 = 32+4+1), then two more steps
-    const Pow3 x2 = mul3(x, x), x4 = mul3(x2, x2), x8 = mul3(x4, x4), x16 = mul3(x8, x8);
-    Pow3 b;
-    if (qtr == 1) { b = mul3(x8, x4); t = 14; n_rho = 13; }
-    else if (qtr == 2) { b = mul3(mul3(x16, x8), x); t = 27; n_rho = 12; }
-    else { b = mul3(mul3(mul3(x16, x16), x4), x); t = 39; n_rho = 11; }
-    const double Sm2 = sum3(b);
-    const Pow3 pm1 = mul3(b, x);
-    Sp = sum3(pm1);
-    p = mul3(pm1, x);
-    Sc = sum3(p);
-    const double ip = fast_rcp(Sp);
-    rp = ((Sc * Sm2) * ip) * ip;                                      // rho(t0 - 1)
-  }
-  int tstar = 0;
-  rho_t += t * RS;
-  fac += (t - 1) * FS;
-  // one EM step: (p, Sp, Sc, rp) at t  ->  (n, Sc, Sn, rho) at t + 1; stores rho(t) and the factors of step t
-  auto step = [&](const Pow3 &pc, double Spv, double Scv, double rpv, Pow3 &pn, double &Snv, double &rhov, int tt, int off) {
-    pn = mul3(pc, x);
-    Snv = sum3(pn);
-    const double inv = fast_rcp(Scv);
-    rhov = ((Snv * Spv) * inv) * inv;
-    if (rhov - rpv > kRise) tstar = tt;
-    rho_t[off * RS] = rhov;
-    fac[off * FS] = pc.v0 * inv;
-    fac[off * FS + FG] = pc.v1 * inv;
-  };
-  if (n_rho & 1) {                                                    // odd count: peel one step, then go two at a time
-    Pow3 n; double Sn, rho;
-    step(p, Sp, Sc, rp, n, Sn, rho, t, 0);
-    p = n; Sp = Sc; Sc = Sn; rp = rho;
-    t++; rho_t += RS; fac += FS;
-  }
-#pragma unroll 1
-  for (int k = n_rho >> 1; k > 0; k--) {                             // ping-pong: no register moves for the carried state
-    Pow3 n; double Sn, rho;
-    step(p, Sp, Sc, rp, n, Sn, rho, t, 0);
-    step(n, Sc, Sn, rho, p, Sp, rp, t + 1, 1);                        // now p = x^(t+2), Sp(out) = S(t+2), rp = rho(t+1)
-    const double S1 = Sn;                                             // S(t+1)
-    Sc = Sp; Sp = S1;
-    t += 2; rho_t += 2 * RS; fac += 2 * FS;
-  }
-  if (qtr == 3) {                                                     // t = 50: the factors only (rho(50) is never tested)
-    const double inv = fast_rcp(Sc);
-    fac[0] = p.v0 * inv;
-    fac[FG] = p.v1 * inv;
-  }
-  return tstar;
-}
-
-// NE pairs of one thread for the current site: rows r0 (+16 when NE == 4), columns lane (+32); T by bisection, then
-// the pair term.  NE == 2 serves diagonal tiles, where rows >= 32 only pair with columns >= 32.
-template <int NE, bool WEIGHTED>
-__device__ __forceinline__ void pair_group(const double *sm, const int *ts, const int *valid, const int (&tcol)[2], const bool (&vcol)[2],
-                                           bool diag, int r0, int lane, double w, const double (&K)[9], double *acc) {
-  const double *rho_row = sm + kRhoRow, *rho_col = sm + kRhoCol, *fac_row = sm + kFacRow, *fac_col = sm + kFacCol;
-  int pos[NE], tfix[NE];
-  const double *pr[NE], *pc[NE];                                      // &rho_row[r][pos], &rho_col[pos][c]
-  bool ok[NE];
-#pragma unroll
-  for (int e = 0; e < NE; e++) {
-    const int h = NE == 4 ? (e & 1) : 1, r = r0 + (NE == 4 ? 16 * (e >> 1) : 16 * e), cc = h * 32 + lane;
-    ok[e] = (!diag || cc > r) && vcol[h] && valid[r] != 0;
-    const int tm = max(ts[r], tcol[h]);
-    pos[e] = ok[e] ? tm + 1 : kIter;
-    tfix[e] = 0;
-    if (ok[e] && tm > 0) {                              // rare: scan the non-monotone prefix 1..tm
-      for (int t = 1; t <= tm; t++)
-        if (rho_row[r * kRowLd + t] * rho_col[t * kEdge + cc] < kExpTol) { tfix[e] = t; pos[e] = kIter; break; }
-    }
-    pr[e] = rho_row + r * kRowLd + pos[e];
-    pc[e] = rho_col + pos[e] * kEdge + cc;
-  }
-  // first t in [pos, 49] whose rho product is below e^0.001, else 50 (branch-free; every t < pos is known to be above)
-#pragma unroll
-  for (int s = 32; s >= 1; s >>= 1) {
-#pragma unroll
-    for (int e = 0; e < NE; e++) {
-      const double prod = pr[e][s - 1] * pc[e][(s - 1) * kEdge];
-      const bool adv = (pos[e] + s <= kIter) && !(prod < kExpTol);
-      pos[e] += adv ? s : 0;
-      pr[e] += adv ? s : 0;
-      pc[e] += adv ? s * kEdge : 0;
-    }
-  }
-#pragma unroll
-  for (int e = 0; e < NE; e++) {
-    const int h = NE == 4 ? (e & 1) : 1, r = r0 + (NE == 4 ? 16 * (e >> 1) : 16 * e), cc = h * 32 + lane;
-    const int T1 = (tfix[e] ? tfix[e] : pos[e]) - 1;
-    const double a0 = fac_row[r * kRowLd + T1], a1 = fac_row[(kEdge + r) * kRowLd + T1];
-    const double b0 = fac_col[(T1 * 2) * kEdge + cc], b1 = fac_col[(T1 * 2 + 1) * kEdge + cc];
-    double d = pair_term(K, a0, a1, b0, b1);
-    if (WEIGHTED) d *= w;
-    if (ok[e]) acc[NE == 4 ? e : 2 * e + 1] += d;
-  }
-}
-
-// grid = n_splits * n_tiles (split-major); block 512
-template <bool WEIGHTED>
-__global__ void __launch_bounds__(kThreads, 1) k_dist_em(EmArgs a) {
-  extern __shared__ __align__(16) double sm[];
-  double *raw = sm + kRaw, *wgt = sm + kWgt;
-  int *tsb = reinterpret_cast<int *>(sm + kDoubles), *valid = tsb + 256;
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const uint32_t q = blockIdx.x / a.n_tiles;
-  uint32_t t_lin = blockIdx.x - q * a.n_tiles, ti = 0;
-  while (t_lin >= a.n64 - ti) { t_lin -= a.n64 - ti; ti++; }
-  const uint32_t tj = ti + t_lin;
-  const bool diag = ti == tj;
-  const uint32_t c0 = (uint32_t) (((uint64_t) q * a.n_chunks) / a.n_splits);
-  const uint32_t c1 = (uint32_t) (((uint64_t) (q + 1) * a.n_chunks) / a.n_splits);
-
-  // build role: warp -> (quarter of the EM steps, side, 32 individuals); rotated so that the row and column warps of a
-  // quarter are spread over the four SM sub-partitions (warp & 3).
-  const int b_qtr = warp >> 2, b_role = ((warp & 3) + b_qtr) & 3, b_side = b_role >> 1, b_k = (b_role & 1) * 32 + lane;
-  double K[9];
-#pragma unroll
-  for (int k = 0; k < 9; k++) K[k] = a.K[k];
-
-  // pairs of this thread: rows warp + 16 k (k = 0..3) x columns lane + 32 h (h = 0, 1): acc[k * 2 + h]
-  double acc[8];
-#pragma unroll
-  for (int k = 0; k < 8; k++) acc[k] = 0.0;
-  if (tid < 256) tsb[tid] = 0;
-  int par = 0;                                               // which tstar array the current site uses
-
-  for (uint32_t c = c0; c < c1; c++) {
-    const uint64_t chunk = a.chunk_ids ? a.chunk_ids[c] : (uint64_t) c;
-    __syncthreads();                                          // everyone is done with the previous chunk's weights
-    // ---- stage the chunk: 2 sides x 6 k4-groups x (64 individuals x 4 sites) = 12 contiguous 2 KiB segments ----
-#pragma unroll
-    for (int h = 0; h < 6; h++) {
-      const int seg = h * 2 + (tid >> 8);
-      const uint64_t gi0 = (uint64_t) (seg < 6 ? ti : tj) * kEdge;
-      const double *src = a.Apack + ((gi0 >> 7) * a.NC + chunk) * NGSD_TILE_DOUBLES + (seg % 6) * 512 + ((gi0 & 127) >> 3) * 32;
-      raw[seg * 256 + (tid & 255)] = src[tid & 255];
-    }
-    if (WEIGHTED && tid < NGSD_SC) wgt[tid] = a.weights[chunk * NGSD_SC + tid];
-    __syncthreads();
-
-    for (int s8 = 0; s8 < NGSD_SC; s8++) {
-      if (chunk * NGSD_SC + s8 >= a.n_sites) break;          // padding sites of the last chunk (CTA-uniform)
-      const double w = WEIGHTED ? wgt[s8] : 1.0;
-      if (WEIGHTED && w == 0.0) continue;                     // block not drawn in this replicate (CTA-uniform)
-      int *ts = tsb + par * 128;
-
-      // ================= build: tables of this site's 128 individual-sites =================
-      {
-        const double *rw = raw + (b_side * 6 + (s8 >> 2)) * 256 + b_k * 4 + (s8 & 3);
-        Pow3 x = {rw[0], rw[2 * 256], rw[4 * 256]};                        // planes g = 0,1,2 -> k4-group g*2 + h
-        const double m = fmax(x.v0, fmax(x.v1, x.v2));
-        const bool ok = m > 0;                                             // all-zero = padded or pairwise-deleted
-        if (ok) {
-          const double im = fast_rcp(m);                                   // rho and ahat are scale invariant: the largest
-          x.v0 *= im; x.v1 *= im; x.v2 *= im;                              // entry only has to be ~1 so that nothing underflows
-          int tstar;
-          if (b_side == 0) tstar = build_steps<0>(x, b_qtr, sm + kRhoRow + b_k * kRowLd, sm + kFacRow + b_k * kRowLd);
-          else tstar = build_steps<1>(x, b_qtr, sm + kRhoCol + b_k, sm + kFacCol + b_k);
-          if (tstar) atomicMax(&ts[b_side * 64 + b_k], tstar);
-        }
-        if (b_qtr == 0) valid[b_side * 64 + b_k] = ok ? 1 : 0;
-      }
-      __syncthreads();
-
-      // ================= pairs =================
-      if (tid < 128) tsb[(par ^ 1) * 128 + tid] = 0;         // the next site's tstar accumulators
-      int tcol[2];
-      bool vcol[2];
-#pragma unroll
-      for (int h = 0; h < 2; h++) { tcol[h] = ts[64 + h * 32 + lane]; vcol[h] = valid[64 + h * 32 + lane] != 0; }
-      pair_group<4, WEIGHTED>(sm, ts, valid, tcol, vcol, diag, warp, lane, w, K, acc);
-      if (diag) pair_group<2, WEIGHTED>(sm, ts, valid, tcol, vcol, diag, warp + 32, lane, w, K, acc + 4);
-      else pair_group<4, WEIGHTED>(sm, ts, valid, tcol, vcol, diag, warp + 32, lane, w, K, acc + 4);
-      par ^= 1;
-      __syncthreads();
-    }
-  }
-
-#pragma unroll
-  for (int k = 0; k < 4; k++)
-#pragma unroll
-    for (int h = 0; h < 2; h++) {
-      const int r = warp + 16 * k, cc = h * 32 + lane;
-      const uint64_t i = (uint64_t) ti * kEdge + r, j = (uint64_t) tj * kEdge + cc;
-      a.partials[((uint64_t) q * a.ld + i) * a.ld + j] = (i < j) ? acc[k * 2 + h] : 0.0;
-    }
-}
-
-
 // ---------------------------------------------------------------------------------------------------------------------
-// k_dist_em3 (round 2): the same closed form with three changes that follow from measurements of k_dist_em.
-//  * ncu + arithmetic: the build is FP64-pipe bound (128 individual-sites x 50 steps per 4096 pairs), the pair phase is
+// k_dist_em3 (round 2): the closed form above with three changes that follow from measurements of the round-1 kernel
+// k_dist_em (50-step tables, one site per build / pairs round; since removed).
+//  * ncu + arithmetic: the build was FP64-pipe bound (128 individual-sites x 50 steps per 4096 pairs), the pair phase
 //    shared-memory bound (12 LDS.64 per pair in the bisection + 4 for the factors).  On the bench data 99.9 % of the pairs
 //    stop within 26 EM steps (mean 7.8) -- but nearly every 64 x 64 tile has one pair that does not, so windowing the
 //    tables per tile does not help (tried: k_dist_em2, 164 ms against 115 ms).  Instead:
@@ -304,7 +87,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_em(EmArgs a) {
 //    rho >= 1 always (log-convexity of power sums), hence a pair can only stop at t >= max(lo_i, lo_j) and has stopped
 //    by max(hi_i, hi_j): the bisection runs on that interval -- typically 1-3 steps wide instead of 26 -- and rounds in
 //    which no lane of the warp can move are skipped.  (Margins of 1e-9 on both thresholds keep rounding out of it: the
-//    stop index is the one k_dist_em finds, from the same products.)
+//    interval always holds the first t whose rho product, of the same values, is below e^0.001.)
 //  * with 26-step tables two sites fit in shared memory at once: one barrier pair per TWO sites and twice the
 //    independent work per phase.
 constexpr int kW_RhoRow = 0;                                 // [64][27]     rho of row r at step t:    [r * 27 + t]        t = 1..26
@@ -322,8 +105,11 @@ constexpr double kSqrtTolHi = 1.0005001250208359 * (1.0 - 1e-9);   // e^0.0005: 
 
 struct TailState { Pow3 x, p; double Sp, Sc; };
 
-// build_steps for the first two quarters (t = 1..13 / 14..26) plus what k_dist_em3 needs: lo / hi of this thread's steps
-// (first t with rho < kTolLo, 1 + last t with rho >= kSqrtTolHi) and, from the second quarter, the state at t = 27.
+// EM steps of one half (qtr: t = 1..13 or 14..26) of one individual-site.  SIDE 0 = row of the tile (tables indexed
+// [individual][t]), 1 = column ([t][individual]).  Stores rho(t) and the factors ahat(t) of these steps and returns t*
+// (the last step at which rho rises); also gives lo / hi of this thread's steps (first t with rho < kTolLo, 1 + last t
+// with rho >= kSqrtTolHi) and, from the second half, the state at t = 27.  A rolled two-step loop keeps the kernel
+// inside the instruction cache without register moves.
 template <int SIDE>
 __device__ __forceinline__ int build_steps26(const Pow3 &x, int qtr, double *rho_t, double *fac, int *lo_out, int *hi_out, TailState *tail) {
   constexpr int RS = SIDE == 0 ? 1 : kEdge;
@@ -334,7 +120,7 @@ __device__ __forceinline__ int build_steps26(const Pow3 &x, int qtr, double *rho
   int t;
   if (qtr == 0) {
     p = x; Sp = 3.0; Sc = sum3(x); rp = INFINITY; t = 1;
-  } else {                                                              // x^12 by square-and-multiply, then two more steps (as build_steps)
+  } else {                                                              // x^12 by square-and-multiply, then two more steps
     const Pow3 x2 = mul3(x, x), x4 = mul3(x2, x2), x8 = mul3(x4, x4);
     const Pow3 b = mul3(x8, x4);
     t = 14;
@@ -650,15 +436,9 @@ uint32_t ngsd_em_splits(const ngsd_ctx *ctx, uint32_t n_chunks) {
 
 cudaError_t ngsd_launch_dist_em(ngsd_ctx *ctx, uint32_t n_chunks, uint32_t n_splits, bool weighted) {
   static bool attr_set[64] = {};
-  static const bool v1 = getenv("NGSD_EM_V1") != nullptr;      // A/B: the round-1 kernel (build and pairs alternate, 50-step tables)
   if (!attr_set[ctx->device & 63]) {
-    const void *fns[2] = {(const void *) k_dist_em<false>, (const void *) k_dist_em<true>};
+    const void *fns[2] = {(const void *) k_dist_em3<false>, (const void *) k_dist_em3<true>};
     for (const void *f : fns) {
-      cudaError_t e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) kSmemBytes);
-      if (e != cudaSuccess) return e;
-    }
-    const void *fns2[2] = {(const void *) k_dist_em3<false>, (const void *) k_dist_em3<true>};
-    for (const void *f : fns2) {
       cudaError_t e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) kSmem3Bytes);
       if (e != cudaSuccess) return e;
     }
@@ -688,17 +468,10 @@ cudaError_t ngsd_launch_dist_em(ngsd_ctx *ctx, uint32_t n_chunks, uint32_t n_spl
   a.K[8] = D[4] - D[5] - D[7] + D[8];
   const uint64_t grid = (uint64_t) n_splits * a.n_tiles;
   if (grid == 0 || grid > 0x7fffffffull) return cudaErrorInvalidConfiguration;
-  if (v1) {
-    if (weighted)
-      k_dist_em<true><<<(unsigned) grid, kThreads, kSmemBytes, ctx->stream>>>(a);
-    else
-      k_dist_em<false><<<(unsigned) grid, kThreads, kSmemBytes, ctx->stream>>>(a);
-  } else {
-    if (weighted)
-      k_dist_em3<true><<<(unsigned) grid, kThreads, kSmem3Bytes, ctx->stream>>>(a);
-    else
-      k_dist_em3<false><<<(unsigned) grid, kThreads, kSmem3Bytes, ctx->stream>>>(a);
-  }
+  if (weighted)
+    k_dist_em3<true><<<(unsigned) grid, kThreads, kSmem3Bytes, ctx->stream>>>(a);
+  else
+    k_dist_em3<false><<<(unsigned) grid, kThreads, kSmem3Bytes, ctx->stream>>>(a);
   return cudaGetLastError();
 }
 

@@ -1,13 +1,23 @@
-// K2c' dist_umma: the called-genotype contraction of dist_imma.cu on the 5th-generation tensor cores:
-// tcgen05.mma kind::i8 (SASS UTCIMMA), A operand and int32 accumulators in tensor memory, B operand in shared memory.
+// K2c dist_umma: the pair loop of gen_dist (ngsDist.cpp:333-364) for CALLED genotypes as an exact integer contraction on
+// the 5th-generation tensor cores: tcgen05.mma kind::i8 (SASS UTCIMMA), A operand and int32 accumulators in tensor
+// memory, B operand in shared memory.
 //
-// The arithmetic.  With codes c in {0, 1, 2, 3 = missing}, f(c_i, c_j) = the site term of ngsDist.cpp:351-353 for two called
-// genotypes, and S = 2 (--pairwise_del) or 18: acc(i,j) = S sum_s w_s f(c_i(s), c_j(s)) as an int8 GEMM with exact int32
-// accumulation and THREE K bytes per site (round 2; dist_imma.cu keeps the four-byte form):
+// When every individual-site is either a hard call or missing -- genotype input (read_data.cpp:88-95) or --call_geno with
+// N_thresh == call_thresh (gen_func.cpp:903-913; the default 0/0) -- its posterior triple is one of four states:
+// one-hot(0), one-hot(1), one-hot(2) or the uniform triple of a missing entry (code 3).  The site term
+// sum_{g1,g2} score[g1][g2] p_i[g1] p_j[g2] (ngsDist.cpp:351-353) then only depends on the two codes: a 4 x 4 table
+// f(c_i, c_j).  HBM holds 2 bits per individual-site (plus the same codes as 4-bit selectors) instead of FP64 planes.
+//
+// The arithmetic.  With S = 2 (--pairwise_del) or 18 (otherwise: the uniform 1/3 makes f a multiple of 1/18) and w_s the
+// bootstrap multiplicity of the site (ngsDist.cpp:416-437; 1 for replicate 0, 0 for padding):
+// acc(i,j) = S sum_s w_s f(c_i(s), c_j(s)) as an int8 GEMM with exact int32 accumulation and THREE K bytes per site:
 //     A_i[s][k] = w_s (m [c_i = k] + [c_i = 3] t),     B_j[s][k] = (S / m) f(k, c_j),     k = 0, 1, 2
 // with (m, t) = (1, 0) with --pairwise_del (row and column 3 of f are zero) and (3, 1) without (a missing genotype is the
 // uniform triple, gen_func.cpp:895-899, so its row of f is the mean of the other three) -- the same S f(c_i, c_j) exactly,
-// a quarter fewer operand bytes, MMAs and expansion instructions than one K byte per code value.  UMMA runs the int8 GEMM
+// a quarter fewer operand bytes, MMAs and expansion instructions than one K byte per code value.  Weights above
+// ngsd_int_weight_cap go into further weight layers (api.cu).  k_epilogue_int (epilogue.cu) sums the splits in int64 and
+// applies num = acc / S and the tail of gen_dist: num, cnt and the model-0 distances are bit-exact whenever the
+// reference's own sum is exact (no missing data, or --pairwise_del).  UMMA runs the int8 GEMM
 // 4x faster than mma.sync (probe: 2.3e15 vs 5.7e14 MAC/s) but cannot take operands from registers, so the expansion of the
 // 2-bit codes is written out every stage.  A CTA is a four-role pipeline connected by mbarrier rings:
 //
@@ -517,7 +527,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_umma(const __grid_constant
   if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512u) : "memory");
 }
 
-// register / smem-resident UMMA loop: the int8 tensor issue-rate ceiling through tcgen05 (roofline denominator of K2c')
+// register / smem-resident UMMA loop: the int8 tensor issue-rate ceiling through tcgen05 (roofline denominator of K2c)
 __global__ void __launch_bounds__(128, 1) k_umma_peak(int iters) {
   __shared__ __align__(128) unsigned char sA[2 * 16 * 128];
   __shared__ __align__(128) unsigned char sB[2 * 16 * 128];
@@ -550,6 +560,29 @@ __global__ void __launch_bounds__(128, 1) k_umma_peak(int iters) {
   if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(128u) : "memory");
 }
 
+// register-only loop of the older warp-level int8 MMA (mma.sync, SASS IMMA.16832): its issue-rate ceiling, for comparison
+__device__ __forceinline__ void imma16832(int (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+  asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.s8.s8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+               : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3])
+               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
+
+__global__ void k_imma_peak(int *out, int iters) {
+  int c[8][4];
+#pragma unroll
+  for (int i = 0; i < 8; i++) c[i][0] = c[i][1] = c[i][2] = c[i][3] = 0;
+  const uint32_t a[4] = {threadIdx.x, threadIdx.x * 3u, 7u, 9u};
+  const uint32_t b0 = threadIdx.x + 1u, b1 = 5u;
+  for (int it = 0; it < iters; it++) {
+#pragma unroll
+    for (int i = 0; i < 8; i++) imma16832(c[i], a, b0, b1);
+  }
+  int s = 0;
+#pragma unroll
+  for (int i = 0; i < 8; i++) s += c[i][0] + c[i][1] + c[i][2] + c[i][3];
+  if (s == 0x12345678) out[0] = s;
+}
+
 }  // namespace
 
 extern "C" int ngsd_probe_umma_tmacs(int device, double *umma_tmacs) {
@@ -576,8 +609,61 @@ extern "C" int ngsd_probe_umma_tmacs(int device, double *umma_tmacs) {
   return NGSD_OK;
 }
 
+extern "C" int ngsd_probe_int8_tmacs(int device, double *imma_tmacs) {
+  if (cudaSetDevice(device) != cudaSuccess) return NGSD_ERR_CUDA;
+  cudaDeviceProp prop;
+  if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return NGSD_ERR_CUDA;
+  int *d = nullptr;
+  if (cudaMalloc(&d, 64) != cudaSuccess) return NGSD_ERR_CUDA;
+  const int iters = 8192, warps = 16, nsm = prop.multiProcessorCount;
+  cudaEvent_t e0, e1;
+  cudaEventCreate(&e0);
+  cudaEventCreate(&e1);
+  float best = 1e30f;
+  for (int r = 0; r < 4; r++) {
+    cudaEventRecord(e0);
+    k_imma_peak<<<nsm, warps * 32>>>(d, iters);
+    cudaEventRecord(e1);
+    if (cudaEventSynchronize(e1) != cudaSuccess) { cudaFree(d); return NGSD_ERR_CUDA; }
+    float ms;
+    cudaEventElapsedTime(&ms, e0, e1);
+    if (r > 0 && ms < best) best = ms;
+  }
+  cudaEventDestroy(e0);
+  cudaEventDestroy(e1);
+  cudaFree(d);
+  *imma_tmacs = (double) nsm * warps * iters * 8 * 4096.0 / (best * 1e-3) * 1e-12;
+  return NGSD_OK;
+}
+
+// f(k, c) * S as int8 bytes; returns false when the score matrix does not give small integers (-> FP64 path)
+bool ngsd_int_lut(const double *score, bool pairwise_del, uint32_t lut[4], double *scale, int *max_byte) {
+  const double S = pairwise_del ? 2.0 : 18.0;
+  double f[4][4];
+  double rs[3] = {0, 0, 0}, cs[3] = {0, 0, 0}, tot = 0;
+  for (int k = 0; k < 3; k++)
+    for (int c = 0; c < 3; c++) { f[k][c] = score[k * 3 + c]; rs[k] += score[k * 3 + c]; cs[c] += score[k * 3 + c]; tot += score[k * 3 + c]; }
+  for (int k = 0; k < 3; k++) { f[k][3] = pairwise_del ? 0.0 : rs[k] / 3.0; f[3][k] = pairwise_del ? 0.0 : cs[k] / 3.0; }
+  f[3][3] = pairwise_del ? 0.0 : tot / 9.0;
+  int mx = 0;
+  for (int c = 0; c < 4; c++) {
+    uint32_t wv = 0;
+    for (int k = 0; k < 4; k++) {
+      const double v = f[k][c] * S, r = nearbyint(v);
+      if (fabs(v - r) > 1e-9 || r < 0 || r > 127) return false;
+      if (!pairwise_del && k < 3 && ((int) r) % 3) return false;   // the three-plane form (header) carries S / 3 on the B side
+      wv |= (uint32_t) (int) r << (8 * k);
+      if ((int) r > mx) mx = (int) r;
+    }
+    lut[c] = wv;
+  }
+  *scale = S;
+  *max_byte = mx;
+  return true;
+}
+
 // largest site weight one weight layer may carry: the A bytes are int8 and hold 3 w without --pairwise_del (header)
-uint32_t ngsd_int_weight_cap(const ngsd_ctx *ctx) { return (ngsd_use_umma() && !ctx->cfg.pairwise_del) ? 42u : 127u; }
+uint32_t ngsd_int_weight_cap(const ngsd_ctx *ctx) { return ctx->cfg.pairwise_del ? 127u : 42u; }
 
 cudaError_t ngsd_launch_dist_umma(ngsd_ctx *ctx, uint32_t n_units, int grid, uint32_t pstride, bool count) {
   static bool attr_set[64] = {};

@@ -1,8 +1,7 @@
 // K4 epilogue: deterministic reduction of the K-split partial tiles + the tail of gen_dist (ngsDist.cpp:372-401):
 //   cnt <- tot_sites override; d = num / (double) cnt; model 0: d, 1: -log(1-d), 2: -log(1-(d*4/3))*3/4;
 // symmetric write of both triangles as gen_dist_slave does (ngsDist.cpp:408-412), 0.0 diagonal (ngsDist.cpp:200).
-#include <stdlib.h>
-
+// k_epilogue reduces the FP64 partials of dist_dmma.cu, k_epilogue_int the exact int32 partials of dist_umma.cu.
 #include "ngsd_internal.h"
 
 namespace {
@@ -20,7 +19,6 @@ struct EpiArgs {
   uint64_t n_ind, n_pad, const_cnt, tot_sites;
   uint32_t n_splits, n_tiles;
   int evol_model;
-  int no_diag;
 };
 
 // grid (n_tiles, 32); block 256: one thread per double2 slot of the tile (8192 slots), splits summed in a fixed order
@@ -31,7 +29,7 @@ __global__ void __launch_bounds__(256) k_epilogue(EpiArgs a) {
   const int lane = e & 31, frag = (e >> 5) & 31, warp = e >> 10;
   // decode the slot -> (row, first column) inside the tile; layouts written by dist_dmma.cu
   int row, col0;
-  if (tl.ti == tl.tj && !a.no_diag) {     // diagonal tile: warp owns 8x8 block-rows `warp` (frags 0..15) and 15-warp (frags 16..31)
+  if (tl.ti == tl.tj) {     // diagonal tile: warp owns 8x8 block-rows `warp` (frags 0..15) and 15-warp (frags 16..31)
     const int R = (frag < 16) ? warp : 15 - warp, c = frag & 15;
     if (c < R) return;      // below the diagonal: never computed, never stored
     row = R * 8 + (lane >> 2);
@@ -86,6 +84,62 @@ __global__ void __launch_bounds__(256) k_epilogue(EpiArgs a) {
         if (w != 0.0) cnt += (uint64_t) w * (uint64_t) pc[(uint64_t) q2 * cstride];
       }
     }
+    if (a.num) a.num[i * a.n_ind + j] = a.num[j * a.n_ind + i] = num;
+    if (a.cntout) a.cntout[i * a.n_ind + j] = a.cntout[j * a.n_ind + i] = cnt;
+    if (a.tot_sites > 0) cnt = a.tot_sites;
+    double d = num / (double) cnt;
+    if (a.evol_model == 1) d = -log(1 - d);
+    else if (a.evol_model == 2) d = -log(1 - (d * 4 / 3)) * 3 / 4;
+    a.out[i * a.n_ind + j] = a.out[j * a.n_ind + i] = d;
+  }
+}
+
+struct EpiIntArgs {
+  const int32_t *partials;    // [n_splits][n_tiles][pstride] row-major tiles of dist_umma.cu (sum tile, then count tile when in_kernel_cnt)
+  const double *split_w;      // [n_splits] integer weight of each split (bootstrap block cache) or nullptr
+  uint32_t pstride;
+  int in_kernel_cnt;
+  const ngsd_tile *tiles;
+  double *out, *num;
+  uint64_t *cntout;
+  uint64_t n_ind, const_cnt, tot_sites;
+  uint32_t n_splits, n_tiles;
+  int evol_model;
+  double scale;               // S
+};
+
+// Integer path (dist_umma.cu): grid (n_tiles, 16); block 256: one thread per 4 elements of the tile (rows row0 and
+// row0 + 8, columns col0 and col0 + 1); splits summed in int64 (order-free, exact), then num = acc / S
+__global__ void __launch_bounds__(256) k_epilogue_int(EpiIntArgs a) {
+  const uint32_t t = blockIdx.x;
+  const ngsd_tile tl = a.tiles[t];
+  const uint32_t e = blockIdx.y * 256 + threadIdx.x;
+  const int lane = e & 31, frag = (e >> 5) & 15, warp = e >> 9;
+  const int wm = warp >> 2, wn = warp & 3, mi = frag >> 2, ni = frag & 3;
+  const int row0 = wm * 64 + mi * 16 + (lane >> 2), col0 = wn * 32 + ni * 8 + 2 * (lane & 3);
+  const int32_t *src = a.partials + (uint64_t) t * a.pstride + row0 * NGSD_TILE + col0;
+  const uint64_t stride = (uint64_t) a.n_tiles * a.pstride;
+  long long s[4] = {0, 0, 0, 0}, c[4] = {0, 0, 0, 0};
+  for (uint32_t q = 0; q < a.n_splits; q++) {
+    long long m = 1;
+    if (a.split_w) {                     // per-block partials x block multiplicities: integers, exact
+      m = (long long) a.split_w[q];
+      if (m == 0) continue;
+    }
+    const int32_t *p = src + (uint64_t) q * stride;
+    const int2 lo = *reinterpret_cast<const int2 *>(p), hi = *reinterpret_cast<const int2 *>(p + 8 * NGSD_TILE);
+    s[0] += m * lo.x; s[1] += m * lo.y; s[2] += m * hi.x; s[3] += m * hi.y;
+    if (a.in_kernel_cnt) {
+      const int2 clo = *reinterpret_cast<const int2 *>(p + NGSD_TILE_ELEMS), chi = *reinterpret_cast<const int2 *>(p + NGSD_TILE_ELEMS + 8 * NGSD_TILE);
+      c[0] += m * clo.x; c[1] += m * clo.y; c[2] += m * chi.x; c[3] += m * chi.y;
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < 4; k++) {
+    const uint64_t i = (uint64_t) tl.ti * NGSD_TILE + row0 + (k >> 1) * 8, j = (uint64_t) tl.tj * NGSD_TILE + col0 + (k & 1);
+    if (i >= j || j >= a.n_ind) continue;
+    const double num = (double) s[k] / a.scale;
+    uint64_t cnt = a.in_kernel_cnt ? (uint64_t) c[k] : a.const_cnt;
     if (a.num) a.num[i * a.n_ind + j] = a.num[j * a.n_ind + i] = num;
     if (a.cntout) a.cntout[i * a.n_ind + j] = a.cntout[j * a.n_ind + i] = cnt;
     if (a.tot_sites > 0) cnt = a.tot_sites;
@@ -160,6 +214,20 @@ __global__ void __launch_bounds__(256) k_deficit_fix(const uint32_t *__restrict_
   }
 }
 
+// Before an epilogue: zero the diagonal, and with a tile shard every entry, since the tiles of other ranks must read as
+// 0 (ngsd_set_tile_shard).
+cudaError_t clear_outputs(ngsd_ctx *ctx) {
+  if (ctx->shard_world > 1) {
+    const uint64_t n2 = ctx->n_ind * ctx->n_ind;
+    cudaError_t e = cudaMemsetAsync(ctx->d_out, 0, n2 * sizeof(double), ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(ctx->d_num, 0, n2 * sizeof(double), ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(ctx->d_cntout, 0, n2 * sizeof(uint64_t), ctx->stream);
+    if (e != cudaSuccess) return e;
+  }
+  k_zero_diag<<<(unsigned) ((ctx->n_ind + 255) / 256), 256, 0, ctx->stream>>>(ctx->d_out, ctx->d_num, ctx->d_cntout, ctx->n_ind);
+  return cudaGetLastError();
+}
+
 }  // namespace
 
 cudaError_t ngsd_launch_deficit_fix(ngsd_ctx *ctx, bool weighted, uint64_t n_eff) {
@@ -201,15 +269,31 @@ cudaError_t ngsd_launch_epilogue(ngsd_ctx *ctx, const ngsd_epilogue_args &e) {
   a.n_splits = e.n_splits;
   a.n_tiles = ctx->n_tiles;
   a.evol_model = ctx->cfg.evol_model;
-  a.no_diag = getenv("NGSD_NODIAG") ? 1 : 0;
-  if (ctx->shard_world > 1) {   // entries of tiles owned by other ranks must read as 0 (ngsd_set_tile_shard)
-    const uint64_t n2 = ctx->n_ind * ctx->n_ind;
-    cudaError_t e = cudaMemsetAsync(ctx->d_out, 0, n2 * sizeof(double), ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(ctx->d_num, 0, n2 * sizeof(double), ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(ctx->d_cntout, 0, n2 * sizeof(uint64_t), ctx->stream);
-    if (e != cudaSuccess) return e;
-  }
-  k_zero_diag<<<(unsigned) ((ctx->n_ind + 255) / 256), 256, 0, ctx->stream>>>(ctx->d_out, ctx->d_num, ctx->d_cntout, ctx->n_ind);
+  cudaError_t err = clear_outputs(ctx);
+  if (err != cudaSuccess) return err;
   k_epilogue<<<dim3(ctx->n_tiles, 32), 256, 0, ctx->stream>>>(a);
+  return cudaGetLastError();
+}
+
+cudaError_t ngsd_launch_epilogue_int(ngsd_ctx *ctx, uint32_t n_splits, uint64_t const_cnt, bool in_kernel_cnt) {
+  EpiIntArgs a;
+  a.partials = reinterpret_cast<const int32_t *>(ctx->cur_partials);
+  a.split_w = ctx->cur_split_w;
+  a.pstride = in_kernel_cnt ? 2 * NGSD_TILE_ELEMS : NGSD_TILE_ELEMS;
+  a.in_kernel_cnt = in_kernel_cnt ? 1 : 0;
+  a.tiles = ctx->d_tiles;
+  a.out = ctx->d_out;
+  a.num = ctx->d_num;
+  a.cntout = ctx->d_cntout;
+  a.n_ind = ctx->n_ind;
+  a.const_cnt = const_cnt;
+  a.tot_sites = ctx->cfg.tot_sites;
+  a.n_splits = n_splits;
+  a.n_tiles = ctx->n_tiles;
+  a.evol_model = ctx->cfg.evol_model;
+  a.scale = ctx->int_scale;
+  cudaError_t err = clear_outputs(ctx);
+  if (err != cudaSuccess) return err;
+  k_epilogue_int<<<dim3(ctx->n_tiles, 16), 256, 0, ctx->stream>>>(a);
   return cudaGetLastError();
 }

@@ -30,7 +30,7 @@ struct FrontCfg {
   int call_geno;
   int pairwise_del;
   int planes;        // 3, or 2 (sum-to-one reduction, see ngsd_internal.h)
-  int int_path;      // called genotypes: write 2-bit codes for dist_imma.cu instead of FP64 planes
+  int int_path;      // called genotypes: write 2-bit codes for dist_umma.cu instead of FP64 planes
   double N_thresh, call_thresh;
   double score[9];
   ngsd_deferred *defer;      // knife-edge triples handed to the host's libm (api.cu resolve_deferred)
@@ -373,7 +373,7 @@ __device__ __noinline__ unsigned called_code_exact(int kind, int in_log, double 
   return code | (ok ? 0u : 4u);
 }
 
-// Front end of the integer path (called genotypes / genotype input; dist_imma.cu): same thread mapping as k_frontend,
+// Front end of the integer path (called genotypes / genotype input; dist_umma.cu): same thread mapping as k_frontend,
 // but the only outputs are 2 bits per individual-site (codes [RB][NW][4][128], 16 sites per word, 3 = missing or
 // padding) and the presence mask.  HBM-bound: 24 B (or 1 B of genotype code) read per individual-site, 0.4 B written.
 __global__ void __launch_bounds__(512, 2) k_frontend_codes(FrontCfg c, const double *__restrict__ raw, const int8_t *__restrict__ codes,

@@ -1,9 +1,10 @@
-// K3 mask_count: shared-site counts under --pairwise_del, bit-exact.
-//   cnt(i,j) = sum_s w_s * m_i(s) * m_j(s)        m = !miss_data (gen_func.cpp:862-868; skip at ngsDist.cpp:335-338,362)
+// K3 mask_count: the per-block shared-site counts of the bootstrap block cache under --pairwise_del, bit-exact.
+//   cnt_b(i,j) = sum_{s in block b} m_i(s) * m_j(s)        m = !miss_data (gen_func.cpp:862-868; skip at ngsDist.cpp:335-338,362)
 // as an integer AND+POPC "mask GEMM" over 64-site words (1-bit MMA is emulated on sm_100a, SURVEY App. D, so the
-// CUDA-core LOP3+POPC path is the native one).  Bootstrap weights are small integers: the host decomposes them into
-// level masks W_v = {s : w_s >= v}, so cnt = sum_v popc(m_i & m_j & W_v); the kernel just walks a list of
-// (word index, level-mask word) entries -- replicate 0 is the list of all words with all-ones masks.
+// CUDA-core LOP3+POPC path is the native one).  The host lists the sites of every block as (word index, mask word)
+// entries -- a block need not start or end on a word -- and split y of the grid counts block y.  The counts are kept
+// next to the per-block partial sums, and every replicate takes sum_b c[b] * cnt_b (epilogue.cu, dist_em.cu).  The
+// counts of a matrix without the cache come from the int8 tensor cores instead (dist_umma.cu, ngsd_launch_count_umma).
 #include "ngsd_internal.h"
 
 namespace {
@@ -15,17 +16,15 @@ struct CountArgs {
   const uint32_t *ent_word;
   const uint64_t *ent_mask;
   const ngsd_tile *tiles;
-  uint32_t *cnt;              // [n_pad][n_pad], zeroed
-  uint64_t NW, n_pad, n_entries;
-  uint32_t n_splits;
-  // bootstrap block cache: split y = source block y, entries [ent_begin[y], ent_begin[y+1]); the per-block counts are
-  // stored (no atomics) to cache[((y * n_tiles + tile) * 4 + quadrant) * 4096 + row * 64 + col]
+  uint64_t NW;
+  // split y = source block y, entries [ent_begin[y], ent_begin[y+1]); the per-block counts are stored (no atomics) to
+  // cache[((y * n_tiles + tile) * 4 + quadrant) * 4096 + row * 64 + col]
   const uint32_t *ent_begin;
   uint32_t *cache;
   uint32_t n_tiles;
 };
 
-// grid (4 * n_tiles, n_splits): a CTA owns the 64 x 64 quadrant `blockIdx.x & 3` of tile `blockIdx.x >> 2`.
+// grid (4 * n_tiles, n_blocks): a CTA owns the 64 x 64 quadrant `blockIdx.x & 3` of tile `blockIdx.x >> 2`.
 // block 128 = 8 x 16 threads, each 8 x 4 pairs (rows r*8+ty, cols c*16+tx).  Sized (4 warps x 64 registers, 8 KiB
 // shared memory) so that a CTA fits on an SM NEXT TO the persistent k_dist_dmma CTA (9 warps x 168 registers): the
 // counts run on the XU/ALU pipes in the shadow of the FP64 tensor contraction (api.cu launches K3 on a second stream
@@ -36,8 +35,7 @@ __global__ void __launch_bounds__(128, 8) k_mask_count(CountArgs a) {
   const ngsd_tile tl = a.tiles[blockIdx.x >> 2];
   const int qr = (blockIdx.x >> 1) & 1, qc = blockIdx.x & 1;
   const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-  const uint64_t e0 = a.ent_begin ? a.ent_begin[blockIdx.y] : (a.n_entries * blockIdx.y) / a.n_splits;
-  const uint64_t e1 = a.ent_begin ? a.ent_begin[blockIdx.y + 1] : (a.n_entries * (blockIdx.y + 1)) / a.n_splits;
+  const uint64_t e0 = a.ent_begin[blockIdx.y], e1 = a.ent_begin[blockIdx.y + 1];
   const uint64_t *ma = a.mask + (uint64_t) tl.ti * a.NW * 128 + qr * 64;
   const uint64_t *mb = a.mask + (uint64_t) tl.tj * a.NW * 128 + qc * 64;
   uint32_t acc[8][4];
@@ -75,56 +73,29 @@ __global__ void __launch_bounds__(128, 8) k_mask_count(CountArgs a) {
       }
     }
   }
-  if (a.cache) {
-    uint32_t *dst = a.cache + ((uint64_t) blockIdx.y * a.n_tiles * 4 + blockIdx.x) * 4096;
-#pragma unroll
-    for (int r = 0; r < 8; r++)
-#pragma unroll
-      for (int c = 0; c < 4; c++) dst[(r * 8 + ty) * 64 + c * 16 + tx] = acc[r][c];
-    return;
-  }
+  uint32_t *dst = a.cache + ((uint64_t) blockIdx.y * a.n_tiles * 4 + blockIdx.x) * 4096;
 #pragma unroll
   for (int r = 0; r < 8; r++)
 #pragma unroll
-    for (int c = 0; c < 4; c++) {
-      const uint64_t i = (uint64_t) tl.ti * 128 + qr * 64 + r * 8 + ty, j = (uint64_t) tl.tj * 128 + qc * 64 + c * 16 + tx;
-      if (acc[r][c]) atomicAdd(&a.cnt[i * a.n_pad + j], acc[r][c]);
-    }
+    for (int c = 0; c < 4; c++) dst[(r * 8 + ty) * 64 + c * 16 + tx] = acc[r][c];
 }
 
 }  // namespace
 
-cudaError_t ngsd_launch_mask_count(ngsd_ctx *ctx, uint64_t n_entries, cudaStream_t stream, uint32_t cache_blocks) {
-  cudaError_t e = cudaSuccess;
-  if (!cache_blocks) {
-    e = cudaMemsetAsync(ctx->d_cnt, 0, ctx->n_pad * ctx->n_pad * sizeof(uint32_t), stream);
-    if (e != cudaSuccess) return e;
-    if (n_entries == 0) return cudaSuccess;
-  }
+// one split per source block (gridDim.y <= 65535: checked by the caller)
+cudaError_t ngsd_launch_mask_count(ngsd_ctx *ctx, uint32_t n_blocks, cudaStream_t stream) {
   // same shared-memory carveout as k_dist_dmma, otherwise the SMs would have to drain before K3 could be placed on them
-  e = cudaFuncSetAttribute(k_mask_count, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  cudaError_t e = cudaFuncSetAttribute(k_mask_count, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (e != cudaSuccess) return e;
   CountArgs a;
   a.mask = ctx->mask;
   a.ent_word = ctx->d_ent_word;
   a.ent_mask = ctx->d_ent_mask;
   a.tiles = ctx->d_tiles;
-  a.cnt = ctx->d_cnt;
   a.NW = ctx->NW;
-  a.n_pad = ctx->n_pad;
-  a.n_entries = n_entries;
-  uint64_t want = (uint64_t) (8 * ctx->n_sm + 4 * ctx->n_tiles - 1) / (4 * ctx->n_tiles);
-  uint64_t maxs = (n_entries + kEB - 1) / kEB;
-  a.n_splits = (uint32_t) (want < 1 ? 1 : (want > maxs ? maxs : want));
-  if (a.n_splits > 65535) a.n_splits = 65535;
-  a.ent_begin = nullptr;
-  a.cache = nullptr;
+  a.ent_begin = ctx->d_ent_begin;
+  a.cache = ctx->d_cnt_cache;
   a.n_tiles = ctx->n_tiles;
-  if (cache_blocks) {          // one split per source block (gridDim.y <= 65535: checked by the caller)
-    a.n_splits = cache_blocks;
-    a.ent_begin = ctx->d_ent_begin;
-    a.cache = ctx->d_cnt_cache;
-  }
-  k_mask_count<<<dim3(4 * ctx->n_tiles, a.n_splits), 128, 0, stream>>>(a);
+  k_mask_count<<<dim3(4 * ctx->n_tiles, n_blocks), 128, 0, stream>>>(a);
   return cudaGetLastError();
 }

@@ -66,7 +66,7 @@ struct ngsd_ctx {
   double *d_cvec = nullptr;                    // [n_pad] weighted row sums of Cplane for the current matrix
   double *Apack = nullptr, *Bpack = nullptr;   // [RB][NC][3072]
   uint64_t *mask = nullptr;                    // [RB][NW][128] presence bits (1 = data present)
-  // called-genotype integer path (dist_imma.cu): 2-bit codes instead of FP64 planes
+  // called-genotype integer path (dist_umma.cu): 2-bit codes instead of FP64 planes
   bool int_path = false;
   uint32_t *codes = nullptr;                   // [RB][NW][4][128] 16 sites per word, code 3 = missing
   uint32_t *codes4 = nullptr;                  // [RB][NW][8][128] the same codes as PRMT selector nibbles, 8 sites per word (k_dist_umma)
@@ -183,7 +183,7 @@ struct ngsd_dist_plan {
   int grid;
 };
 cudaError_t ngsd_launch_dist_dmma(ngsd_ctx *ctx, const ngsd_dist_plan &p);
-cudaError_t ngsd_launch_mask_count(ngsd_ctx *ctx, uint64_t n_entries, cudaStream_t stream, uint32_t cache_blocks = 0);
+cudaError_t ngsd_launch_mask_count(ngsd_ctx *ctx, uint32_t n_blocks, cudaStream_t stream);   // per-block counts of the block cache
 struct ngsd_epilogue_args {
   uint32_t n_splits;
   uint64_t const_cnt;       // used when !pairwise_del
@@ -199,13 +199,10 @@ cudaError_t ngsd_launch_finish(ngsd_ctx *ctx, uint64_t const_cnt = 0);   // cons
 cudaError_t ngsd_launch_cvec(ngsd_ctx *ctx, bool weighted, uint64_t n_eff);
 cudaError_t ngsd_launch_deficit_fix(ngsd_ctx *ctx, bool weighted, uint64_t n_eff);
 cudaError_t ngsd_launch_epilogue_em(ngsd_ctx *ctx, uint32_t n_splits, uint64_t const_cnt, bool use_cnt);
-// K2c: called genotypes on the int8 tensor cores (dist_imma.cu)
+// K2c: called genotypes on the int8 tensor cores (dist_umma.cu, tcgen05)
 bool ngsd_int_lut(const double *score, bool pairwise_del, uint32_t lut[4], double *scale, int *max_byte);
-cudaError_t ngsd_launch_dist_imma(ngsd_ctx *ctx, uint32_t n_units, int grid, bool count);
-int ngsd_imma_ctas_per_sm();
-bool ngsd_use_umma();
-uint32_t ngsd_int_weight_cap(const ngsd_ctx *ctx);   // dist_umma.cu: largest site weight per weight layer of the integer path
-cudaError_t ngsd_launch_dist_umma(ngsd_ctx *ctx, uint32_t n_units, int grid, uint32_t pstride, bool count);   // dist_umma.cu (tcgen05)
+uint32_t ngsd_int_weight_cap(const ngsd_ctx *ctx);   // largest site weight per weight layer of the integer path
+cudaError_t ngsd_launch_dist_umma(ngsd_ctx *ctx, uint32_t n_units, int grid, uint32_t pstride, bool count);
 struct ngsd_count_umma_args {
   const uint32_t *split_begin;   // [n_splits + 1] positions in the word list
   uint32_t n_splits;
@@ -214,7 +211,7 @@ struct ngsd_count_umma_args {
   const uint32_t *word_ids, *word_layer;
 };
 cudaError_t ngsd_launch_count_umma(ngsd_ctx *ctx, const ngsd_count_umma_args &c);   // dist_umma.cu: --pairwise_del counts of the FP64 path
-cudaError_t ngsd_launch_epilogue_int(ngsd_ctx *ctx, uint32_t n_splits, uint64_t const_cnt, bool use_cnt, bool in_kernel_cnt);
+cudaError_t ngsd_launch_epilogue_int(ngsd_ctx *ctx, uint32_t n_splits, uint64_t const_cnt, bool in_kernel_cnt);   // epilogue.cu
 
 // ---- multi-GPU (comm.cu) ----
 extern "C" int ngsd_frontend_resolve(ngsd_ctx *ctx);      // api.cu: knife-edge triples -> host libm -> k_patch

@@ -1,4 +1,4 @@
-"""Called-genotype integer path (K2c dist_imma.cu, int8 tensor cores on 2-bit codes) through the C ABI.
+"""Called-genotype integer path (K2c dist_umma.cu, int8 tensor cores on 2-bit codes) through the C ABI.
 
 Everything is integer until num = acc / S, so against the oracle: cnt bit-exact everywhere; num and model-0 distances
 bit-exact with --pairwise_del or without missing data; 1e-9 otherwise (the reference's own sequential FP sum of the

@@ -12,7 +12,7 @@ import oracle
 
 
 def f_table(score, pairwise_del):
-    """f[c_i][c_j] for codes 0..2 and 3 = missing (what ngsd_int_lut tabulates, csrc/dist_imma.cu)."""
+    """f[c_i][c_j] for codes 0..2 and 3 = missing (what ngsd_int_lut tabulates, csrc/dist_umma.cu)."""
     s = np.asarray(score, dtype=np.float64).reshape(3, 3)
     p = np.zeros((4, 3))
     p[:3] = np.eye(3)

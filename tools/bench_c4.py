@@ -1,4 +1,4 @@
-"""Called-genotype integer path (K2c dist_imma) at a C4-like shape; development / profiling helper.
+"""Called-genotype integer path (K2c k_dist_umma) at a C4-like shape; development / profiling helper.
    N_IND, N_SITES, PDEL (0/1), MISS, FORCE_FP64 (1 = reserved bit 1: run the same data through the FP64 contraction)."""
 import os, sys, statistics, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

@@ -2,7 +2,7 @@
 // memory (K-major, no swizzle: 8-row x 16-byte core matrices), int32 accumulators in TMEM.
 //   1. correctness of the descriptor / layout conventions against a CPU product on random int8 data;
 //   2. issue rate of back-to-back accumulating MMAs (one CTA per SM) -> int8 tensor peak through the UMMA path,
-//      to compare with the 570 TMAC/s of mma.sync IMMA.16832 that K2c (dist_imma.cu) runs on.
+//      to compare with the 570 TMAC/s of mma.sync IMMA.16832 that the first K2c kernel (k_dist_imma, mma.sync; since removed) ran on.
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o tools/probe_utcimma tools/probe_utcimma.cu
 #include <cstdint>
 #include <cstdio>

@@ -26,8 +26,6 @@ C4="env N_SITES=50000 PDEL=0 python tools/bench_c4.py"
 $C4 > gpurun_out/${R}_plain_c4.log 2>&1 &&
 $NCU -k regex:k_dist_umma -s 1 -c 1 -f -o gpurun_out/${R}_dist_umma $C4 > gpurun_out/${R}_ncu8.log 2>&1
 echo "umma rc=$?"
-NGSD_IMMA_SYNC=1 $NCU -k regex:k_dist_imma -s 1 -c 1 -f -o gpurun_out/${R}_dist_imma $C4 > gpurun_out/${R}_ncu6.log 2>&1
-echo "imma rc=$?"
 $NCU -k regex:k_frontend_codes -s 2 -c 1 -f -o gpurun_out/${R}_frontend_codes $C4 > gpurun_out/${R}_ncu7.log 2>&1
 echo "frontend codes rc=$?"
 ls -la gpurun_out | grep $R
