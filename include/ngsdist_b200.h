@@ -183,8 +183,9 @@ NGSD_API int ngsd_distances_batch(ngsd_ctx *ctx, const uint32_t *block_counts, u
  *
  * Output-triangle tiles: after ngsd_set_tile_shard(rank, world) the context computes only the 128 x 128 upper-triangle
  * tiles dealt to `rank` (pairs of neighbouring tiles of one row block, each to the rank holding the fewest so far); every entry it does not own is written as 0 in out / num /
- * cnt, so an element-wise SUM over the ranks assembles the full matrices exactly (x + 0 == x).  Not available for the
- * per pair-site EM path.
+ * cnt, so an element-wise SUM over the ranks assembles the full matrices exactly (x + 0 == x).  On the per pair-site EM
+ * path (indep_geno == 0) the context contracts the 64 x 64 tiles inside the 128 x 128 tiles it owns; its bootstrap
+ * block cache then holds only those tiles.
  *
  * Sites: each rank creates its context for its own contiguous, block-aligned site range, calls ngsd_distances with
  * out == NULL (raw sums stay on the device), all-reduces the buffers returned by ngsd_device_results (num: FP64 sum,
@@ -210,8 +211,9 @@ NGSD_API int ngsd_comm_allgather_operands(ngsd_ctx *ctx, const uint64_t *site_be
  * num (FP64) -- and of cnt (uint64) only under --pairwise_del, otherwise cnt is the constant n_eff_total -- onto `root`,
  * which then runs the tail of gen_dist (ngsDist.cpp:372-401) and returns the matrix in out_host (NULL elsewhere). */
 NGSD_API int ngsd_comm_reduce_sites(ngsd_ctx *ctx, uint32_t root, uint64_t n_eff_total, double *out_host);
-/* Tile shards (ngsd_set_tile_shard(rank, world) on every rank): after ngsd_distances(out == NULL), the matrices are
- * assembled on `root` by an NCCL sum (entries a rank does not own are exact zeros).  with_num_cnt (the same value on
+/* Tile shards (ngsd_set_tile_shard(rank, world) on every rank), on every contraction path including the per pair-site
+ * EM: after ngsd_distances(out == NULL), the matrices are assembled on `root` by an NCCL sum (entries a rank does not
+ * own are exact zeros; a NaN matrix of the EM path keeps its NaNs only on the owned entries).  with_num_cnt (the same value on
  * every rank) also assembles the raw sums and counts; the host pointers are only read on `root`. */
 NGSD_API int ngsd_comm_reduce_tiles(ngsd_ctx *ctx, uint32_t root, int32_t with_num_cnt, double *out_host, double *num_host, uint64_t *cnt_host);
 NGSD_API int ngsd_comm_barrier(ngsd_ctx *ctx);

@@ -140,6 +140,33 @@ cudaError_t upload_tile_index(ngsd_ctx *ctx, const std::vector<ngsd_tile> &tiles
   return copy_sync(ctx, ctx->d_pairs, pairs.data(), pairs.size() * sizeof(uint32_t), cudaMemcpyHostToDevice);
 }
 
+// The 64 x 64 tiles of the per pair-site EM path (dist_em.cu) that lie in the owned 128 x 128 tiles: 64-tile (ti, tj)
+// belongs to 128-tile (ti / 2, tj / 2).  Listed in upper-triangle order (row by row) whether sharded or not, so that a
+// shard's CTAs keep the relative order of the whole matrix's; the slot index maps a 64-tile to its position in the list.
+cudaError_t upload_em_tiles(ngsd_ctx *ctx, const std::vector<ngsd_tile> &owned) {
+  const uint64_t n64 = (ctx->n_ind + NGSD_EM_EDGE - 1) / NGSD_EM_EDGE;
+  std::vector<uint8_t> own(ctx->RB * ctx->RB, 0);
+  for (const ngsd_tile &t : owned) own[(uint64_t) t.ti * ctx->RB + t.tj] = 1;
+  std::vector<uint32_t> list, slot(n64 * n64, 0xFFFFFFFFu);
+  for (uint64_t ti = 0; ti < n64; ti++)
+    for (uint64_t tj = ti; tj < n64; tj++)
+      if (own[(ti / 2) * ctx->RB + tj / 2]) {
+        slot[ti * n64 + tj] = (uint32_t) (list.size() / 2);
+        list.push_back((uint32_t) ti);
+        list.push_back((uint32_t) tj);
+      }
+  cudaError_t e = cudaSuccess;
+  if (!ctx->d_em_tiles) {
+    e = cudaMalloc((void **) &ctx->d_em_tiles, (n64 * (n64 + 1) + 2) * sizeof(uint32_t));
+    if (e == cudaSuccess) e = cudaMalloc((void **) &ctx->d_em_slot, slot.size() * sizeof(uint32_t));
+    if (e != cudaSuccess) return e;
+  }
+  ctx->em_n_tiles = (uint32_t) (list.size() / 2);
+  if (!list.empty()) e = copy_sync(ctx, ctx->d_em_tiles, list.data(), list.size() * sizeof(uint32_t), cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) return e;
+  return copy_sync(ctx, ctx->d_em_slot, slot.data(), slot.size() * sizeof(uint32_t), cudaMemcpyHostToDevice);
+}
+
 }  // namespace
 
 extern "C" {
@@ -283,6 +310,7 @@ int ngsd_create(const ngsd_cfg *cfg, ngsd_ctx **out) {
   CREATE_CUDA(dev_alloc(&ctx->d_tiles, tiles.size()));
   CREATE_CUDA(copy_sync(ctx, ctx->d_tiles, tiles.data(), tiles.size() * sizeof(ngsd_tile), cudaMemcpyHostToDevice));
   CREATE_CUDA(upload_tile_index(ctx, tiles));
+  if (!cfg->indep_geno) CREATE_CUDA(upload_em_tiles(ctx, tiles));
 #undef CREATE_CUDA
   *out = ctx;
   return NGSD_OK;
@@ -302,6 +330,7 @@ int ngsd_destroy(ngsd_ctx *ctx) {
   cudaFree(ctx->d_ent_word); cudaFree(ctx->d_ent_mask); cudaFree(ctx->d_cnt); cudaFree(ctx->d_split_begin); cudaFree(ctx->d_split_scale); cudaFree(ctx->d_sched);
   cudaFree(ctx->d_out); cudaFree(ctx->d_num); cudaFree(ctx->d_cntout);
   cudaFree(ctx->d_cache); cudaFree(ctx->d_cnt_cache); cudaFree(ctx->d_ent_begin); cudaFree(ctx->d_tile_index); cudaFree(ctx->d_pairs);
+  cudaFree(ctx->d_em_tiles); cudaFree(ctx->d_em_slot);
   cudaFree(ctx->codes); cudaFree(ctx->codes4); cudaFree(ctx->d_wsite); cudaFree(ctx->d_word_layer); cudaFree(ctx->d_word_ids);
   cudaFree(ctx->d_defer); cudaFree(ctx->d_defer_n); cudaFree(ctx->d_blank);
   cudaFree(ctx->d_def_rowptr); cudaFree(ctx->d_def_rowind); cudaFree(ctx->d_def_site); cudaFree(ctx->d_def_delta); cudaFree(ctx->d_fix);
@@ -1069,6 +1098,7 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
       NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_num, 0, n2z * sizeof(double), ctx->stream));
       NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_cntout, 0, n2z * sizeof(uint64_t), ctx->stream));
       NGSD_CUDA(ctx, ngsd_launch_finish(ctx));
+      if (em_path) NGSD_CUDA(ctx, ngsd_clear_unowned(ctx));
       rc0 = copy_out(ctx, out, num_opt, cnt_opt);
       if (rc0) return rc0;
       ctx->timing = ngsd_timing();
@@ -1092,6 +1122,7 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
       const uint64_t n2z = ctx->n_ind * ctx->n_ind;
       NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_num, 0xFF, n2z * sizeof(double), ctx->stream));   // all-ones = the negative quiet NaN x86 gives 0/0
       NGSD_CUDA(ctx, ngsd_launch_finish(ctx, n_eff));
+      NGSD_CUDA(ctx, ngsd_clear_unowned(ctx));
       rc0 = copy_out(ctx, out, num_opt, cnt_opt);
       if (rc0) return rc0;
       ctx->timing = ngsd_timing();
@@ -1125,11 +1156,11 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
   // weighted split reduction in the epilogue -- ~100x less work per replicate at C3 (SURVEY §7 design option (a)).
   // It needs blocks that are whole site chunks and room for n_blocks partials; otherwise (and with ngsd_cfg.reserved
   // bit 2, which benchmarks of the per-replicate weighted contraction set) the replicate is contracted directly.
-  const uint64_t em_ld = em_path ? ngsd_em_ld(ctx) : 0;
+  const uint64_t em_split_doubles = em_path ? ngsd_em_split_doubles(ctx) : 0;
   bool use_cache = false, build_cache = false;
   if (weighted && !(ctx->cfg.reserved & 4) && block_size % SC == 0 && n_blocks >= 2 &&
       n_blocks < 0x7fffffffull / std::max<uint32_t>(ctx->n_tiles, 1)) {
-    const uint64_t need = em_path ? n_blocks * em_ld * em_ld : n_blocks * (uint64_t) ctx->n_tiles * NGSD_TILE_ELEMS;
+    const uint64_t need = em_path ? n_blocks * em_split_doubles : n_blocks * (uint64_t) ctx->n_tiles * NGSD_TILE_ELEMS;
     // with --pairwise_del the per-block shared-site counts are cached next to the sums (one K3 split per block)
     const uint64_t need_cnt = (ctx->cfg.pairwise_del && n_blocks <= 65535) ? n_blocks * (uint64_t) ctx->n_tiles * NGSD_TILE_ELEMS : 0;
     if (ctx->cache_valid && ctx->cache_blocks == n_blocks && ctx->cache_bs == block_size) {
@@ -1281,7 +1312,7 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
   plan.grid = (int) std::min<uint64_t>(plan.grid, plan.n_units);
   if (em_path) {
     em_splits = use_cache ? (uint32_t) n_blocks : ngsd_em_splits(ctx, plan.n_chunks);
-    plan.n_units = (uint32_t) (((uint64_t) em_splits * em_ld * em_ld + NGSD_TILE_ELEMS - 1) / NGSD_TILE_ELEMS);   // workspace slots
+    plan.n_units = (uint32_t) (((uint64_t) em_splits * em_split_doubles + NGSD_TILE_ELEMS - 1) / NGSD_TILE_ELEMS);   // workspace slots
   }
   if (splits.size() > ctx->split_cap) {
     cudaFree(ctx->d_split_begin);
@@ -1430,7 +1461,6 @@ int ngsd_set_tile_shard(ngsd_ctx *ctx, uint32_t rank, uint32_t world) {
   if (!ctx) return NGSD_ERR_ARG;
   if (!ctx->kids.empty()) { ngsd_set_error(ctx, "a multi-GPU context deals the tiles to its GPUs itself"); return NGSD_ERR_ARG; }
   if (world == 0 || rank >= world) { ngsd_set_error(ctx, "invalid tile shard %u of %u", rank, world); return NGSD_ERR_ARG; }
-  if (!ctx->cfg.indep_geno && world > 1) { ngsd_set_error(ctx, "tile sharding is not available on the per pair-site EM path"); return NGSD_ERR_ARG; }
   NGSD_CUDA(ctx, cudaSetDevice(ctx->device));
   // the unit of ownership is a PAIR of neighbouring tiles of one row block (the odd tile of a row alone): dist_umma.cu
   // contracts such pairs with one shared A operand, so a shard keeps them together
@@ -1451,6 +1481,7 @@ int ngsd_set_tile_shard(ngsd_ctx *ctx, uint32_t rank, uint32_t world) {
   for (auto &t : mine) ctx->n_diag_tiles += (t.ti == t.tj);
   if (!mine.empty()) NGSD_CUDA(ctx, copy_sync(ctx, ctx->d_tiles, mine.data(), mine.size() * sizeof(ngsd_tile), cudaMemcpyHostToDevice));
   NGSD_CUDA(ctx, upload_tile_index(ctx, mine));
+  if (!ctx->cfg.indep_geno) NGSD_CUDA(ctx, upload_em_tiles(ctx, mine));   // the EM path contracts the 64 x 64 tiles inside them
   ctx->shard_rank = rank;
   ctx->shard_world = world;
   ctx->cache_valid = false;

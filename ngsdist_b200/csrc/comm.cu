@@ -572,10 +572,6 @@ int ngsd_group_distances(ngsd_ctx *parent, const uint32_t *block_counts, uint64_
     if (rc) return rc;
     const uint64_t n_eff = weighted ? n_blocks * block_size : parent->n_sites;
     rc = reduce_sites_impl(parent, parent->kids, 0, n_eff, out, num_opt, cnt_opt);
-  } else if (!parent->cfg.indep_geno) {
-    // the per pair-site EM has no tile sharding: one matrix runs on the first GPU (replicates still shard, see batch)
-    rc = ngsd_distances(root, block_counts, n_blocks, block_size, out, num_opt, cnt_opt);
-    if (rc) ngsd_set_error(parent, "%s", root->err);
   } else {
     if (!parent->kids_tile_sharded) {
       rc = for_each_kid(parent, [&](ngsd_ctx *k, uint32_t g) { return ngsd_set_tile_shard(k, g, N); });
@@ -650,7 +646,13 @@ int ngsd_group_distances_batch(ngsd_ctx *ctx, const uint32_t *block_counts, uint
     int rc = ngsd_group_frontend(parent);
     if (rc) return rc;
   }
-  if (parent->shard_mode == NGSD_SHARD_SITES) {   // every replicate needs every GPU
+  // The per pair-site EM with the bootstrap block cache (blocks of whole site chunks, at least two, cache not turned off
+  // by ngsd_cfg.reserved bit 2): every replicate on every GPU, each on its own tiles, so that each GPU builds the cache of
+  // its tiles once.  The kids stay tile-sharded from matrix 0 on: ngsd_set_tile_shard would drop the cache.  Otherwise
+  // whole replicates are dealt to the GPUs, which at one site per block is the better use of them.
+  const ngsd_ctx *k0 = parent->kids[0];
+  const bool em_tiles = !parent->cfg.indep_geno && block_size % (uint64_t) k0->sc == 0 && n_blocks >= 2 && !(parent->cfg.reserved & 4);
+  if (parent->shard_mode == NGSD_SHARD_SITES || em_tiles) {   // every replicate needs every GPU
     ngsd_timing acc = ngsd_timing();
     for (uint64_t r = 0; r < n_rep; r++) {
       int rc = ngsd_group_distances(parent, block_counts + r * n_blocks, n_blocks, block_size, out + r * n2, nullptr, nullptr);

@@ -33,7 +33,7 @@
 
 namespace {
 
-constexpr int kEdge = 64;                       // pairs tile: 64 rows x 64 columns
+constexpr int kEdge = NGSD_EM_EDGE;             // pairs tile: 64 rows x 64 columns
 constexpr int kIter = 50;                       // maxIter of em2 (ngsDist.cpp:349)
 constexpr int kThreads = 512;                   // 16 warps: the kernel is bound by FP64 / shared-memory latency
 constexpr double kExpTol = 1.0010005001667084;  // e^0.001 (tole of ngsDist.cpp:349)
@@ -45,9 +45,10 @@ struct EmArgs {
   const double *Apack;          // packed posterior planes (A operand of dist_dmma, 3-plane layout)
   const double *weights;        // [NC*8] per-site bootstrap weights or nullptr
   const uint32_t *chunk_ids;    // active chunk list or nullptr (identity)
-  double *partials;             // [n_splits][ld][ld]
-  uint64_t NC, n_sites, ld;
-  uint32_t n_chunks, n_splits, n64, n_tiles;
+  const uint32_t *tiles;        // [n_tiles][2] (ti, tj) of the owned 64 x 64 tiles
+  double *partials;             // [n_splits][n_tiles][64][64]
+  uint64_t NC, n_sites;
+  uint32_t n_chunks, n_splits, n_tiles;
   double K[9];                  // score folded with a2 = 1 - a0 - a1, b2 = 1 - b0 - b1 (see pair_term)
 };
 
@@ -252,7 +253,7 @@ __device__ __forceinline__ void pair_group26(const double *tb, const int *meta, 
   }
 }
 
-// grid = n_splits * n_tiles (split-major); block 512
+// grid = n_splits * n_tiles (split-major) over the owned tile list; block 512
 template <bool WEIGHTED>
 __global__ void __launch_bounds__(kThreads, 1) k_dist_em3(EmArgs a) {
   extern __shared__ __align__(16) double sm[];
@@ -260,10 +261,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_em3(EmArgs a) {
   int *metab = reinterpret_cast<int *>(sm + k3_Doubles);                 // [2 sites][tstar, lo, hi, valid][128]
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const uint32_t q = blockIdx.x / a.n_tiles;
-  uint32_t t_lin = blockIdx.x - q * a.n_tiles, ti = 0;
-  while (t_lin >= a.n64 - ti) { t_lin -= a.n64 - ti; ti++; }
-  const uint32_t tj = ti + t_lin;
+  const uint32_t q = blockIdx.x / a.n_tiles, slot = blockIdx.x - q * a.n_tiles;
+  const uint32_t ti = a.tiles[2 * slot], tj = a.tiles[2 * slot + 1];
   const bool diag = ti == tj;
   const uint32_t c0 = (uint32_t) (((uint64_t) q * a.n_chunks) / a.n_splits);
   const uint32_t c1 = (uint32_t) (((uint64_t) (q + 1) * a.n_chunks) / a.n_splits);
@@ -354,18 +353,20 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_em3(EmArgs a) {
     }
   }
 
+  double *dst = a.partials + ((uint64_t) q * a.n_tiles + slot) * (kEdge * kEdge);
 #pragma unroll
   for (int k = 0; k < 4; k++)
 #pragma unroll
     for (int h = 0; h < 2; h++) {
       const int r = warp + 16 * (k & 1) + 32 * (k >> 1), cc = h * 32 + lane;
-      const uint64_t i = (uint64_t) ti * kEdge + r, j = (uint64_t) tj * kEdge + cc;
-      a.partials[((uint64_t) q * a.ld + i) * a.ld + j] = (i < j) ? acc[(k >> 1) * 4 + (k & 1) * 2 + h] : 0.0;
+      dst[r * kEdge + cc] = (!diag || r < cc) ? acc[(k >> 1) * 4 + (k & 1) * 2 + h] : 0.0;
     }
 }
 
 struct EmEpiArgs {
-  const double *partials;
+  const double *partials;     // [n_splits][n_tiles64][64][64]
+  const uint32_t *slot;       // [n64][n64] position of the 64 x 64 tile (ti, tj) in the owned list (0xFFFFFFFF: not owned)
+  uint32_t n64, n_tiles64;
   const double *split_w;      // [n_splits] weight of each split (bootstrap block cache) or nullptr
   const uint32_t *cnt;        // [n_pad][n_pad] or nullptr
   const uint32_t *cnt_cache;  // per-block counts [n_splits][n_tiles128][4][64][64] (bootstrap block cache) or nullptr
@@ -373,12 +374,13 @@ struct EmEpiArgs {
   uint32_t n_tiles128, RB;
   double *out, *num;
   uint64_t *cntout;
-  uint64_t n_ind, n_pad, ld, const_cnt, tot_sites;
+  uint64_t n_ind, n_pad, const_cnt, tot_sites;
   uint32_t n_splits;
   int evol_model;
 };
 
-// tail of gen_dist (ngsDist.cpp:372-401) for the EM path; fixed-order reduction over the K splits
+// tail of gen_dist (ngsDist.cpp:372-401) for the EM path; fixed-order reduction over the K splits.  Pairs of tiles a
+// tile shard does not own are left as ngsd_clear_outputs set them (0).
 __global__ void __launch_bounds__(256) k_epilogue_em(EmEpiArgs a) {
   const uint64_t j = (uint64_t) blockIdx.x * 16 + (threadIdx.x & 15), i = (uint64_t) blockIdx.y * 16 + (threadIdx.x >> 4);
   if (i >= a.n_ind || j >= a.n_ind) return;
@@ -389,14 +391,18 @@ __global__ void __launch_bounds__(256) k_epilogue_em(EmEpiArgs a) {
     return;
   }
   if (i > j) return;
+  const uint32_t s = a.slot[(i / kEdge) * a.n64 + j / kEdge];
+  if (s == 0xFFFFFFFFu) return;
+  const double *src = a.partials + (uint64_t) s * (kEdge * kEdge) + (i % kEdge) * kEdge + j % kEdge;
+  const uint64_t stride = (uint64_t) a.n_tiles64 * (kEdge * kEdge);
   double num = 0;
   if (a.split_w) {
     for (uint32_t q = 0; q < a.n_splits; q++) {
       const double w = a.split_w[q];
-      if (w != 0.0) num += w * a.partials[((uint64_t) q * a.ld + i) * a.ld + j];
+      if (w != 0.0) num += w * src[(uint64_t) q * stride];
     }
   } else {
-    for (uint32_t q = 0; q < a.n_splits; q++) num += a.partials[((uint64_t) q * a.ld + i) * a.ld + j];
+    for (uint32_t q = 0; q < a.n_splits; q++) num += src[(uint64_t) q * stride];
   }
   uint64_t cnt = a.cnt ? (uint64_t) a.cnt[i * a.n_pad + j] : a.const_cnt;
   if (a.cnt_cache) {          // sum_b c[b] * cnt_b(i,j) from the 128 x 128 tile list of K3 (row-major upper triangle in bands)
@@ -423,13 +429,14 @@ uint64_t em_n64(const ngsd_ctx *ctx) { return (ctx->n_ind + kEdge - 1) / kEdge; 
 
 }  // namespace
 
-uint64_t ngsd_em_ld(const ngsd_ctx *ctx) { return em_n64(ctx) * kEdge; }
+uint64_t ngsd_em_split_doubles(const ngsd_ctx *ctx) { return (uint64_t) ctx->em_n_tiles * (kEdge * kEdge); }
 
+// planned from the tiles this context owns, so that a tile shard still fills the SMs
 uint32_t ngsd_em_splits(const ngsd_ctx *ctx, uint32_t n_chunks) {
-  const uint64_t n64 = em_n64(ctx), tiles = n64 * (n64 + 1) / 2, ld = n64 * kEdge;
+  const uint64_t tiles = std::max<uint32_t>(ctx->em_n_tiles, 1);
   uint64_t want = ((uint64_t) 8 * ctx->n_sm + tiles - 1) / tiles;             // ~8 units per SM: short tail, 1 CTA per SM
   const uint64_t maxs = std::max<uint64_t>(1, n_chunks / 2);
-  const uint64_t cap_mem = std::max<uint64_t>(1, ((uint64_t) 2 << 30) / (ld * ld * 8));
+  const uint64_t cap_mem = std::max<uint64_t>(1, ((uint64_t) 2 << 30) / (tiles * kEdge * kEdge * 8));
   want = std::max<uint64_t>(1, std::min(std::min(want, maxs), cap_mem));
   return (uint32_t) std::min<uint64_t>(want, 65535);
 }
@@ -448,14 +455,13 @@ cudaError_t ngsd_launch_dist_em(ngsd_ctx *ctx, uint32_t n_chunks, uint32_t n_spl
   a.Apack = ctx->Apack;
   a.weights = weighted ? ctx->d_weights : nullptr;
   a.chunk_ids = weighted ? ctx->d_chunk_ids : nullptr;
+  a.tiles = ctx->d_em_tiles;
   a.partials = ctx->cur_partials;
   a.NC = ctx->NC;
   a.n_sites = ctx->n_sites;
   a.n_chunks = n_chunks;
   a.n_splits = n_splits;
-  a.n64 = (uint32_t) em_n64(ctx);
-  a.n_tiles = a.n64 * (a.n64 + 1) / 2;
-  a.ld = (uint64_t) a.n64 * kEdge;
+  a.n_tiles = ctx->em_n_tiles;
   const double *D = ctx->cfg.score;   // D[g1 * 3 + g2], g1 = genotype of the row individual (i1 < i2, ngsDist.cpp:351-353)
   a.K[0] = D[8];
   a.K[1] = D[2] - D[8];
@@ -478,6 +484,9 @@ cudaError_t ngsd_launch_dist_em(ngsd_ctx *ctx, uint32_t n_chunks, uint32_t n_spl
 cudaError_t ngsd_launch_epilogue_em(ngsd_ctx *ctx, uint32_t n_splits, uint64_t const_cnt, bool use_cnt) {
   EmEpiArgs a;
   a.partials = ctx->cur_partials;
+  a.slot = ctx->d_em_slot;
+  a.n64 = (uint32_t) em_n64(ctx);
+  a.n_tiles64 = ctx->em_n_tiles;
   a.split_w = ctx->cur_split_w;
   a.cnt = (use_cnt && !ctx->cur_cnt_cache) ? ctx->d_cnt : nullptr;
   a.cnt_cache = use_cnt ? ctx->cur_cnt_cache : nullptr;
@@ -489,11 +498,14 @@ cudaError_t ngsd_launch_epilogue_em(ngsd_ctx *ctx, uint32_t n_splits, uint64_t c
   a.cntout = ctx->d_cntout;
   a.n_ind = ctx->n_ind;
   a.n_pad = ctx->n_pad;
-  a.ld = ngsd_em_ld(ctx);
   a.const_cnt = const_cnt;
   a.tot_sites = ctx->cfg.tot_sites;
   a.n_splits = n_splits;
   a.evol_model = ctx->cfg.evol_model;
+  if (ctx->shard_world > 1) {
+    cudaError_t e = ngsd_clear_outputs(ctx);
+    if (e != cudaSuccess) return e;
+  }
   const uint32_t n16 = (uint32_t) ((ctx->n_ind + 15) / 16);
   k_epilogue_em<<<dim3(n16, n16), 256, 0, ctx->stream>>>(a);
   return cudaGetLastError();

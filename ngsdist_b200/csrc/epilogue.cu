@@ -214,9 +214,22 @@ __global__ void __launch_bounds__(256) k_deficit_fix(const uint32_t *__restrict_
   }
 }
 
+// Entries (i, j) and (j, i) whose 128 x 128 tile a tile shard does not own -> 0, the diagonal of such tiles included.
+__global__ void k_clear_unowned(const uint32_t *__restrict__ tile_index, uint64_t RB, double *out, double *num, uint64_t *cnt, uint64_t n) {
+  const uint64_t idx = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n * n) return;
+  const uint64_t i = idx / n, j = idx - i * n, lo = (i < j ? i : j) / NGSD_TILE, hi = (i < j ? j : i) / NGSD_TILE;
+  if (tile_index[lo * RB + hi] != 0xFFFFFFFFu) return;
+  out[idx] = 0.0;
+  num[idx] = 0.0;
+  cnt[idx] = 0;
+}
+
+}  // namespace
+
 // Before an epilogue: zero the diagonal, and with a tile shard every entry, since the tiles of other ranks must read as
 // 0 (ngsd_set_tile_shard).
-cudaError_t clear_outputs(ngsd_ctx *ctx) {
+cudaError_t ngsd_clear_outputs(ngsd_ctx *ctx) {
   if (ctx->shard_world > 1) {
     const uint64_t n2 = ctx->n_ind * ctx->n_ind;
     cudaError_t e = cudaMemsetAsync(ctx->d_out, 0, n2 * sizeof(double), ctx->stream);
@@ -228,7 +241,14 @@ cudaError_t clear_outputs(ngsd_ctx *ctx) {
   return cudaGetLastError();
 }
 
-}  // namespace
+// After a result that was written for every pair (the early-outs of ngsd_distances): with a tile shard, keep only the
+// tiles this context owns, so that the sum over the ranks is the whole-matrix result.
+cudaError_t ngsd_clear_unowned(ngsd_ctx *ctx) {
+  if (ctx->shard_world <= 1) return cudaSuccess;
+  const uint64_t n2 = ctx->n_ind * ctx->n_ind;
+  k_clear_unowned<<<(unsigned) ((n2 + 255) / 256), 256, 0, ctx->stream>>>(ctx->d_tile_index, ctx->RB, ctx->d_out, ctx->d_num, ctx->d_cntout, ctx->n_ind);
+  return cudaGetLastError();
+}
 
 cudaError_t ngsd_launch_deficit_fix(ngsd_ctx *ctx, bool weighted, uint64_t n_eff) {
   cudaError_t e = cudaMemsetAsync(ctx->d_fix, 0, ctx->n_ind * ctx->n_ind * sizeof(double), ctx->stream);
@@ -269,7 +289,7 @@ cudaError_t ngsd_launch_epilogue(ngsd_ctx *ctx, const ngsd_epilogue_args &e) {
   a.n_splits = e.n_splits;
   a.n_tiles = ctx->n_tiles;
   a.evol_model = ctx->cfg.evol_model;
-  cudaError_t err = clear_outputs(ctx);
+  cudaError_t err = ngsd_clear_outputs(ctx);
   if (err != cudaSuccess) return err;
   k_epilogue<<<dim3(ctx->n_tiles, 32), 256, 0, ctx->stream>>>(a);
   return cudaGetLastError();
@@ -292,7 +312,7 @@ cudaError_t ngsd_launch_epilogue_int(ngsd_ctx *ctx, uint32_t n_splits, uint64_t 
   a.n_tiles = ctx->n_tiles;
   a.evol_model = ctx->cfg.evol_model;
   a.scale = ctx->int_scale;
-  cudaError_t err = clear_outputs(ctx);
+  cudaError_t err = ngsd_clear_outputs(ctx);
   if (err != cudaSuccess) return err;
   k_epilogue_int<<<dim3(ctx->n_tiles, 16), 256, 0, ctx->stream>>>(a);
   return cudaGetLastError();

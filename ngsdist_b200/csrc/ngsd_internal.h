@@ -105,6 +105,9 @@ struct ngsd_ctx {
   // distance workspaces (allocated lazily)
   ngsd_tile *d_tiles = nullptr; uint32_t n_tiles = 0;
   uint32_t *d_tile_index = nullptr;            // [RB][RB] position of tile (ti, tj) in d_tiles (0xFFFFFFFF: not owned)
+  // the per pair-site EM path (dist_em.cu) works on 64 x 64 tiles: the owned ones (those inside an owned 128 x 128 tile)
+  uint32_t *d_em_tiles = nullptr; uint32_t em_n_tiles = 0;   // [em_n_tiles][2] (ti, tj) in upper-triangle order
+  uint32_t *d_em_slot = nullptr;               // [n64][n64] position of 64-tile (ti, tj) in d_em_tiles (0xFFFFFFFF: not owned)
   uint32_t *d_pairs = nullptr; uint32_t n_pairs = 0;   // [n_pairs][2] positions of two tiles of one row block (second 0xFFFFFFFF: single); dist_umma.cu
   double *d_partials = nullptr; uint64_t partial_slots = 0;
   // what the contraction launchers write and the epilogues read: d_partials, or the per-block cache below
@@ -192,13 +195,16 @@ struct ngsd_epilogue_args {
 cudaError_t ngsd_launch_epilogue(ngsd_ctx *ctx, const ngsd_epilogue_args &a);
 size_t ngsd_dist_smem_bytes();
 // K2b: per pair-site EM path (indep_geno == 0)
+constexpr int NGSD_EM_EDGE = 64;               // pair tile edge of k_dist_em3
 uint32_t ngsd_em_splits(const ngsd_ctx *ctx, uint32_t n_chunks);
-uint64_t ngsd_em_ld(const ngsd_ctx *ctx);     // leading dimension of the EM partials (64-row tiles)
+uint64_t ngsd_em_split_doubles(const ngsd_ctx *ctx);   // EM partials of one K split: one 64 x 64 slot per owned tile
 cudaError_t ngsd_launch_dist_em(ngsd_ctx *ctx, uint32_t n_chunks, uint32_t n_splits, bool weighted);
 cudaError_t ngsd_launch_finish(ngsd_ctx *ctx, uint64_t const_cnt = 0);   // const_cnt > 0: cnt is that constant (no --pairwise_del)
 cudaError_t ngsd_launch_cvec(ngsd_ctx *ctx, bool weighted, uint64_t n_eff);
 cudaError_t ngsd_launch_deficit_fix(ngsd_ctx *ctx, bool weighted, uint64_t n_eff);
 cudaError_t ngsd_launch_epilogue_em(ngsd_ctx *ctx, uint32_t n_splits, uint64_t const_cnt, bool use_cnt);
+cudaError_t ngsd_clear_outputs(ngsd_ctx *ctx);       // epilogue.cu: zero diagonal; with a tile shard, every entry
+cudaError_t ngsd_clear_unowned(ngsd_ctx *ctx);       // epilogue.cu: with a tile shard, zero every entry of a tile it does not own
 // K2c: called genotypes on the int8 tensor cores (dist_umma.cu, tcgen05)
 bool ngsd_int_lut(const double *score, bool pairwise_del, uint32_t lut[4], double *scale, int *max_byte);
 uint32_t ngsd_int_weight_cap(const ngsd_ctx *ctx);   // largest site weight per weight layer of the integer path
