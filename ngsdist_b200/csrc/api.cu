@@ -52,7 +52,8 @@ std::vector<ngsd_tile> make_tiles(uint32_t RB) {
 // K-split boundaries (in positions of the active chunk list) for the dynamically scheduled (split, tile) units of
 // k_dist_dmma.  Two unit sizes: ~8 "main" units per CTA cover the first 84 % of the chunks, then units a quarter of
 // that size fill the tail so that the CTAs finish within one small unit of each other.  `cost_tiles` is the tile
-// count in full-tile equivalents (a diagonal tile costs 136/256).  The partial workspace (128 KiB per unit) is
+// count in full-tile equivalents (a diagonal tile costs 136/256; edge tiles count as full ones, so the splits do not
+// depend on how k_dist_dmma contracts them).  The partial workspace (128 KiB per unit) is
 // capped at 6 GiB.
 std::vector<uint32_t> plan_splits(uint32_t n_chunks, uint32_t n_tiles, double cost_tiles, int grid) {
   std::vector<uint32_t> b;
@@ -108,6 +109,26 @@ int copy_out(ngsd_ctx *ctx, double *out, double *num_opt, uint64_t *cnt_opt) {
   if (num_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(num_opt, ctx->d_num, n2 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
   if (cnt_opt) NGSD_CUDA(ctx, cudaMemcpyAsync(cnt_opt, ctx->d_cntout, n2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
   NGSD_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return NGSD_OK;
+}
+
+// Host-to-device copy of a small host list, queued on ctx->stream from the pinned scratch h_lists: from pageable memory
+// the call could wait for the work queued before it, and the replicate loop enqueues the next matrix while the device
+// still runs the last one.  The scratch is rewritten once ctx->ev_pin has passed (distances_enqueue resets it); growing
+// it first drains the stream, so no queued copy reads a freed buffer.
+int upload_list(ngsd_ctx *ctx, void *dst, const void *src, uint64_t bytes) {
+  if (bytes == 0) return NGSD_OK;
+  uint64_t at = (ctx->h_lists_used + 15) & ~(uint64_t) 15;
+  if (at + bytes > ctx->h_lists_bytes) {
+    NGSD_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    int rc = ensure_pinned(ctx, &ctx->h_lists, &ctx->h_lists_bytes, std::max<uint64_t>(2 * ctx->h_lists_bytes, bytes + 4096));
+    if (rc) return rc;
+    at = 0;
+  }
+  char *h = (char *) ctx->h_lists + at;
+  memcpy(h, src, bytes);
+  NGSD_CUDA(ctx, cudaMemcpyAsync(dst, h, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  ctx->h_lists_used = at + bytes;
   return NGSD_OK;
 }
 
@@ -251,8 +272,11 @@ int ngsd_create(const ngsd_cfg *cfg, ngsd_ctx **out) {
   CREATE_CUDA(cudaStreamCreateWithFlags(&ctx->aux_stream, cudaStreamNonBlocking));
   CREATE_CUDA(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
   CREATE_CUDA(cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming));
-  for (auto &e : ctx->ev) CREATE_CUDA(cudaEventCreate(&e));
+  for (auto &set : ctx->ev_sets)
+    for (auto &e : set) CREATE_CUDA(cudaEventCreate(&e));
+  CREATE_CUDA(cudaEventCreateWithFlags(&ctx->ev_pin, cudaEventDisableTiming));
   for (int b = 0; b < 2; b++) {
+    CREATE_CUDA(cudaEventCreateWithFlags(&ctx->ev_copied[b], cudaEventDisableTiming));
     CREATE_CUDA(cudaEventCreateWithFlags(&ctx->stage_free[b], cudaEventDisableTiming));
     CREATE_CUDA(cudaEventCreateWithFlags(&ctx->stage_ready[b], cudaEventDisableTiming));
   }
@@ -307,6 +331,7 @@ int ngsd_create(const ngsd_cfg *cfg, ngsd_ctx **out) {
   std::vector<ngsd_tile> tiles = make_tiles((uint32_t) ctx->RB);
   ctx->n_tiles = (uint32_t) tiles.size();
   ctx->n_diag_tiles = (uint32_t) ctx->RB;
+  ctx->n_edge_tiles = ngsd_edge_c8(ctx->n_ind) ? (uint32_t) ctx->RB - 1 : 0;
   CREATE_CUDA(dev_alloc(&ctx->d_tiles, tiles.size()));
   CREATE_CUDA(copy_sync(ctx, ctx->d_tiles, tiles.data(), tiles.size() * sizeof(ngsd_tile), cudaMemcpyHostToDevice));
   CREATE_CUDA(upload_tile_index(ctx, tiles));
@@ -328,7 +353,7 @@ int ngsd_destroy(ngsd_ctx *ctx) {
   cudaFree(ctx->stage_dev[0]); cudaFree(ctx->stage_dev[1]);
   cudaFree(ctx->d_tiles); cudaFree(ctx->d_partials); cudaFree(ctx->d_weights); cudaFree(ctx->d_chunk_ids);
   cudaFree(ctx->d_ent_word); cudaFree(ctx->d_ent_mask); cudaFree(ctx->d_cnt); cudaFree(ctx->d_split_begin); cudaFree(ctx->d_split_scale); cudaFree(ctx->d_sched);
-  cudaFree(ctx->d_out); cudaFree(ctx->d_num); cudaFree(ctx->d_cntout);
+  cudaFree(ctx->d_out); cudaFree(ctx->d_out_alt); cudaFree(ctx->d_num); cudaFree(ctx->d_cntout);
   cudaFree(ctx->d_cache); cudaFree(ctx->d_cnt_cache); cudaFree(ctx->d_ent_begin); cudaFree(ctx->d_tile_index); cudaFree(ctx->d_pairs);
   cudaFree(ctx->d_em_tiles); cudaFree(ctx->d_em_slot);
   cudaFree(ctx->codes); cudaFree(ctx->codes4); cudaFree(ctx->d_wsite); cudaFree(ctx->d_word_layer); cudaFree(ctx->d_word_ids);
@@ -336,9 +361,13 @@ int ngsd_destroy(ngsd_ctx *ctx) {
   cudaFree(ctx->d_def_rowptr); cudaFree(ctx->d_def_rowind); cudaFree(ctx->d_def_site); cudaFree(ctx->d_def_delta); cudaFree(ctx->d_fix);
   if (ctx->h_pin) cudaFreeHost(ctx->h_pin);
   if (ctx->h_pin2) cudaFreeHost(ctx->h_pin2);
+  if (ctx->h_lists) cudaFreeHost(ctx->h_lists);
   cudaFree(ctx->d_cs_begin); cudaFree(ctx->d_cnt_part);
-  for (auto &e : ctx->ev) if (e) cudaEventDestroy(e);
+  for (auto &set : ctx->ev_sets)
+    for (auto &e : set) if (e) cudaEventDestroy(e);
+  if (ctx->ev_pin) cudaEventDestroy(ctx->ev_pin);
   for (int b = 0; b < 2; b++) {
+    if (ctx->ev_copied[b]) cudaEventDestroy(ctx->ev_copied[b]);
     if (ctx->stage_free[b]) cudaEventDestroy(ctx->stage_free[b]);
     if (ctx->stage_ready[b]) cudaEventDestroy(ctx->stage_ready[b]);
   }
@@ -1062,7 +1091,8 @@ static int count_on_tensor_cores(ngsd_ctx *ctx, const uint32_t *block_counts, ui
     NGSD_CUDA(ctx, dev_alloc(&ctx->d_cnt_part, part));
     ctx->cnt_part_ints = part;
   }
-  NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_cs_begin, splits.data(), splits.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));   // pageable: staged before return
+  rc = upload_list(ctx, ctx->d_cs_begin, splits.data(), splits.size() * sizeof(uint32_t));
+  if (rc) return rc;
   if (ctx->shard_world > 1) NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_cnt, 0, ctx->n_pad * ctx->n_pad * sizeof(uint32_t), ctx->stream));
   ngsd_count_umma_args ca{ctx->d_cs_begin, n_splits, ctx->d_cnt_part, ctx->d_wsite, ctx->d_word_ids, ctx->d_word_layer};
   NGSD_CUDA(ctx, ngsd_launch_count_umma(ctx, ca));
@@ -1070,15 +1100,29 @@ static int count_on_tensor_cores(ngsd_ctx *ctx, const uint32_t *block_counts, ui
   return NGSD_OK;
 }
 
-int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_blocks, uint64_t block_size, double *out,
-                   double *num_opt, uint64_t *cnt_opt) {
-  if (!ctx) return NGSD_ERR_ARG;
-  if (!ctx->kids.empty()) return ngsd_group_distances(ctx, block_counts, n_blocks, block_size, out, num_opt, cnt_opt);
+// One distance matrix of one GPU in three steps: distances_enqueue does the host bookkeeping (weights, chunk list, weight
+// classes, count-pass word list, K splits) and queues the uploads and kernels; the caller copies ctx->d_out to the host;
+// distances_collect reads the device times.  The paths that end early (degenerate replicates, the integer path) copy
+// their matrix themselves and report job->copied.
+struct dist_job {
+  bool copied = false;        // the matrix is already in the caller's buffers and job->timing is complete
+  bool count_timed = false;   // ev[6..7] bracket a count pass
+  cudaEvent_t *ev = nullptr;  // the event set the matrix was timed with
+  ngsd_timing timing = {};
+};
+
+static int distances_enqueue(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_blocks, uint64_t block_size, double *out,
+                             double *num_opt, uint64_t *cnt_opt, dist_job *job) {
+  *job = dist_job();
+  job->ev = ctx->ev;
   NGSD_CUDA(ctx, cudaSetDevice(ctx->device));
   if (!ctx->frontend_done) {
     int rc = ngsd_frontend(ctx);
     if (rc) return rc;
   }
+  // the pinned scratch may still feed the uploads of the matrix enqueued before this one
+  NGSD_CUDA(ctx, cudaEventSynchronize(ctx->ev_pin));
+  ctx->h_lists_used = 0;
   const bool em_path = !ctx->cfg.indep_geno;   // default --probs: per pair-site em2 (ngsDist.cpp:348-349)
   const bool weighted = block_counts != nullptr;
   uint64_t n_eff = ctx->n_sites;
@@ -1103,10 +1147,14 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
       if (rc0) return rc0;
       ctx->timing = ngsd_timing();
       ctx->timing.launches = 1;
+      job->copied = true;
       return NGSD_OK;
     }
   }
-  if (ctx->int_path) return distances_int(ctx, block_counts, n_blocks, block_size, out, num_opt, cnt_opt);
+  if (ctx->int_path) {
+    job->copied = true;
+    return distances_int(ctx, block_counts, n_blocks, block_size, out, num_opt, cnt_opt);
+  }
   if (em_path && ctx->any_blank && !ctx->cfg.pairwise_del) {
     // An empty text line is (0,0,0) for every individual (read_data.cpp:58-59); em2 on it divides 0 by 0
     // (emOptim2.cpp:69-75 normalize), so every pair's sum turns NaN as soon as one such site is in the replicate.
@@ -1127,6 +1175,7 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
       if (rc0) return rc0;
       ctx->timing = ngsd_timing();
       ctx->timing.launches = 1;
+      job->copied = true;
       return NGSD_OK;
     }
   }
@@ -1236,6 +1285,7 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
     NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_num, 0, n2z * sizeof(double), ctx->stream));
     NGSD_CUDA(ctx, cudaMemsetAsync(ctx->d_cntout, 0, n2z * sizeof(uint64_t), ctx->stream));
     ctx->timing = ngsd_timing();
+    job->copied = true;
     return copy_out(ctx, out, num_opt, cnt_opt);
   }
   // The shared-site counts of --pairwise_del come from one of two sources: the per-block counts of the block cache
@@ -1335,10 +1385,12 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
   ctx->cur_cnt_cache = cnt_from_cache ? ctx->d_cnt_cache : nullptr;
 
   ctx->timing = ngsd_timing();
-  // (pageable source: the copy is staged before the call returns, so `splits` may go out of scope afterwards)
-  NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_split_begin, splits.data(), splits.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-  if (uniform_scale || use_cache)
-    NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_split_scale, scales.data(), scales.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+  rc = upload_list(ctx, ctx->d_split_begin, splits.data(), splits.size() * sizeof(uint32_t));
+  if (rc) return rc;
+  if (uniform_scale || use_cache) {
+    rc = upload_list(ctx, ctx->d_split_scale, scales.data(), scales.size() * sizeof(double));
+    if (rc) return rc;
+  }
   if (weighted) {
     if (need_site_weights && (!uniform_scale || ctx->planes == 2))   // per-site weights: scaled B fragments and/or the weighted c-vector
       NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_weights, h_w, bytes_w, cudaMemcpyHostToDevice, ctx->stream));
@@ -1348,8 +1400,10 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
     NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_ent_word, h_ew, n_entries * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
     NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_ent_mask, h_em, n_entries * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
   }
-  if (run_k3)
-    NGSD_CUDA(ctx, cudaMemcpyAsync(ctx->d_ent_begin, ent_begin.data(), ent_begin.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+  if (run_k3) {
+    rc = upload_list(ctx, ctx->d_ent_begin, ent_begin.data(), ent_begin.size() * sizeof(uint32_t));
+    if (rc) return rc;
+  }
   int launches = 0;
   const bool do_count = ctx->cfg.pairwise_del != 0;
   tick(ctx, 2);
@@ -1359,6 +1413,7 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
     if (rcc) return rcc;
     NGSD_CUDA(ctx, cudaEventRecord(ctx->ev[7], ctx->stream));
   }
+  NGSD_CUDA(ctx, cudaEventRecord(ctx->ev_pin, ctx->stream));   // every upload from pinned scratch is queued above
   if (run_k3) NGSD_CUDA(ctx, cudaEventRecord(ctx->ev_fork, ctx->stream));   // K3 entry lists are on the device
   tick(ctx, 3);
   // K2 / K2b first, so that its persistent CTAs own every SM; K3 (building the block cache's counts) is then launched on
@@ -1410,17 +1465,13 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
   }
   NGSD_CUDA(ctx, dbg_sync(ctx, "epilogue"));
   tick(ctx, 5);
-  rc = copy_out(ctx, out, num_opt, cnt_opt);
-  if (rc) return rc;
-  float ms;
-  ctx->timing.count_ms = 0;
-  if (cnt_on_tc || run_k3) { cudaEventElapsedTime(&ms, ctx->ev[6], ctx->ev[7]); ctx->timing.count_ms = ms; }   // K3 overlaps dist_ms; the tensor-core count precedes it
-  cudaEventElapsedTime(&ms, ctx->ev[3], ctx->ev[4]); ctx->timing.dist_ms = ms;
-  cudaEventElapsedTime(&ms, ctx->ev[8], ctx->ev[5]); ctx->timing.epilogue_ms = ms;
-  cudaEventElapsedTime(&ms, ctx->ev[2], ctx->ev[5]); ctx->timing.total_ms = ms;
+  job->count_timed = cnt_on_tc || run_k3;
   ctx->timing.launches = launches;
   ctx->timing.dist_ctas = plan.grid;
-  ctx->timing.dist_dmma = (em_path || (use_cache && !build_cache)) ? 0 : (uint64_t) plan.n_chunks * NGSD_K4_PER_CHUNK * ((uint64_t) (ctx->n_tiles - ctx->n_diag_tiles) * 256ull + (uint64_t) ctx->n_diag_tiles * 136ull);
+  // DMMAs executed per K4 step: 256 per full tile, 136 per diagonal tile, 16 per real 8-column block of an edge tile
+  const uint64_t dmma_step = (uint64_t) (ctx->n_tiles - ctx->n_diag_tiles - ctx->n_edge_tiles) * 256ull + (uint64_t) ctx->n_diag_tiles * 136ull +
+                             (uint64_t) ctx->n_edge_tiles * 16ull * ngsd_edge_c8(ctx->n_ind);
+  ctx->timing.dist_dmma = (em_path || (use_cache && !build_cache)) ? 0 : (uint64_t) plan.n_chunks * NGSD_K4_PER_CHUNK * dmma_step;
   ctx->timing.active_sites = active_sites;
   ctx->timing.block_cache = use_cache ? (build_cache ? 1 : 2) : 0;
   if (use_cache) {
@@ -1431,26 +1482,104 @@ int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_block
   ctx->cur_partials = ctx->d_partials;
   ctx->cur_split_w = nullptr;
   ctx->cur_cnt_cache = nullptr;
+  job->timing = ctx->timing;
   return NGSD_OK;
 }
 
-// The bootstrap loop of main() (ngsDist.cpp:217-238) in one call.  One GPU: replicates back to back on the context's
-// stream; groups and communicators deal them out (comm.cu).
+// Device times of an enqueued matrix into job->timing (waits for its epilogue).
+static int distances_collect(ngsd_ctx *ctx, dist_job *job) {
+  if (job->copied) return NGSD_OK;
+  cudaEvent_t *ev = job->ev;
+  NGSD_CUDA(ctx, cudaEventSynchronize(ev[5]));
+  float ms;
+  ngsd_timing &t = job->timing;
+  t.count_ms = 0;
+  if (job->count_timed) { cudaEventElapsedTime(&ms, ev[6], ev[7]); t.count_ms = ms; }   // K3 overlaps dist_ms; the tensor-core count precedes it
+  cudaEventElapsedTime(&ms, ev[3], ev[4]); t.dist_ms = ms;
+  cudaEventElapsedTime(&ms, ev[8], ev[5]); t.epilogue_ms = ms;
+  cudaEventElapsedTime(&ms, ev[2], ev[5]); t.total_ms = ms;
+  return NGSD_OK;
+}
+
+int ngsd_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_blocks, uint64_t block_size, double *out,
+                   double *num_opt, uint64_t *cnt_opt) {
+  if (!ctx) return NGSD_ERR_ARG;
+  if (!ctx->kids.empty()) return ngsd_group_distances(ctx, block_counts, n_blocks, block_size, out, num_opt, cnt_opt);
+  dist_job job;
+  int rc = distances_enqueue(ctx, block_counts, n_blocks, block_size, out, num_opt, cnt_opt, &job);
+  if (rc || job.copied) return rc;
+  rc = copy_out(ctx, out, num_opt, cnt_opt);
+  if (rc) return rc;
+  rc = distances_collect(ctx, &job);
+  ctx->timing = job.timing;
+  return rc;
+}
+
+// The single-GPU replicate loop.  Replicate r + 1 is enqueued -- its host bookkeeping included -- before replicate r is
+// collected, so the device runs the replicates back to back instead of waiting for each result copy and for the host to
+// build the next replicate's lists.  The matrices alternate between d_out and d_out_alt and reach the host on
+// copy_stream; replicate r + 2 waits for the copy of r before it overwrites that buffer.
+static int distances_pipelined(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_rep, uint64_t n_blocks, uint64_t block_size,
+                               double *out, ngsd_timing *sum) {
+  const uint64_t n2 = ctx->n_ind * ctx->n_ind;
+  if (n_rep > 1) {
+    int rc = ensure_dist_buffers(ctx, 1);
+    if (rc) return rc;
+    if (!ctx->d_out_alt) NGSD_CUDA(ctx, dev_alloc(&ctx->d_out_alt, n2));
+  }
+  double *buf[2] = {ctx->d_out, ctx->d_out_alt};
+  dist_job job[2];
+  auto collect = [&](uint64_t r) -> int {
+    dist_job &j = job[r & 1];
+    if (!j.copied) {
+      NGSD_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, j.ev[5], 0));
+      NGSD_CUDA(ctx, cudaMemcpyAsync(out + r * n2, buf[r & 1], n2 * sizeof(double), cudaMemcpyDeviceToHost, ctx->copy_stream));
+      NGSD_CUDA(ctx, cudaEventRecord(ctx->ev_copied[r & 1], ctx->copy_stream));
+      int rc = distances_collect(ctx, &j);
+      if (rc) return rc;
+    }
+    const ngsd_timing &t = j.timing;
+    sum->count_ms += t.count_ms; sum->dist_ms += t.dist_ms; sum->epilogue_ms += t.epilogue_ms;
+    sum->total_ms += t.total_ms; sum->launches += t.launches; sum->dist_dmma += t.dist_dmma;
+    sum->dist_imma += t.dist_imma; sum->active_sites += t.active_sites;
+    sum->dist_ctas = t.dist_ctas; sum->block_cache = t.block_cache;
+    return NGSD_OK;
+  };
+  int rc = NGSD_OK;
+  for (uint64_t r = 0; r < n_rep && !rc; r++) {
+    if (r >= 2 && cudaStreamWaitEvent(ctx->stream, ctx->ev_copied[r & 1], 0) != cudaSuccess) {
+      ngsd_set_error(ctx, "CUDA error: cannot order replicate %llu after a result copy", (unsigned long long) r);
+      rc = NGSD_ERR_CUDA;
+      break;
+    }
+    ctx->d_out = buf[r & 1];
+    ctx->ev = ctx->ev_sets[r & 1];
+    rc = distances_enqueue(ctx, block_counts + r * n_blocks, n_blocks, block_size, out + r * n2, nullptr, nullptr, &job[r & 1]);
+    buf[r & 1] = ctx->d_out;   // (allocated by the first enqueue when n_rep == 1)
+    if (job[r & 1].copied) job[r & 1].timing = ctx->timing;
+    if (!rc && r >= 1) rc = collect(r - 1);
+    if (!rc && r + 1 == n_rep) rc = collect(r);
+  }
+  // d_out keeps the last matrix (ngsd_device_results, ngsd_finish), d_out_alt the other buffer; set 0 times the pushes
+  ctx->d_out_alt = ctx->d_out == buf[0] ? buf[1] : buf[0];
+  ctx->ev = ctx->ev_sets[0];
+  const cudaError_t e = cudaStreamSynchronize(ctx->copy_stream);
+  if (rc) return rc;
+  NGSD_CUDA(ctx, e);
+  return NGSD_OK;
+}
+
+// The bootstrap loop of main() (ngsDist.cpp:217-238) in one call.  One GPU: distances_pipelined; groups and
+// communicators deal the replicates out (comm.cu).
 int ngsd_distances_batch(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_rep, uint64_t n_blocks, uint64_t block_size, double *out) {
   if (!ctx) return NGSD_ERR_ARG;
   if (!block_counts && n_rep) { ngsd_set_error(ctx, "null block_counts"); return NGSD_ERR_ARG; }
   if (!ctx->kids.empty() || ctx->comm) return ngsd_group_distances_batch(ctx, block_counts, n_rep, n_blocks, block_size, out);
   if (!out && n_rep) { ngsd_set_error(ctx, "null output"); return NGSD_ERR_ARG; }
-  const uint64_t n2 = ctx->n_ind * ctx->n_ind;
+  NGSD_CUDA(ctx, cudaSetDevice(ctx->device));
   ngsd_timing sum = ngsd_timing();
-  for (uint64_t r = 0; r < n_rep; r++) {
-    int rc = ngsd_distances(ctx, block_counts + r * n_blocks, n_blocks, block_size, out + r * n2, nullptr, nullptr);
-    if (rc) return rc;
-    sum.count_ms += ctx->timing.count_ms; sum.dist_ms += ctx->timing.dist_ms; sum.epilogue_ms += ctx->timing.epilogue_ms;
-    sum.total_ms += ctx->timing.total_ms; sum.launches += ctx->timing.launches; sum.dist_dmma += ctx->timing.dist_dmma;
-    sum.dist_imma += ctx->timing.dist_imma; sum.active_sites += ctx->timing.active_sites;
-    sum.dist_ctas = ctx->timing.dist_ctas; sum.block_cache = ctx->timing.block_cache;
-  }
+  int rc = distances_pipelined(ctx, block_counts, n_rep, n_blocks, block_size, out, &sum);
+  if (rc) return rc;
   ctx->timing = sum;
   return NGSD_OK;
 }
@@ -1478,7 +1607,11 @@ int ngsd_set_tile_shard(ngsd_ctx *ctx, uint32_t rank, uint32_t world) {
   NGSD_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   ctx->n_tiles = (uint32_t) mine.size();
   ctx->n_diag_tiles = 0;
-  for (auto &t : mine) ctx->n_diag_tiles += (t.ti == t.tj);
+  ctx->n_edge_tiles = 0;
+  for (auto &t : mine) {
+    ctx->n_diag_tiles += (t.ti == t.tj);
+    ctx->n_edge_tiles += ngsd_is_edge_tile(t, ctx->n_ind, ctx->RB);
+  }
   if (!mine.empty()) NGSD_CUDA(ctx, copy_sync(ctx, ctx->d_tiles, mine.data(), mine.size() * sizeof(ngsd_tile), cudaMemcpyHostToDevice));
   NGSD_CUDA(ctx, upload_tile_index(ctx, mine));
   if (!ctx->cfg.indep_geno) NGSD_CUDA(ctx, upload_em_tiles(ctx, mine));   // the EM path contracts the 64 x 64 tiles inside them

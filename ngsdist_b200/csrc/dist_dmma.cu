@@ -8,6 +8,7 @@
 //                 step with cp.async.bulk (TMA bulk copy, SASS UBLKCP) completing on an mbarrier; 4 stages x 48 KiB.
 //   warps 0..7    consumers, 2 (M) x 4 (N): each owns a 64 x 32 sub-tile = 8 x 4 DMMA accumulators (128 registers);
 //                 fragments come straight from the packed layout with conflict-free 256-byte LDS.64.
+//                 Diagonal tiles (upper triangle only) and edge tiles (real columns only) have their own warp layouts.
 // Work units are (K-split q, upper-triangle tile t), ordered split-major so that the CTAs resident at any moment
 // sweep the same site range of neighbouring tiles (operand tiles are shared through L2); CTA c takes units
 // c, c+grid, ...  Each unit writes its 128 x 128 partial in fragment order to a workspace slot; K4 (epilogue.cu)
@@ -72,9 +73,11 @@ struct DistArgs {
   double *partials;             // [n_units][16384]
   uint64_t NC;                  // chunk stride of the packed planes
   uint32_t n_tiles, n_units;
+  uint32_t edge_tj;             // last row block when n_ind % 128 != 0 (its off-diagonal tiles are edge tiles), else ~0
+  uint32_t edge_c8;             // 8-column blocks of the last row block that hold individuals (1..15)
 };
 
-enum : uint32_t { kFirst = 1u, kLast = 2u, kDiag = 4u, kExit = 8u };
+enum : uint32_t { kFirst = 1u, kLast = 2u, kDiag = 4u, kExit = 8u, kEdge = 16u };
 
 // One K4 step of a full (off-diagonal) tile for one consumer warp: 64 x 32 sub-tile, 12 LDS.64 + 32 DMMA.
 __device__ __forceinline__ void step_full(double (&acc)[64], const double *As, const double *Bs, double w) {
@@ -119,6 +122,39 @@ __device__ __forceinline__ void store_diag(const double (&acc)[64], double2 *dst
   for (int c = 15 - W; c < 16; c++) dst[(16 + c) * 32] = make_double2(acc[32 + c * 2], acc[32 + c * 2 + 1]);
 }
 
+// One chunk of an EDGE tile: off-diagonal, with the last row block as its column block, whose real individuals fill only
+// C8 of the 16 8-column blocks.  Warp W owns block-rows W and W + 8 x the C8 real block-columns: 2 * C8 DMMA + (2 + C8)
+// LDS.64 per K4 step on every warp (the full-tile layout would leave the padding columns on SMSPs 2 and 3 and keep them
+// the busiest).  acc[0 .. 2*C8) = row W, acc[2*C8 .. 4*C8) = row W + 8.  Each 8x8 block takes the same fragments, the
+// same weight product and the same DMMA sequence as in step_full, so its sums are bit-identical.
+template <int C8, int PLANES>
+__device__ __forceinline__ void chunk_edge(double (&acc)[64], const double *As, const double *Bs, const double (&wv)[3]) {
+#pragma unroll
+  for (int k4 = 0; k4 < NGSD_K4_PER_CHUNK; k4++) {
+    const double *Ak = As + k4 * 512, *Bk = Bs + k4 * 512;
+    const double w = wv[PLANES == 3 ? (k4 & 1) : (k4 % 3)];
+    const double a0 = Ak[0], a1 = Ak[8 * 32];
+    double bf[C8];
+#pragma unroll
+    for (int c = 0; c < C8; c++) bf[c] = Bk[c * 32] * w;
+#pragma unroll
+    for (int c = 0; c < C8; c++) dmma884(acc[c * 2], acc[c * 2 + 1], a0, bf[c]);
+#pragma unroll
+    for (int c = 0; c < C8; c++) dmma884(acc[(C8 + c) * 2], acc[(C8 + c) * 2 + 1], a1, bf[c]);
+  }
+}
+
+// Edge-tile partial in the full-tile fragment order (block (R, C) -> warp (R/8)*4 + C/4, frag (R%8)*4 + C%4), so that
+// k_epilogue decodes it like a full tile; the padding blocks are not written (the epilogue reads no column >= n_ind).
+template <int C8>
+__device__ __forceinline__ void store_edge(const double (&acc)[64], double2 *tile, int W) {
+#pragma unroll
+  for (int h = 0; h < 2; h++)
+#pragma unroll
+    for (int c = 0; c < C8; c++)
+      tile[((h * 4 + c / 4) * 32 + W * 4 + (c & 3)) * 32] = make_double2(acc[(h * C8 + c) * 2], acc[(h * C8 + c) * 2 + 1]);
+}
+
 // PLANES = 3: chunk of 8 sites, k4-group = g*2 + h;  PLANES = 2: chunk of 12 sites, k4-group = g*3 + h (ngsd_internal.h).
 // The only place the two differ inside the kernel is which per-site weight a k4-group takes.
 template <bool WEIGHTED, int PLANES>
@@ -152,7 +188,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_dmma(DistArgs a) {
         const uint32_t c0 = a.split_begin[q], c1 = a.split_begin[q + 1];
         const double *Ab = a.Apack + (uint64_t) tl.ti * a.NC * NGSD_TILE_DOUBLES;
         const double *Bb = a.Bpack + (uint64_t) tl.tj * a.NC * NGSD_TILE_DOUBLES;
-        const uint32_t fl = tl.ti == tl.tj ? kDiag : 0u;
+        const uint32_t fl = tl.ti == tl.tj ? kDiag : (tl.tj == a.edge_tj ? kEdge : 0u);
         for (uint32_t c = c0; c < c1; c++) {
           const uint64_t chunk = a.chunk_ids ? a.chunk_ids[c] : c;
           mbar_wait(&empty[stage], phase ^ 1);
@@ -205,6 +241,15 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_dmma(DistArgs a) {
         case 6: chunk_diag<6, PLANES>(acc, As, Bs, wv); break;
         default: chunk_diag<7, PLANES>(acc, As, Bs, wv); break;
       }
+    } else if (fl & kEdge) {
+      const double *As = stageA(stage) + warp * 32 + lane, *Bs = stageB(stage) + lane;
+      switch (a.edge_c8) {  // kernel-uniform
+#define NGSD_EDGE_CASE(C) case C: chunk_edge<C, PLANES>(acc, As, Bs, wv); break;
+        NGSD_EDGE_CASE(1) NGSD_EDGE_CASE(2) NGSD_EDGE_CASE(3) NGSD_EDGE_CASE(4) NGSD_EDGE_CASE(5)
+        NGSD_EDGE_CASE(6) NGSD_EDGE_CASE(7) NGSD_EDGE_CASE(8) NGSD_EDGE_CASE(9) NGSD_EDGE_CASE(10)
+        NGSD_EDGE_CASE(11) NGSD_EDGE_CASE(12) NGSD_EDGE_CASE(13) NGSD_EDGE_CASE(14) default: chunk_edge<15, PLANES>(acc, As, Bs, wv); break;
+#undef NGSD_EDGE_CASE
+      }
     } else {
       const double *As = stageA(stage) + (wm * 8) * 32 + lane, *Bs = stageB(stage) + (wn * 4) * 32 + lane;
 #pragma unroll
@@ -215,7 +260,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_dmma(DistArgs a) {
     if (++stage == kStages) { stage = 0; phase ^= 1; }
     if (fl & kLast) {
       // partial tile in fragment order: [warp][32 accumulator pairs][lane] double2 (decoded in epilogue.cu)
-      double2 *dst = reinterpret_cast<double2 *>(a.partials + (uint64_t) u * NGSD_TILE_ELEMS) + (warp * 32) * 32 + lane;
+      double2 *tile = reinterpret_cast<double2 *>(a.partials + (uint64_t) u * NGSD_TILE_ELEMS) + lane;
+      double2 *dst = tile + (warp * 32) * 32;
       if (a.split_scale) {      // bootstrap multiplicity shared by every chunk of this split (block_size % 8 == 0)
         const double sc = a.split_scale[u / a.n_tiles];
         if (sc != 1.0) {
@@ -233,6 +279,14 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_dmma(DistArgs a) {
           case 5: store_diag<5>(acc, dst); break;
           case 6: store_diag<6>(acc, dst); break;
           default: store_diag<7>(acc, dst); break;
+        }
+      } else if (fl & kEdge) {
+        switch (a.edge_c8) {
+#define NGSD_EDGE_CASE(C) case C: store_edge<C>(acc, tile, warp); break;
+          NGSD_EDGE_CASE(1) NGSD_EDGE_CASE(2) NGSD_EDGE_CASE(3) NGSD_EDGE_CASE(4) NGSD_EDGE_CASE(5)
+          NGSD_EDGE_CASE(6) NGSD_EDGE_CASE(7) NGSD_EDGE_CASE(8) NGSD_EDGE_CASE(9) NGSD_EDGE_CASE(10)
+          NGSD_EDGE_CASE(11) NGSD_EDGE_CASE(12) NGSD_EDGE_CASE(13) NGSD_EDGE_CASE(14) default: store_edge<15>(acc, tile, warp); break;
+#undef NGSD_EDGE_CASE
         }
       } else {
 #pragma unroll
@@ -287,6 +341,9 @@ cudaError_t ngsd_launch_dist_dmma(ngsd_ctx *ctx, const ngsd_dist_plan &p) {
   a.NC = ctx->NC;
   a.n_tiles = ctx->n_tiles;
   a.n_units = p.n_units;
+  const uint32_t c8 = ngsd_edge_c8(ctx->n_ind);
+  a.edge_tj = c8 ? (uint32_t) ctx->RB - 1 : 0xFFFFFFFFu;
+  a.edge_c8 = c8;
   cudaError_t e = cudaMemsetAsync(ctx->d_sched, 0, sizeof(uint32_t), ctx->stream);
   if (e != cudaSuccess) return e;
   if (p.weighted && !p.uniform_scale) {

@@ -41,6 +41,16 @@ constexpr int NGSD_TILE_ELEMS = NGSD_TILE * NGSD_TILE;           // accumulator 
 
 struct ngsd_tile { uint16_t ti, tj; };
 
+// 8-column blocks of the last row block that hold individuals (1..15), or 0 when all 16 do (n_ind % 128 == 0 or > 120).
+// k_dist_dmma contracts only these columns in the off-diagonal tiles of that block ("edge tiles").
+inline uint32_t ngsd_edge_c8(uint64_t n_ind) {
+  const uint32_t c8 = (uint32_t) ((n_ind % NGSD_TILE + 7) / 8);
+  return c8 < 16 ? c8 : 0u;
+}
+inline bool ngsd_is_edge_tile(const ngsd_tile &t, uint64_t n_ind, uint64_t RB) {
+  return ngsd_edge_c8(n_ind) && t.ti != t.tj && t.tj == RB - 1;
+}
+
 // A triple whose outcome hangs on the last ulp of log / exp (a comparison of the reference within 1e-11 of flipping):
 // the front-end kernels append it here and the host re-evaluates it with its own libm -- the reference's -- before
 // anything is contracted (api.cu resolve_deferred, frontend.cu k_patch).
@@ -125,12 +135,17 @@ struct ngsd_ctx {
   double *d_split_scale = nullptr;   // K-split boundaries in the chunk list
   uint32_t *d_sched = nullptr;                 // dynamic unit counter of k_dist_dmma
   uint32_t n_diag_tiles = 0;
+  uint32_t n_edge_tiles = 0;                   // owned off-diagonal tiles of the last row block when n_ind % 128 != 0 (ngsd_edge_c8)
   uint32_t shard_rank = 0, shard_world = 1;   // output-tile sharding
   uint32_t *d_ent_word = nullptr; uint64_t *d_ent_mask = nullptr; uint64_t ent_cap = 0;   // mask-count entries
   uint32_t *d_cnt = nullptr;                   // [n_pad][n_pad] shared-site counts
   double *d_out = nullptr, *d_num = nullptr; uint64_t *d_cntout = nullptr;   // [n_ind][n_ind]
+  double *d_out_alt = nullptr;                 // second result buffer of the single-GPU replicate loop (ngsd_distances_batch)
+  cudaEvent_t ev_copied[2] = {nullptr, nullptr};   // copy_stream: the matrix in d_out / d_out_alt has reached the host
   void *h_pin = nullptr; uint64_t h_pin_bytes = 0;    // pinned scratch for weights / lists / results
   void *h_pin2 = nullptr; uint64_t h_pin2_bytes = 0;  // pinned scratch of the tensor-core count pass of the FP64 path
+  void *h_lists = nullptr; uint64_t h_lists_bytes = 0, h_lists_used = 0;   // pinned staging of small host lists (K splits, scales)
+  cudaEvent_t ev_pin = nullptr;                // ctx->stream: the uploads of the last enqueued matrix have read h_pin, h_pin2 and h_lists
   uint32_t *d_cs_begin = nullptr; uint32_t cs_cap = 0;          // its K-split boundaries
   int32_t *d_cnt_part = nullptr; uint64_t cnt_part_ints = 0;    // its partial count tiles
   // ---- multi-GPU (comm.cu) ----
@@ -147,7 +162,10 @@ struct ngsd_ctx {
   std::vector<uint64_t> site_begin;            // [n_gpus + 1] first site of every kid
   bool kids_tile_sharded = false;
   // timing
-  cudaEvent_t ev[10] = {};
+  // events 0..1 time a push (set 0); 2..8 time one distance matrix.  The single-GPU replicate loop keeps two matrices in
+  // flight and alternates the sets, so `ev` points at the set of the matrix being enqueued.
+  cudaEvent_t ev_sets[2][10] = {};
+  cudaEvent_t *ev = ev_sets[0];
   ngsd_timing timing = {};
   char err[512] = {0};
 };
