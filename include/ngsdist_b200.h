@@ -67,7 +67,9 @@ typedef struct {
   uint64_t n_ind;            /* params.n_ind                                                        */
   uint64_t n_sites;          /* params.n_sites (all sites of the data set)                          */
   uint64_t tot_sites;        /* params.tot_sites; > 0 overrides the per-pair count (ngsDist.cpp:372) */
-  double score[9];           /* params.score[g1][g2], row-major (parse_args.cpp:25-27,134-137)      */
+  double score[9];           /* params.score[g1][g2], row-major (parse_args.cpp:25-27,134-137); g1 is the genotype of
+                                the lower-index individual of the pair, g2 of the higher (i1 < i2, ngsDist.cpp:351-353).
+                                Need not be symmetric                                                 */
   int32_t evol_model;        /* 0 raw p-distance, 1 -log(1-d), 2 JC69 (ngsDist.cpp:378-386)         */
   int32_t pairwise_del;      /* params.pairwise_del                                                  */
   int32_t indep_geno;        /* params.indep_geno AFTER the forcing rules of ngsDist.cpp:55-62      */

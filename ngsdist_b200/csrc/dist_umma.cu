@@ -636,23 +636,39 @@ extern "C" int ngsd_probe_int8_tmacs(int device, double *imma_tmacs) {
   return NGSD_OK;
 }
 
-// f(k, c) * S as int8 bytes; returns false when the score matrix does not give small integers (-> FP64 path)
+// f(k, c) * S as int8 bytes; returns false when S * score is not a matrix of exact small integers (-> FP64 path).
+// Only then is acc / S the reference's sum: a score that is merely close to k / S (1e-12 x the default, or 0.5 + 3e-11)
+// must not be rounded onto the integer grid.  The missing-genotype entries (the uniform triple) are built from those
+// integers: S f(k, 3) = sum_c R[k][c] / 3, S f(3, c) = sum_k R[k][c] / 3, S f(3, 3) = sum R / 9, each an exact quotient.
 bool ngsd_int_lut(const double *score, bool pairwise_del, uint32_t lut[4], double *scale, int *max_byte) {
   const double S = pairwise_del ? 2.0 : 18.0;
-  double f[4][4];
-  double rs[3] = {0, 0, 0}, cs[3] = {0, 0, 0}, tot = 0;
+  long long R[4][4] = {};
   for (int k = 0; k < 3; k++)
-    for (int c = 0; c < 3; c++) { f[k][c] = score[k * 3 + c]; rs[k] += score[k * 3 + c]; cs[c] += score[k * 3 + c]; tot += score[k * 3 + c]; }
-  for (int k = 0; k < 3; k++) { f[k][3] = pairwise_del ? 0.0 : rs[k] / 3.0; f[3][k] = pairwise_del ? 0.0 : cs[k] / 3.0; }
-  f[3][3] = pairwise_del ? 0.0 : tot / 9.0;
+    for (int c = 0; c < 3; c++) {
+      const double v = score[k * 3 + c], r = nearbyint(v * S);
+      if (!(fabs(r) <= 127) || fma(v, S, -r) != 0.0) return false;   // NaN, out of range, or S v not exactly the integer r
+      R[k][c] = (long long) r;
+    }
+  if (!pairwise_del) {
+    long long tot = 0;
+    for (int k = 0; k < 3; k++) {
+      const long long rs = R[k][0] + R[k][1] + R[k][2], cs = R[0][k] + R[1][k] + R[2][k];
+      if (rs % 3 || cs % 3) return false;
+      R[k][3] = rs / 3;
+      R[3][k] = cs / 3;
+      tot += rs;
+    }
+    if (tot % 9) return false;
+    R[3][3] = tot / 9;
+  }
   int mx = 0;
   for (int c = 0; c < 4; c++) {
     uint32_t wv = 0;
     for (int k = 0; k < 4; k++) {
-      const double v = f[k][c] * S, r = nearbyint(v);
-      if (fabs(v - r) > 1e-9 || r < 0 || r > 127) return false;
-      if (!pairwise_del && k < 3 && ((int) r) % 3) return false;   // the three-plane form (header) carries S / 3 on the B side
-      wv |= (uint32_t) (int) r << (8 * k);
+      const long long r = R[k][c];
+      if (r < 0 || r > 127) return false;
+      if (!pairwise_del && k < 3 && r % 3) return false;   // the three-plane form (header) carries S / 3 on the B side
+      wv |= (uint32_t) r << (8 * k);
       if ((int) r > mx) mx = (int) r;
     }
     lut[c] = wv;

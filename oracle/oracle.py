@@ -172,11 +172,12 @@ def distances_block(P, r0, r1, c0, c1, score=None, indep=True, pairwise_del=Fals
 
 def run_job(raw, *, in_log=False, call_geno=False, N_thresh=0.0, call_thresh=0.0, avg_nuc_dist=False, indep=True,
             pairwise_del=False, tot_sites=0, evol_model=1, n_boot_rep=0, boot_block_size=1, seed=12345, kind=0, blank_sites=(),
-            genotypes=False):
+            genotypes=False, score=None):
     """Whole job the way main() runs it (ngsDist.cpp:156-289): returns the list of 1+n_boot_rep result dicts.
     blank_sites: sites that were empty text lines -- read_geno leaves them at the -1e15 fill without normalising
     (read_data.cpp:58-59), so after ngsDist.cpp:165-174 every individual holds (0,0,0) there, or the missing-data triple
-    exp(log(1/3)) when call_geno ran on the all-equal fill (gen_func.cpp:895-905).  genotypes: raw is [site][ind] codes."""
+    exp(log(1/3)) when call_geno ran on the all-equal fill (gen_func.cpp:895-905).  genotypes: raw is [site][ind] codes.
+    score: the 3 x 3 matrix params.score[g1][g2] (9 values, row-major) instead of the one avg_nuc_dist selects."""
     if genotypes:
         P = frontend_geno(raw)
     else:
@@ -188,7 +189,7 @@ def run_job(raw, *, in_log=False, call_geno=False, N_thresh=0.0, call_thresh=0.0
     n_sites = P.shape[1]
     rng = Taus(seed)
     out = []
-    kw = dict(score=score_matrix(avg_nuc_dist), indep=indep, pairwise_del=pairwise_del, tot_sites=tot_sites, evol_model=evol_model)
+    kw = dict(score=score_matrix(avg_nuc_dist) if score is None else score, indep=indep, pairwise_del=pairwise_del, tot_sites=tot_sites, evol_model=evol_model)
     for rep in range(n_boot_rep + 1):
         if rep == 0:
             out.append(distances(P, **kw))
