@@ -238,6 +238,19 @@ NGSD_API int ngsd_bind_host_to_device(int device);
 NGSD_API int ngsd_nj_tree(ngsd_ctx *ctx, const double *dist_host, const char *const *labels, char *newick, uint64_t newick_cap,
                           uint64_t *newick_len);
 
+/* The criterion FastME optimises: a balanced minimum-evolution tree (BME; Desper & Gascuel 2002, Pauplin's length
+ * L(T) = sum_{i<j} 2^(1 - tau_ij) d_ij, tau_ij the number of edges between leaves i and j).  Starts from the tree of
+ * ngsd_nj_tree, applies the BME nearest-neighbour interchange of largest gain (ties: smallest internal node id, then the
+ * swap with the child of the smaller individual index) while its gain exceeds 1e-12 M, M = sum_{i<j} 2^(1 - tau_ij) |d_ij|
+ * (M = L when no distance is negative), and writes the tree with balanced branch lengths (they sum to L; negative lengths
+ * are written as computed).  Every applied interchange lowers L, so the call returns for every finite matrix, negative
+ * entries included.  Every round is O(n^2) work on the device; the matrix is read in place (dist_host: one upload).  Same arguments, matrix source, labels and errors as ngsd_nj_tree; the Newick is rooted as a trifurcation at the
+ * neighbour of individual 0, "(Ind_0:l,(...):l,(...):l);", every node's children in order of their smallest individual
+ * index.  n_nni (may be NULL) receives the number of interchanges applied.  Parity is against a CPU restatement of the
+ * same rules (oracle/bme_oracle.py); DESIGN §3 N4 states them. */
+NGSD_API int ngsd_bme_tree(ngsd_ctx *ctx, const double *dist_host, const char *const *labels, char *newick, uint64_t newick_cap,
+                           uint64_t *newick_len, uint64_t *n_nni);
+
 /* Bootstrap support of a tree -- the last step of the reference's workflow (README.md:83-98: `raxmlHPC -f b -t main -z
  * boots` on FastME's trees).  HOST code only, no context: for every internal edge of `main_newick`, the number of trees among
  * `rep_newicks[n_reps]` that hold the same bipartition of the leaf labels is written as the node's label

@@ -22,6 +22,7 @@ ABI_SYMBOLS = [
     "ngsd_probe_fp64_tflops", "ngsd_probe_int8_tmacs", "ngsd_probe_umma_tmacs", "ngsd_host_alloc", "ngsd_host_free", "ngsd_set_tile_shard", "ngsd_device_results", "ngsd_finish",
     "ngsd_distances_batch", "ngsd_comm_unique_id", "ngsd_comm_attach", "ngsd_comm_allgather_operands", "ngsd_comm_reduce_sites", "ngsd_comm_reduce_tiles",
     "ngsd_comm_barrier", "ngsd_comm_stats", "ngsd_bind_host_to_device", "ngsd_deferred_stats", "ngsd_push_sites_packed", "ngsd_nj_tree", "ngsd_tree_support",
+    "ngsd_bme_tree",
 ]
 ABI_VERSION = 2
 COMM_ID_BYTES = 128
@@ -131,6 +132,11 @@ def lib():
                  "ngsd_comm_allgather_operands", "ngsd_comm_reduce_sites", "ngsd_comm_reduce_tiles", "ngsd_comm_barrier", "ngsd_comm_stats",
                  "ngsd_bind_host_to_device", "ngsd_deferred_stats", "ngsd_push_sites_packed", "ngsd_nj_tree", "ngsd_tree_support"):
         getattr(L, name).restype = i32
+    # (a build from before ngsd_bme_tree, named by NGSDIST_B200_LIB for an A/B comparison of the other entry points, lacks it;
+    # build() and tests/test_abi_surface.py require it of this package's library)
+    if hasattr(L, "ngsd_bme_tree"):
+        L.ngsd_bme_tree.argtypes = [vp, vp, vp, vp, u64, C.POINTER(u64), C.POINTER(u64)]
+        L.ngsd_bme_tree.restype = i32
     _lib = L
     return L
 
@@ -553,6 +559,26 @@ class NgsDistB200:
             rc = lib().ngsd_nj_tree(self._h, _ptr(d), lab, buf, cap, C.byref(need))
             if rc == 0:
                 return buf.value.decode()
+            if need.value + 1 > cap:
+                cap = need.value + 1
+                continue
+            self._check(rc)
+        self._check(rc)
+
+    def bme_tree(self, dist=None, labels=None):
+        """Balanced minimum-evolution tree (Newick, balanced branch lengths) refined by BME interchanges from the
+        neighbour-joining tree of the last matrix on the device, or of `dist`; returns (newick, interchanges applied)."""
+        d = None if dist is None else np.ascontiguousarray(dist, dtype=np.float64)
+        lab = None
+        if labels is not None:
+            lab = (C.c_char_p * len(labels))(*[str(x).encode() for x in labels])
+        need, n_nni = C.c_uint64(0), C.c_uint64(0)
+        cap = 64 * self.p.n_ind + 1024
+        for _ in range(2):
+            buf = C.create_string_buffer(cap)
+            rc = lib().ngsd_bme_tree(self._h, _ptr(d), lab, buf, cap, C.byref(need), C.byref(n_nni))
+            if rc == 0:
+                return buf.value.decode(), n_nni.value
             if need.value + 1 > cap:
                 cap = need.value + 1
                 continue

@@ -10,7 +10,8 @@
 //
 // Differences on purpose (documented in DESIGN.md): text lines may be longer than the reference's 500 000-character
 // buffer; input is streamed in chunks (the whole data set is never held on the host); --verbose >= 5 per-site dumps are
-// not produced; additive flags: --device N (first GPU), --tree FILE (a neighbour-joining tree per matrix, and FILE.support with bootstrap support values), --n_gpus N and
+// not produced; additive flags: --device N (first GPU), --tree FILE (a neighbour-joining tree per matrix, and FILE.support with bootstrap support values),
+// --nni_bme (with --tree: balanced minimum-evolution trees refined from the neighbour-joining ones), --n_gpus N and
 // --shard auto|replicated|sites (multi-GPU inside
 // the library, SURVEY §8e).  The tail of gen_dist (ngsDist.cpp:372-386: division, -log(1-d), JC69) runs HERE with the
 // host's libm on the raw distance the device returns, so that the written values are the reference's to the last digit.
@@ -55,6 +56,7 @@ struct Pars {
   unsigned n_threads = 1, verbose = 1, seed = 0;
   int device = 0, n_gpus = 1, shard = 0;
   const char *tree = nullptr;   // --tree FILE: one neighbour-joining tree (Newick) per matrix
+  bool nni_bme = false;         // --nni_bme: with --tree, refine each tree by balanced minimum-evolution NNIs (ngsd_bme_tree)
 };
 
 // error(): same shape as the reference's (shared/gen_func.cpp:12-18): banner on stderr, perror, exit(-1)
@@ -88,7 +90,7 @@ static void parse_args(Pars *p, int argc, char **argv) {
       {"n_threads", required_argument, nullptr, 'x'},  {"verbose", required_argument, nullptr, 'V'},
       {"seed", required_argument, nullptr, 'r'},       {"device", required_argument, nullptr, 1000},
       {"n_gpus", required_argument, nullptr, 1001},    {"shard", required_argument, nullptr, 1002},
-      {"tree", required_argument, nullptr, 1003},
+      {"tree", required_argument, nullptr, 1003},      {"nni_bme", no_argument, nullptr, 1004},
       {nullptr, 0, nullptr, 0}};
   p->seed = (unsigned) time(nullptr);
   int c;
@@ -120,6 +122,7 @@ static void parse_args(Pars *p, int argc, char **argv) {
       case 1000: p->device = atoi(optarg); break;
       case 1001: p->n_gpus = atoi(optarg); break;
       case 1003: p->tree = optarg; break;
+      case 1004: p->nni_bme = true; break;
       case 1002:
         if (strcmp(optarg, "auto") == 0) p->shard = NGSD_SHARD_AUTO;
         else if (strcmp(optarg, "replicated") == 0) p->shard = NGSD_SHARD_REPLICATED;
@@ -158,6 +161,7 @@ static void parse_args(Pars *p, int argc, char **argv) {
   if (p->out == nullptr) die("parse_cmd_args", "output prefix (--out) missing!");
   if (p->n_threads < 1) die("parse_cmd_args", "number of threads cannot be less than 1!");
   if (p->n_gpus < 1) die("parse_cmd_args", "number of GPUs (--n_gpus) cannot be less than 1!");
+  if (p->nni_bme && p->tree == nullptr) die("parse_cmd_args", "balanced NNI refinement (--nni_bme) needs a tree output file (--tree)!");
 }
 
 // ---- line-oriented gz reading (labels, positions, text genotypes) --------------------------------------------
@@ -346,17 +350,22 @@ static int selftest_io(uint64_t n) {
   return bad ? 1 : 0;
 }
 
-// --tree: the step the reference's workflow (README.md:83-98) runs FastME for -- one neighbour-joining tree per matrix,
-// computed on the device from the matrix that was just written (after the host's -log / JC69 tail)
-static void write_tree(FILE *fh, ngsd_ctx *ctx, const double *d, const std::vector<std::string> &lab, std::vector<std::string> *keep) {
+// --tree: the step the reference's workflow (README.md:83-98) runs FastME for -- one neighbour-joining tree per matrix
+// (with --nni_bme: refined by balanced minimum-evolution NNIs, FastME's criterion), computed on the device from the
+// matrix that was just written (after the host's -log / JC69 tail)
+static void write_tree(FILE *fh, ngsd_ctx *ctx, bool bme, const double *d, const std::vector<std::string> &lab, std::vector<std::string> *keep) {
   std::vector<const char *> names;
   for (auto &l : lab) names.push_back(l.c_str());
   uint64_t need = 0;
   std::vector<char> buf(64 * lab.size() + 1024);
-  int rc = ngsd_nj_tree(ctx, d, names.data(), buf.data(), buf.size(), &need);
+  auto tree = [&]() {
+    return bme ? ngsd_bme_tree(ctx, d, names.data(), buf.data(), buf.size(), &need, nullptr)
+               : ngsd_nj_tree(ctx, d, names.data(), buf.data(), buf.size(), &need);
+  };
+  int rc = tree();
   if (rc && need + 1 > buf.size()) {
     buf.resize(need + 1);
-    rc = ngsd_nj_tree(ctx, d, names.data(), buf.data(), buf.size(), &need);
+    rc = tree();
   }
   if (rc) {
     fprintf(stderr, "> no tree for this matrix: %s\n", ngsd_last_error(ctx));
@@ -802,7 +811,7 @@ int main(int argc, char **argv) {
         if (host_model) apply_model(dist.data() + q * n2, p.n_ind, p.evol_model, p.n_threads);
         if (p.verbose >= 2) fprintf(stderr, "> Printing distance matrix\n");
         write_matrix(out_fh, labels, dist.data() + q * n2, p.n_ind, p.n_threads);
-        if (tree_fh) write_tree(tree_fh, ctx, dist.data() + q * n2, labels, &trees);
+        if (tree_fh) write_tree(tree_fh, ctx, p.nni_bme, dist.data() + q * n2, labels, &trees);
       }
       rep += k - 1;
       continue;
@@ -833,7 +842,7 @@ int main(int argc, char **argv) {
     if (host_model) apply_model(dist.data(), p.n_ind, p.evol_model, p.n_threads);
     if (p.verbose >= 2) fprintf(stderr, "> Printing distance matrix\n");
     write_matrix(out_fh, labels, dist.data(), p.n_ind, p.n_threads);
-    if (tree_fh) write_tree(tree_fh, ctx, dist.data(), labels, &trees);
+    if (tree_fh) write_tree(tree_fh, ctx, p.nni_bme, dist.data(), labels, &trees);
   }
   fclose(out_fh);
   if (tree_fh) fclose(tree_fh);

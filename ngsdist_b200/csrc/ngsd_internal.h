@@ -237,6 +237,14 @@ struct ngsd_count_umma_args {
 cudaError_t ngsd_launch_count_umma(ngsd_ctx *ctx, const ngsd_count_umma_args &c);   // dist_umma.cu: --pairwise_del counts of the FP64 path
 cudaError_t ngsd_launch_epilogue_int(ngsd_ctx *ctx, uint32_t n_splits, uint64_t const_cnt, bool in_kernel_cnt);   // epilogue.cu
 
+// ---- N4 trees (nj.cu, bme.cu) ----
+// join t merged the subtrees in slots i < j with limb lengths li, lj; the new node takes slot i, slot j retires
+struct NjJoin { uint32_t i, j; double li, lj; };
+// the neighbour-joining loop on the device, on a working copy of dist_host, or of the device matrix dist_dev when
+// dist_host == NULL: the n - 3 joins, the three slots left (in increasing order) and their distances d(a,b), d(a,c),
+// d(b,c).  NGSD_ERR_ARG for a non-finite matrix.
+int ngsd_nj_joins(ngsd_ctx *ctx, const double *dist_host, const double *dist_dev, std::vector<NjJoin> *joins, uint64_t rem[3], double d3[3]);
+
 // ---- multi-GPU (comm.cu) ----
 extern "C" int ngsd_frontend_resolve(ngsd_ctx *ctx);      // api.cu: knife-edge triples -> host libm -> k_patch
 extern "C" int ngsd_frontend_flags(ngsd_ctx *ctx);        // api.cu: the deferred error flags of the front end, without the completeness check

@@ -27,8 +27,6 @@
 
 namespace {
 
-struct NjJoin { uint32_t i, j; double li, lj; };
-
 __global__ void __launch_bounds__(256) k_nj_rowsum(const double *__restrict__ D, uint64_t n, double *__restrict__ r, int *__restrict__ bad) {
   __shared__ double red[256];
   const uint64_t i = blockIdx.x;
@@ -152,20 +150,16 @@ void append_len(std::string &s, double v) {
 
 }  // namespace
 
-extern "C" int ngsd_nj_tree(ngsd_ctx *ctx, const double *dist_host, const char *const *labels, char *newick, uint64_t newick_cap,
-                            uint64_t *newick_len) {
-  if (!ctx || !newick_len) return NGSD_ERR_ARG;
-  if (!ctx->kids.empty()) ctx = ctx->kids[0];
+// the join loop, shared by ngsd_nj_tree and ngsd_bme_tree (bme.cu)
+int ngsd_nj_joins(ngsd_ctx *ctx, const double *dist_host, const double *dist_dev, std::vector<NjJoin> *joins, uint64_t rem[3], double d3[3]) {
   const uint64_t n = ctx->n_ind;
-  if (n < 3) { ngsd_set_error(ctx, "a tree needs at least 3 individuals"); return NGSD_ERR_ARG; }
-  if (!dist_host && !ctx->d_out) { ngsd_set_error(ctx, "no distance matrix yet: call ngsd_distances first or pass one"); return NGSD_ERR_STATE; }
   NGSD_CUDA(ctx, cudaSetDevice(ctx->device));
   double *D = nullptr, *r = nullptr, *rowq = nullptr;
   uint32_t *rowj = nullptr, *m_dev = nullptr;
   uint8_t *active = nullptr;
-  NjJoin *joins = nullptr;
+  NjJoin *jdev = nullptr;
   int *bad = nullptr;
-  auto release = [&]() { cudaFree(D); cudaFree(r); cudaFree(rowq); cudaFree(rowj); cudaFree(m_dev); cudaFree(active); cudaFree(joins); cudaFree(bad); };
+  auto release = [&]() { cudaFree(D); cudaFree(r); cudaFree(rowq); cudaFree(rowj); cudaFree(m_dev); cudaFree(active); cudaFree(jdev); cudaFree(bad); };
 #define NJ_CUDA(call)                                                                                   \
   do {                                                                                                  \
     cudaError_t e_ = (call);                                                                            \
@@ -181,11 +175,11 @@ extern "C" int ngsd_nj_tree(ngsd_ctx *ctx, const double *dist_host, const char *
   NJ_CUDA(cudaMalloc((void **) &rowj, n * sizeof(uint32_t)));
   NJ_CUDA(cudaMalloc((void **) &m_dev, sizeof(uint32_t)));
   NJ_CUDA(cudaMalloc((void **) &active, n));
-  NJ_CUDA(cudaMalloc((void **) &joins, (n - 2) * sizeof(NjJoin)));
+  NJ_CUDA(cudaMalloc((void **) &jdev, (n - 2) * sizeof(NjJoin)));
   NJ_CUDA(cudaMalloc((void **) &bad, sizeof(int)));
   cudaStream_t st = ctx->stream;
   if (dist_host) NJ_CUDA(cudaMemcpyAsync(D, dist_host, n * n * sizeof(double), cudaMemcpyHostToDevice, st));
-  else NJ_CUDA(cudaMemcpyAsync(D, ctx->d_out, n * n * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  else NJ_CUDA(cudaMemcpyAsync(D, dist_dev, n * n * sizeof(double), cudaMemcpyDeviceToDevice, st));
   const uint32_t m0 = (uint32_t) n;
   NJ_CUDA(cudaMemcpyAsync(m_dev, &m0, sizeof(uint32_t), cudaMemcpyHostToDevice, st));
   NJ_CUDA(cudaMemsetAsync(active, 1, n, st));
@@ -193,27 +187,42 @@ extern "C" int ngsd_nj_tree(ngsd_ctx *ctx, const double *dist_host, const char *
   k_nj_rowsum<<<(unsigned) n, 256, 0, st>>>(D, n, r, bad);
   for (uint32_t step = 0; step + 3 < n + 0u; step++) {          // n - 3 joins: three nodes are left
     k_nj_rowmin<<<(unsigned) n, 256, 0, st>>>(D, r, active, n, m_dev, rowq, rowj);
-    k_nj_join<<<1, 1024, 0, st>>>(D, r, active, n, m_dev, rowq, rowj, joins, step);
+    k_nj_join<<<1, 1024, 0, st>>>(D, r, active, n, m_dev, rowq, rowj, jdev, step);
   }
   NJ_CUDA(cudaGetLastError());
-  std::vector<NjJoin> hj(n - 3);
+  std::vector<NjJoin> &hj = *joins;
+  hj.resize(n - 3);
   std::vector<uint8_t> hact(n);
   int hbad = 0;
-  if (n > 3) NJ_CUDA(cudaMemcpyAsync(hj.data(), joins, (n - 3) * sizeof(NjJoin), cudaMemcpyDeviceToHost, st));
+  if (n > 3) NJ_CUDA(cudaMemcpyAsync(hj.data(), jdev, (n - 3) * sizeof(NjJoin), cudaMemcpyDeviceToHost, st));
   NJ_CUDA(cudaMemcpyAsync(hact.data(), active, n, cudaMemcpyDeviceToHost, st));
   NJ_CUDA(cudaMemcpyAsync(&hbad, bad, sizeof(int), cudaMemcpyDeviceToHost, st));
   NJ_CUDA(cudaStreamSynchronize(st));
   if (hbad) { release(); ngsd_set_error(ctx, "the distance matrix holds non-finite values (pairs without shared sites?): no tree"); return NGSD_ERR_ARG; }
-  uint64_t rem[3], nr = 0;
+  uint64_t nr = 0;
   for (uint64_t k = 0; k < n && nr < 3; k++)
     if (hact[k]) rem[nr++] = k;
-  double d3[3] = {0, 0, 0};                                     // d(a,b), d(a,c), d(b,c)
+  d3[0] = d3[1] = d3[2] = 0;
   NJ_CUDA(cudaMemcpyAsync(&d3[0], D + rem[0] * n + rem[1], sizeof(double), cudaMemcpyDeviceToHost, st));
   NJ_CUDA(cudaMemcpyAsync(&d3[1], D + rem[0] * n + rem[2], sizeof(double), cudaMemcpyDeviceToHost, st));
   NJ_CUDA(cudaMemcpyAsync(&d3[2], D + rem[1] * n + rem[2], sizeof(double), cudaMemcpyDeviceToHost, st));
   NJ_CUDA(cudaStreamSynchronize(st));
   release();
 #undef NJ_CUDA
+  return NGSD_OK;
+}
+
+extern "C" int ngsd_nj_tree(ngsd_ctx *ctx, const double *dist_host, const char *const *labels, char *newick, uint64_t newick_cap,
+                            uint64_t *newick_len) {
+  if (!ctx || !newick_len) return NGSD_ERR_ARG;
+  if (!ctx->kids.empty()) ctx = ctx->kids[0];
+  const uint64_t n = ctx->n_ind;
+  if (n < 3) { ngsd_set_error(ctx, "a tree needs at least 3 individuals"); return NGSD_ERR_ARG; }
+  if (!dist_host && !ctx->d_out) { ngsd_set_error(ctx, "no distance matrix yet: call ngsd_distances first or pass one"); return NGSD_ERR_STATE; }
+  std::vector<NjJoin> hj;
+  uint64_t rem[3];
+  double d3[3];                                                 // d(a,b), d(a,c), d(b,c)
+  if (int rc = ngsd_nj_joins(ctx, dist_host, ctx->d_out, &hj, rem, d3)) return rc;
   // replay the joins: the subtree living in every slot, as Newick text
   std::vector<std::string> sub(n);
   for (uint64_t k = 0; k < n; k++) sub[k] = labels && labels[k] ? std::string(labels[k]) : "Ind_" + std::to_string(k);
