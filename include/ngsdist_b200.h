@@ -251,6 +251,24 @@ NGSD_API int ngsd_nj_tree(ngsd_ctx *ctx, const double *dist_host, const char *co
 NGSD_API int ngsd_bme_tree(ngsd_ctx *ctx, const double *dist_host, const char *const *labels, char *newick, uint64_t newick_cap,
                            uint64_t *newick_len, uint64_t *n_nni);
 
+/* The trees of a whole batch of matrices -- e.g. every bootstrap replicate -- in one pass per GPU: one launch of each
+ * kernel serves every matrix of a chunk, so a batch pays the launches of one tree while the device work grows with it.
+ * dist_host: n_mat x n_ind x n_ind host matrices (required when n_mat > 0); method NGSD_TREE_NJ (ngsd_nj_tree) or
+ * NGSD_TREE_BME (ngsd_bme_tree).  Tree k is byte-identical to what that call gives for matrix k alone; it is the
+ * NUL-terminated string at newicks + offsets[k] (offsets has n_mat + 1 entries; offsets[n_mat] = bytes used).
+ * status[k] is NGSD_OK, or NGSD_ERR_ARG for a matrix with non-finite entries, whose tree is then the empty string -- the
+ * other trees are still built.  n_nni (may be NULL) receives the interchanges applied per tree (0 for NJ).  When cap is too
+ * small the call returns NGSD_ERR_ARG with the bytes needed in offsets[n_mat].  n_mat == 0 does nothing.
+ * The matrices are processed in chunks sized from the free device memory at call time; chunking changes no result.
+ * A multi-GPU context (ngsd_cfg.n_gpus > 1) deals contiguous slices of the batch to its GPUs, each uploading only its own
+ * matrices; results come back in input order.  A context with a communicator (ngsd_comm_attach) builds trees on its own GPU
+ * only: each rank passes its own matrices. */
+#define NGSD_TREE_NJ 0
+#define NGSD_TREE_BME 1
+NGSD_API int ngsd_trees_batch(ngsd_ctx *ctx, const double *dist_host /* n_mat x n_ind x n_ind */, uint64_t n_mat, int32_t method,
+                              const char *const *labels, char *newicks, uint64_t cap, uint64_t *offsets /* n_mat + 1 */,
+                              uint64_t *n_nni /* n_mat, may be NULL */, int32_t *status /* n_mat */);
+
 /* Bootstrap support of a tree -- the last step of the reference's workflow (README.md:83-98: `raxmlHPC -f b -t main -z
  * boots` on FastME's trees).  HOST code only, no context: for every internal edge of `main_newick`, the number of trees among
  * `rep_newicks[n_reps]` that hold the same bipartition of the leaf labels is written as the node's label

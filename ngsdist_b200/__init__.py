@@ -6,9 +6,9 @@ works without a GPU, but every compute entry point fails loudly when the library
 """
 from .api import (NgsDistError, Params, NgsDistB200, Timing, lib, lib_path, build_library, taus_block_counts, probe_fp64_tflops, probe_int8_tmacs, probe_umma_tmacs,
                   ABI_SYMBOLS, pack_genotypes, PLINK_BED_CODES, comm_unique_id, bind_host_to_device, SHARD_AUTO, SHARD_REPLICATED,
-                  SHARD_SITES, BLANK_SITE, BLANK_SITE_CODE, pack_u20x3, XFER_F32, XFER_U32, XFER_U20X3, tree_support)
+                  SHARD_SITES, BLANK_SITE, BLANK_SITE_CODE, pack_u20x3, XFER_F32, XFER_U32, XFER_U20X3, tree_support, TREE_NJ, TREE_BME)
 from . import api
 
 __all__ = ["tree_support", "NgsDistError", "Params", "NgsDistB200", "Timing", "lib", "lib_path", "build_library", "taus_block_counts",
            "probe_fp64_tflops", "probe_int8_tmacs", "probe_umma_tmacs", "ABI_SYMBOLS", "pack_genotypes", "PLINK_BED_CODES", "comm_unique_id", "bind_host_to_device",
-           "SHARD_AUTO", "SHARD_REPLICATED", "SHARD_SITES", "api"]
+           "SHARD_AUTO", "SHARD_REPLICATED", "SHARD_SITES", "TREE_NJ", "TREE_BME", "api"]

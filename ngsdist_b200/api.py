@@ -22,11 +22,12 @@ ABI_SYMBOLS = [
     "ngsd_probe_fp64_tflops", "ngsd_probe_int8_tmacs", "ngsd_probe_umma_tmacs", "ngsd_host_alloc", "ngsd_host_free", "ngsd_set_tile_shard", "ngsd_device_results", "ngsd_finish",
     "ngsd_distances_batch", "ngsd_comm_unique_id", "ngsd_comm_attach", "ngsd_comm_allgather_operands", "ngsd_comm_reduce_sites", "ngsd_comm_reduce_tiles",
     "ngsd_comm_barrier", "ngsd_comm_stats", "ngsd_bind_host_to_device", "ngsd_deferred_stats", "ngsd_push_sites_packed", "ngsd_nj_tree", "ngsd_tree_support",
-    "ngsd_bme_tree",
+    "ngsd_bme_tree", "ngsd_trees_batch",
 ]
 ABI_VERSION = 2
 COMM_ID_BYTES = 128
 SHARD_AUTO, SHARD_REPLICATED, SHARD_SITES = 0, 1, 2
+TREE_NJ, TREE_BME = 0, 1
 
 
 class NgsDistError(RuntimeError):
@@ -132,11 +133,14 @@ def lib():
                  "ngsd_comm_allgather_operands", "ngsd_comm_reduce_sites", "ngsd_comm_reduce_tiles", "ngsd_comm_barrier", "ngsd_comm_stats",
                  "ngsd_bind_host_to_device", "ngsd_deferred_stats", "ngsd_push_sites_packed", "ngsd_nj_tree", "ngsd_tree_support"):
         getattr(L, name).restype = i32
-    # (a build from before ngsd_bme_tree, named by NGSDIST_B200_LIB for an A/B comparison of the other entry points, lacks it;
-    # build() and tests/test_abi_surface.py require it of this package's library)
+    # (a build from before ngsd_bme_tree or ngsd_trees_batch, named by NGSDIST_B200_LIB for an A/B comparison of the other
+    # entry points, lacks them; build() and tests/test_abi_surface.py require them of this package's library)
     if hasattr(L, "ngsd_bme_tree"):
         L.ngsd_bme_tree.argtypes = [vp, vp, vp, vp, u64, C.POINTER(u64), C.POINTER(u64)]
         L.ngsd_bme_tree.restype = i32
+    if hasattr(L, "ngsd_trees_batch"):
+        L.ngsd_trees_batch.argtypes = [vp, vp, u64, C.c_int32, vp, vp, u64, vp, vp, vp]
+        L.ngsd_trees_batch.restype = i32
     _lib = L
     return L
 
@@ -584,6 +588,40 @@ class NgsDistB200:
                 continue
             self._check(rc)
         self._check(rc)
+
+    def trees_batch(self, dists, method="nj", labels=None):
+        """Trees of a batch of n x n host matrices (ngsd_trees_batch: one pass per GPU for the whole batch), method "nj"
+        (nj_tree) or "bme" (bme_tree).  Returns one (newick, interchanges applied) per matrix, in input order; newick is
+        None for a matrix with non-finite entries.  Every string equals what nj_tree / bme_tree give for that matrix."""
+        n = self.p.n_ind
+        d = np.ascontiguousarray(dists, dtype=np.float64)
+        if d.size == 0:
+            d = d.reshape(0, n, n)
+        assert d.ndim == 3 and d.shape[1:] == (n, n), d.shape
+        m = {"nj": TREE_NJ, "bme": TREE_BME}.get(method)
+        if m is None:
+            raise ValueError("method must be 'nj' or 'bme', not %r" % (method,))
+        n_mat = d.shape[0]
+        lab = None
+        if labels is not None:
+            lab = (C.c_char_p * len(labels))(*[str(x).encode() for x in labels])
+        offsets = np.zeros(n_mat + 1, dtype=np.uint64)
+        nni = np.zeros(max(1, n_mat), dtype=np.uint64)
+        status = np.zeros(max(1, n_mat), dtype=np.int32)
+        cap = n_mat * (64 * n + 1024)
+        for _ in range(2):
+            buf = C.create_string_buffer(max(1, cap))
+            rc = lib().ngsd_trees_batch(self._h, _ptr(d), n_mat, m, lab, buf, cap, _ptr(offsets), _ptr(nni), _ptr(status))
+            if rc == 0 or int(offsets[n_mat]) <= cap:
+                break
+            cap = int(offsets[n_mat])
+        self._check(rc)
+        raw = buf.raw
+        out = []
+        for k in range(n_mat):
+            s = raw[int(offsets[k]):int(offsets[k + 1]) - 1].decode()
+            out.append((s if status[k] == 0 else None, int(nni[k])))
+        return out
 
     def deferred_stats(self):
         """Individual-sites the host's libm decided (knife edges of the reference's comparisons)."""

@@ -2,7 +2,7 @@
 //
 // The reference's workflow (README.md:83-98) hands every matrix to FastME, whose criterion is balanced minimum evolution
 // (BME; Desper & Gascuel 2002): the length of a tree is Pauplin's  L(T) = sum_{i<j} 2^(1 - tau_ij) d_ij,  tau_ij the number
-// of edges between leaves i and j.  ngsd_bme_tree starts from the NJ tree (ngsd_nj_joins, nj.cu), applies the best BME
+// of edges between leaves i and j.  ngsd_bme_tree starts from the NJ tree (the join loop of nj.cu), applies the best BME
 // nearest-neighbour interchange while its gain exceeds 1e-12 M, M = sum_{i<j} 2^(1 - tau_ij) |d_ij| (M = L when no distance is
 // negative), and writes the tree with balanced branch lengths.  Every applied NNI lowers L, so no tree comes back and the
 // loop ends for every finite matrix, whatever the signs of its entries; with M as the scale a matrix of all-equal negative
@@ -63,16 +63,20 @@ struct AddOp { __device__ double operator()(double a, double b) const { return a
 
 // Row p of the DFS layout: R[p][0] = 0 and R[p][q + 1] = sum_{k <= q} P(perm[p], perm[k]), P = 2^-tau d, P_pp = 0, and
 // Rabs[p] = sum_q |P(perm[p], perm[q])|.  The depth of the LCA of positions p < q is min(h[p .. q - 1]): a forward running minimum for q > p, a backward one for q < p.
-__global__ void __launch_bounds__(kThreads) k_bme_rows(const double *__restrict__ D, uint32_t n, const uint32_t *__restrict__ perm,
-                                                       const uint32_t *__restrict__ dep, const uint32_t *__restrict__ h, double *__restrict__ R,
-                                                       double *__restrict__ Rabs) {
+// Slot blockIdx.y is tree act[slot]: its layout is slots[slot], its matrix, prefix rows and Rabs those of the tree.
+__global__ void __launch_bounds__(kThreads) k_bme_rows(const double *__restrict__ D, uint64_t dstride, uint32_t n, const uint32_t *__restrict__ act,
+                                                       const uint32_t *__restrict__ slots, uint64_t lay_words, double *__restrict__ R,
+                                                       uint64_t rstride, double *__restrict__ Rabs_all) {
   __shared__ uint32_t shu[8];
   __shared__ double shd[8];
   __shared__ uint32_t carry_u;
   __shared__ double carry_d;
+  const uint32_t t = act[blockIdx.y];
+  const uint32_t *__restrict__ perm = slots + blockIdx.y * lay_words, *__restrict__ dep = perm + n, *__restrict__ h = perm + 2 * n;
+  double *__restrict__ Rabs = Rabs_all + (uint64_t) t * n;
   const uint32_t p = blockIdx.x;
-  const double *__restrict__ Drow = D + (uint64_t) perm[p] * n;
-  double *__restrict__ Rrow = R + (uint64_t) p * (n + 1);
+  const double *__restrict__ Drow = D + t * dstride + (uint64_t) perm[p] * n;
+  double *__restrict__ Rrow = R + t * rstride + (uint64_t) p * (n + 1);
   const int dp = (int) dep[p];
   double a = 0;
   if (threadIdx.x == 0) { carry_u = 0xFFFFFFFFu; Rrow[0] = 0; Rrow[p + 1] = 0; }
@@ -162,19 +166,23 @@ __device__ __forceinline__ void edge_sums(const double *__restrict__ R, uint32_t
 
 __device__ __forceinline__ bool better(double g, uint32_t k, double g2, uint32_t k2) { return g > g2 || (g == g2 && k < k2); }
 
-// One CTA per internal edge: its two gains, the better of them; the last CTA to finish reduces all edges (and M) into *best
-__global__ void __launch_bounds__(kThreads) k_bme_gains(const double *__restrict__ R, const double *__restrict__ Rabs, uint32_t n,
-                                                        const uint32_t *__restrict__ edges,
-                                                        double *__restrict__ part_g, uint32_t *__restrict__ part_k, uint32_t *__restrict__ ticket,
-                                                        BmeBest *__restrict__ best) {
+// One CTA per internal edge of slot blockIdx.y (tree act[slot]): its two gains, the better of them; the last CTA of the
+// slot to finish reduces the tree's edges (and M) into best[slot]
+__global__ void __launch_bounds__(kThreads) k_bme_gains(const double *__restrict__ R_all, uint64_t rstride, const double *__restrict__ Rabs_all,
+                                                        uint32_t n, const uint32_t *__restrict__ act, const uint32_t *__restrict__ slots,
+                                                        uint64_t lay_words, double *__restrict__ part_g_all, uint32_t *__restrict__ part_k_all,
+                                                        uint32_t *__restrict__ ticket_all, BmeBest *__restrict__ best_all) {
   __shared__ bool last;
   __shared__ double sg[kThreads], sM[kThreads];
   __shared__ uint32_t sk[kThreads];
-  const uint32_t *e = edges + (uint64_t) blockIdx.x * kEdgeWords;
-  const uint32_t v = e[8];
+  const uint32_t t = act[blockIdx.y];
+  const uint32_t *e = slots + blockIdx.y * lay_words + 3 * n + (uint64_t) blockIdx.x * kEdgeWords;
   double s[6];
-  edge_sums(R, n, e, s);
+  edge_sums(R_all + t * rstride, n, e, s);
+  double *__restrict__ part_g = part_g_all + (uint64_t) t * n;
+  uint32_t *__restrict__ part_k = part_k_all + (uint64_t) t * n, *__restrict__ ticket = ticket_all + t;
   if (threadIdx.x == 0) {
+    const uint32_t v = e[8];
     const double g0 = s[0] + s[1] - 2 * (s[2] + s[3]), g1 = s[0] + s[1] - 2 * (s[4] + s[5]);
     const bool one = g1 > g0;
     part_g[blockIdx.x] = one ? g1 : g0;
@@ -192,7 +200,7 @@ __global__ void __launch_bounds__(kThreads) k_bme_gains(const double *__restrict
     const uint32_t k2 = __ldcg(part_k + b);
     if (better(g2, k2, g, k)) { g = g2; k = k2; }
   }
-  for (uint32_t p = threadIdx.x; p < n; p += kThreads) M += __ldcg(Rabs + p);
+  for (uint32_t p = threadIdx.x; p < n; p += kThreads) M += __ldcg(Rabs_all + (uint64_t) t * n + p);
   sg[threadIdx.x] = g; sk[threadIdx.x] = k; sM[threadIdx.x] = M;
   __syncthreads();
   for (int o = kThreads / 2; o > 0; o >>= 1) {
@@ -206,14 +214,19 @@ __global__ void __launch_bounds__(kThreads) k_bme_gains(const double *__restrict
     __syncthreads();
   }
   if (threadIdx.x == 0) {
-    *best = {sg[0], sM[0], sk[0], 0};
+    best_all[blockIdx.y] = {sg[0], sM[0], sk[0], 0};
     *ticket = 0;
   }
 }
 
-// The 2n - 3 balanced lengths: CTA b < n_int is internal edge b, the others the pendant edges in `leaves` order
-__global__ void __launch_bounds__(kThreads) k_bme_lengths(const double *__restrict__ R, uint32_t n, uint32_t n_int, const uint32_t *__restrict__ edges,
-                                                          const uint32_t *__restrict__ leaves, double *__restrict__ len) {
+// The 2n - 3 balanced lengths of slot blockIdx.y (tree act[slot]): CTA b < n_int is internal edge b, the others the pendant
+// edges in `leaves` order
+__global__ void __launch_bounds__(kThreads) k_bme_lengths(const double *__restrict__ R_all, uint64_t rstride, uint32_t n, uint32_t n_int,
+                                                          const uint32_t *__restrict__ act, const uint32_t *__restrict__ slots, uint64_t lay_words,
+                                                          double *__restrict__ len_all) {
+  const double *__restrict__ R = R_all + act[blockIdx.y] * rstride;
+  const uint32_t *__restrict__ edges = slots + blockIdx.y * lay_words + 3 * n, *__restrict__ leaves = edges + (uint64_t) n_int * kEdgeWords;
+  double *__restrict__ len = len_all + blockIdx.y * 2 * (uint64_t) n;
   double s[6];
   if (blockIdx.x < n_int) {
     edge_sums(R, n, edges + (uint64_t) blockIdx.x * kEdgeWords, s);
@@ -245,14 +258,14 @@ struct BmeTree {
   bool leaf(uint32_t w) const { return w < n; }
 
   // NJ joins -> adjacency -> rooted at individual 0
-  void build(uint32_t n_, const std::vector<NjJoin> &joins, const uint64_t rem[3]) {
+  void build(uint32_t n_, const NjJoin *joins, const uint32_t rem[3]) {
     n = n_;
     const uint32_t N = 2 * n - 2;
     std::vector<std::vector<uint32_t>> adj(N);
     std::vector<uint32_t> slot(n);
     for (uint32_t k = 0; k < n; k++) slot[k] = k;
     auto link = [&](uint32_t a, uint32_t b) { adj[a].push_back(b); adj[b].push_back(a); };
-    for (uint32_t t = 0; t < joins.size(); t++) {
+    for (uint32_t t = 0; t + 3 < n; t++) {
       link(n + t, slot[joins[t].i]);
       link(n + t, slot[joins[t].j]);
       slot[joins[t].i] = n + t;
@@ -357,81 +370,12 @@ void append_len(std::string &s, double v) {
   s += b;
 }
 
-struct BmeBuffers {
-  double *D = nullptr, *R = nullptr, *Rabs = nullptr, *part_g = nullptr, *len = nullptr;
-  uint32_t *part_k = nullptr, *ticket = nullptr, *lay = nullptr;
-  BmeBest *best = nullptr;
-  ~BmeBuffers() { cudaFree(D); cudaFree(R); cudaFree(Rabs); cudaFree(part_g); cudaFree(len); cudaFree(part_k); cudaFree(ticket); cudaFree(lay); cudaFree(best); }
-};
-
-}  // namespace
-
-extern "C" int ngsd_bme_tree(ngsd_ctx *ctx, const double *dist_host, const char *const *labels, char *newick, uint64_t newick_cap,
-                             uint64_t *newick_len, uint64_t *n_nni) {
-  if (!ctx || !newick_len) return NGSD_ERR_ARG;
-  if (!ctx->kids.empty()) ctx = ctx->kids[0];
-  const uint64_t n = ctx->n_ind;
-  if (n < 3) { ngsd_set_error(ctx, "a tree needs at least 3 individuals"); return NGSD_ERR_ARG; }
-  if (!dist_host && !ctx->d_out) { ngsd_set_error(ctx, "no distance matrix yet: call ngsd_distances first or pass one"); return NGSD_ERR_STATE; }
-  NGSD_CUDA(ctx, cudaSetDevice(ctx->device));
-  cudaStream_t st = ctx->stream;
-  BmeBuffers b;
-  const double *D = ctx->d_out;                 // read in place; a host matrix is uploaded once, for NJ and the rounds alike
-  if (dist_host) {
-    NGSD_CUDA(ctx, cudaMalloc((void **) &b.D, n * n * sizeof(double)));
-    NGSD_CUDA(ctx, cudaMemcpyAsync(b.D, dist_host, n * n * sizeof(double), cudaMemcpyHostToDevice, st));
-    D = b.D;
-  }
-  std::vector<NjJoin> joins;
-  uint64_t rem[3];
-  double d3[3];
-  if (int rc = ngsd_nj_joins(ctx, nullptr, D, &joins, rem, d3)) return rc;     // (also refuses a non-finite matrix)
-  BmeTree t;
-  t.build((uint32_t) n, joins, rem);
-
-  const uint32_t n_int = (uint32_t) n - 3;
-  // layout words: perm, dep, h (n each), the edges, then the leaves
-  const uint64_t edge_end = 3 * n + (uint64_t) n_int * kEdgeWords, lay_words = edge_end + n * kLeafWords;
-  NGSD_CUDA(ctx, cudaMalloc((void **) &b.R, n * (n + 1) * sizeof(double)));
-  NGSD_CUDA(ctx, cudaMalloc((void **) &b.Rabs, n * sizeof(double)));
-  NGSD_CUDA(ctx, cudaMalloc((void **) &b.part_g, n * sizeof(double)));
-  NGSD_CUDA(ctx, cudaMalloc((void **) &b.part_k, n * sizeof(uint32_t)));
-  NGSD_CUDA(ctx, cudaMalloc((void **) &b.len, 2 * n * sizeof(double)));
-  NGSD_CUDA(ctx, cudaMalloc((void **) &b.ticket, sizeof(uint32_t)));
-  NGSD_CUDA(ctx, cudaMalloc((void **) &b.lay, lay_words * sizeof(uint32_t)));
-  NGSD_CUDA(ctx, cudaMalloc((void **) &b.best, sizeof(BmeBest)));
-  std::vector<uint32_t> hlay(lay_words);
-  uint32_t *hperm = hlay.data(), *hdep = hperm + n, *hh = hperm + 2 * n, *hedges = hperm + 3 * n, *hleaves = hperm + edge_end;
-  const uint32_t *dperm = b.lay, *ddep = b.lay + n, *dh = b.lay + 2 * n, *dedges = b.lay + 3 * n, *dleaves = b.lay + edge_end;
-  BmeBest hbest;
-  NGSD_CUDA(ctx, cudaMemsetAsync(b.ticket, 0, sizeof(uint32_t), st));
-
-  uint64_t applied = 0;
-  for (;;) {
-    t.layout(hperm, hdep, hh);
-    t.edges(hedges);
-    NGSD_CUDA(ctx, cudaMemcpyAsync(b.lay, hperm, edge_end * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-    k_bme_rows<<<(unsigned) n, kThreads, 0, st>>>(D, (uint32_t) n, dperm, ddep, dh, b.R, b.Rabs);
-    if (n_int == 0) break;
-    k_bme_gains<<<n_int, kThreads, 0, st>>>(b.R, b.Rabs, (uint32_t) n, dedges, b.part_g, b.part_k, b.ticket, b.best);
-    NGSD_CUDA(ctx, cudaGetLastError());
-    NGSD_CUDA(ctx, cudaMemcpyAsync(&hbest, b.best, sizeof(BmeBest), cudaMemcpyDeviceToHost, st));
-    NGSD_CUDA(ctx, cudaStreamSynchronize(st));
-    if (!(hbest.gain > 1e-12 * hbest.M)) break;
-    t.nni(hbest.key);
-    applied++;
-  }
-  t.leaves(hleaves);
-  NGSD_CUDA(ctx, cudaMemcpyAsync(b.lay + edge_end, hleaves, n * kLeafWords * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-  k_bme_lengths<<<(unsigned) (n_int + n), kThreads, 0, st>>>(b.R, (uint32_t) n, n_int, dedges, dleaves, b.len);
-  NGSD_CUDA(ctx, cudaGetLastError());
-  std::vector<double> len(n_int + n);
-  NGSD_CUDA(ctx, cudaMemcpyAsync(len.data(), b.len, (n_int + n) * sizeof(double), cudaMemcpyDeviceToHost, st));
-  NGSD_CUDA(ctx, cudaStreamSynchronize(st));
-
-  // length of the edge above every node (individual 0: its pendant edge); the edges were listed in increasing v, skipping u0
+// the Newick string of a refined tree from its 2n - 3 lengths (internal edges in increasing v skipping u0, then the leaves)
+std::string bme_newick(const BmeTree &t, const double *len, const char *const *labels) {
+  const uint32_t n = t.n, n_int = n - 3;
+  // length of the edge above every node (individual 0: its pendant edge)
   std::vector<double> above(2 * n - 2, 0.0);
-  for (uint32_t v = (uint32_t) n, e = 0; v < 2 * n - 2; v++)
+  for (uint32_t v = n, e = 0; v < 2 * n - 2; v++)
     if (v != t.u0) above[v] = len[e++];
   for (uint32_t i = 0; i < n; i++) above[i] = len[n_int + i];
   auto label = [&](uint32_t k) { return labels && labels[k] ? std::string(labels[k]) : "Ind_" + std::to_string(k); };
@@ -451,9 +395,97 @@ extern "C" int ngsd_bme_tree(ngsd_ctx *ctx, const double *dist_host, const char 
     }
   }
   out += ");";
-  if (n_nni) *n_nni = applied;
-  *newick_len = out.size();
-  if (!newick || newick_cap < out.size() + 1) { ngsd_set_error(ctx, "newick buffer too small: %llu bytes needed", (unsigned long long) out.size() + 1); return NGSD_ERR_ARG; }
-  memcpy(newick, out.c_str(), out.size() + 1);
+  return out;
+}
+
+// per tree of a chunk: Rabs, part_g, len (2n) in doubles, part_k, the ticket and BmeBest; the device copy of the layouts
+// (act, then one slot per tree) lives in `lay`, its pinned host twin in `hlay`
+struct BmeBuffers {
+  double *Rabs = nullptr, *part_g = nullptr, *len = nullptr;
+  uint32_t *part_k = nullptr, *ticket = nullptr, *lay = nullptr, *hlay = nullptr;
+  BmeBest *best = nullptr;
+  ~BmeBuffers() { cudaFree(Rabs); cudaFree(part_g); cudaFree(len); cudaFree(part_k); cudaFree(ticket); cudaFree(lay); cudaFree(best); cudaFreeHost(hlay); }
+};
+
+uint64_t lay_words_of(uint64_t n) { return 3 * n + (n - 3) * kEdgeWords + n * kLeafWords; }   // perm, dep, h, the edges, the leaves
+
+}  // namespace
+
+uint64_t ngsd_bme_bytes(uint64_t n) {
+  return n * (4 * sizeof(double) + sizeof(uint32_t)) + sizeof(uint32_t) + sizeof(BmeBest) + (1 + lay_words_of(n)) * sizeof(uint32_t);
+}
+
+// One round: the host applies each active tree's NNI and lays the tree out (one host thread per tree); one upload of all
+// layouts; k_bme_rows and k_bme_gains over every active tree; one copy of a BmeBest per active tree.  A tree whose best
+// gain is not above 1e-12 M leaves the active set with its R rows as its final layout left them; one k_bme_lengths pass
+// over all trees ends the chunk.
+int ngsd_bme_chunk(ngsd_ctx *ctx, const double *D, uint64_t dstride, double *R, uint64_t rstride, const NjBatch &nj, const char *const *labels,
+                   std::string *out, uint64_t *n_nni) {
+  const uint32_t n = nj.n, C = nj.count, n_int = n - 3;
+  const uint64_t edge_end = 3 * (uint64_t) n + (uint64_t) n_int * kEdgeWords, lay_words = lay_words_of(n);
+  cudaStream_t st = ctx->stream;
+  BmeBuffers b;
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.Rabs, (uint64_t) C * n * sizeof(double)));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.part_g, (uint64_t) C * n * sizeof(double)));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.len, (uint64_t) C * 2 * n * sizeof(double)));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.part_k, (uint64_t) C * n * sizeof(uint32_t)));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.ticket, C * sizeof(uint32_t)));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.lay, (C + C * lay_words) * sizeof(uint32_t)));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.best, C * sizeof(BmeBest)));
+  NGSD_CUDA(ctx, cudaMallocHost((void **) &b.hlay, (C + C * lay_words) * sizeof(uint32_t)));
+  NGSD_CUDA(ctx, cudaMemsetAsync(b.ticket, 0, C * sizeof(uint32_t), st));
+  uint32_t *hact = b.hlay, *hslots = b.hlay + C;
+  const uint32_t *dact = b.lay, *dslots = b.lay + C;
+  std::vector<BmeTree> t(C);
+  std::vector<uint32_t> act;                        // the trees still improving, in slot order
+  for (uint32_t k = 0; k < C; k++) {
+    if (nj.bad[k]) continue;
+    t[k].build(n, nj.joins.data() + (uint64_t) k * (n - 2), nj.last[k].rem);
+    act.push_back(k);
+  }
+  const std::vector<uint32_t> good = act;
+  std::vector<BmeBest> hbest(C);
+  while (!act.empty()) {
+    const uint32_t A = (uint32_t) act.size();
+    memcpy(hact, act.data(), A * sizeof(uint32_t));
+    ngsd_parallel_for(A, [&](uint64_t s) {
+      uint32_t *L = hslots + s * lay_words;
+      t[act[s]].layout(L, L + n, L + 2 * n);
+      t[act[s]].edges(L + 3 * n);
+    });
+    NGSD_CUDA(ctx, cudaMemcpyAsync(b.lay, b.hlay, (C + (A - 1) * lay_words + edge_end) * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    k_bme_rows<<<dim3(n, A), kThreads, 0, st>>>(D, dstride, n, dact, dslots, lay_words, R, rstride, b.Rabs);
+    if (n_int == 0) {                               // three leaves: no internal edge, nothing to interchange
+      NGSD_CUDA(ctx, cudaStreamSynchronize(st));
+      break;
+    }
+    k_bme_gains<<<dim3(n_int, A), kThreads, 0, st>>>(R, rstride, b.Rabs, n, dact, dslots, lay_words, b.part_g, b.part_k, b.ticket, b.best);
+    NGSD_CUDA(ctx, cudaGetLastError());
+    NGSD_CUDA(ctx, cudaMemcpyAsync(hbest.data(), b.best, A * sizeof(BmeBest), cudaMemcpyDeviceToHost, st));
+    NGSD_CUDA(ctx, cudaStreamSynchronize(st));
+    uint32_t keep = 0;
+    for (uint32_t s = 0; s < A; s++) {
+      if (!(hbest[s].gain > 1e-12 * hbest[s].M)) continue;
+      t[act[s]].nni(hbest[s].key);
+      n_nni[act[s]]++;
+      act[keep++] = act[s];
+    }
+    act.resize(keep);
+  }
+  const uint32_t G = (uint32_t) good.size();
+  if (G == 0) return NGSD_OK;
+  memcpy(hact, good.data(), G * sizeof(uint32_t));
+  ngsd_parallel_for(G, [&](uint64_t s) {
+    uint32_t *L = hslots + s * lay_words;
+    t[good[s]].edges(L + 3 * n);
+    t[good[s]].leaves(L + edge_end);
+  });
+  NGSD_CUDA(ctx, cudaMemcpyAsync(b.lay, b.hlay, (C + G * lay_words) * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+  k_bme_lengths<<<dim3(n_int + n, G), kThreads, 0, st>>>(R, rstride, n, n_int, dact, dslots, lay_words, b.len);
+  NGSD_CUDA(ctx, cudaGetLastError());
+  std::vector<double> len((uint64_t) G * 2 * n);
+  NGSD_CUDA(ctx, cudaMemcpyAsync(len.data(), b.len, len.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
+  NGSD_CUDA(ctx, cudaStreamSynchronize(st));
+  ngsd_parallel_for(G, [&](uint64_t s) { out[good[s]] = bme_newick(t[good[s]], len.data() + s * 2 * n, labels); });
   return NGSD_OK;
 }

@@ -725,6 +725,16 @@ int ngsd_group_get_timing(ngsd_ctx *parent, ngsd_timing *t) {
   return NGSD_OK;
 }
 
+// ngsd_trees_batch: GPU g builds the trees of matrices [n_mat g / N, n_mat (g + 1) / N), uploading only those
+int ngsd_group_trees(ngsd_ctx *parent, const double *dist_host, uint64_t n_mat, int method, const char *const *labels, std::string *out,
+                     uint64_t *n_nni, int32_t *status) {
+  const uint64_t N = parent->kids.size(), n2 = parent->kids[0]->n_ind * parent->kids[0]->n_ind;
+  return for_each_kid(parent, [&](ngsd_ctx *k, uint32_t g) {
+    const uint64_t b = n_mat * g / N, e = n_mat * (g + 1) / N;
+    return b == e ? NGSD_OK : ngsd_trees_run(k, dist_host + b * n2, nullptr, e - b, method, labels, out + b, n_nni + b, status + b);
+  });
+}
+
 // ------------------------------------------------------------------------------------------------ C ABI ----
 
 extern "C" {

@@ -352,31 +352,47 @@ static int selftest_io(uint64_t n) {
 
 // --tree: the step the reference's workflow (README.md:83-98) runs FastME for -- one neighbour-joining tree per matrix
 // (with --nni_bme: refined by balanced minimum-evolution NNIs, FastME's criterion), computed on the device from the
-// matrix that was just written (after the host's -log / JC69 tail)
-static void write_tree(FILE *fh, ngsd_ctx *ctx, bool bme, const double *d, const std::vector<std::string> &lab, std::vector<std::string> *keep) {
+// matrices as written (after the host's -log / JC69 tail).  The matrices are kept until `cap` of them are held (a fixed
+// host budget, at least one per GPU) and their trees are then built by one ngsd_trees_batch call, written in order.
+struct TreeBatch {
+  FILE *fh = nullptr;
+  ngsd_ctx *ctx = nullptr;
+  int32_t method = NGSD_TREE_NJ;
+  uint64_t n2 = 0, cap = 1, held = 0;
   std::vector<const char *> names;
-  for (auto &l : lab) names.push_back(l.c_str());
-  uint64_t need = 0;
-  std::vector<char> buf(64 * lab.size() + 1024);
-  auto tree = [&]() {
-    return bme ? ngsd_bme_tree(ctx, d, names.data(), buf.data(), buf.size(), &need, nullptr)
-               : ngsd_nj_tree(ctx, d, names.data(), buf.data(), buf.size(), &need);
-  };
-  int rc = tree();
-  if (rc && need + 1 > buf.size()) {
-    buf.resize(need + 1);
-    rc = tree();
+  std::vector<double> mats;
+  std::vector<std::string> *keep = nullptr;
+
+  void add(const double *d) {
+    memcpy(mats.data() + held * n2, d, n2 * sizeof(double));
+    if (++held == cap) flush();
   }
-  if (rc) {
-    fprintf(stderr, "> no tree for this matrix: %s\n", ngsd_last_error(ctx));
-    fprintf(fh, "NA\n");
-    keep->push_back("NA");
-    return;
+  void flush() {
+    if (!held) return;
+    std::vector<uint64_t> offsets(held + 1);
+    std::vector<int32_t> status(held);
+    std::vector<char> buf(held * (64 * names.size() + 1024));
+    int rc = ngsd_trees_batch(ctx, mats.data(), held, method, names.data(), buf.data(), buf.size(), offsets.data(), nullptr, status.data());
+    if (rc && offsets[held] > buf.size()) {
+      buf.resize(offsets[held]);
+      rc = ngsd_trees_batch(ctx, mats.data(), held, method, names.data(), buf.data(), buf.size(), offsets.data(), nullptr, status.data());
+    }
+    if (rc) die("main", ngsd_last_error(ctx));
+    for (uint64_t k = 0; k < held; k++) {
+      if (status[k]) {
+        fprintf(stderr, "> no tree for this matrix: it holds non-finite values (pairs without shared sites?)\n");
+        fprintf(fh, "NA\n");
+        keep->push_back("NA");
+        continue;
+      }
+      const uint64_t len = offsets[k + 1] - offsets[k] - 1;
+      fwrite(buf.data() + offsets[k], 1, len, fh);
+      fputc('\n', fh);
+      keep->emplace_back(buf.data() + offsets[k], len);
+    }
+    held = 0;
   }
-  fwrite(buf.data(), 1, need, fh);
-  fputc('\n', fh);
-  keep->emplace_back(buf.data(), need);
-}
+};
 
 // FILE.support: the main tree with, on every internal edge, the percentage of bootstrap trees that hold it -- what the
 // reference's workflow gets from `raxmlHPC -f b -t main -z boots` (README.md:83-98)
@@ -786,6 +802,18 @@ int main(int argc, char **argv) {
   std::vector<std::string> trees;                                      // --tree: the Newick strings, for FILE.support
   FILE *tree_fh = p.tree ? fopen(p.tree, "w") : nullptr;
   if (p.tree && !tree_fh) die("main", "cannot open tree output file!");
+  TreeBatch tb;
+  if (tree_fh) {
+    const uint64_t budget = 2ull << 30, per = p.n_ind * p.n_ind * sizeof(double);   // host bytes of the held matrices
+    tb.fh = tree_fh;
+    tb.ctx = ctx;
+    tb.method = p.nni_bme ? NGSD_TREE_BME : NGSD_TREE_NJ;
+    tb.n2 = p.n_ind * p.n_ind;
+    tb.cap = std::min<uint64_t>(p.n_boot_rep + 1, std::max<uint64_t>({1, (uint64_t) p.n_gpus, budget / per}));
+    for (auto &l : labels) tb.names.push_back(l.c_str());
+    tb.mats.resize(tb.cap * tb.n2);
+    tb.keep = &trees;
+  }
   static char obuf[1 << 22];
   setvbuf(out_fh, obuf, _IOFBF, sizeof(obuf));
 
@@ -811,7 +839,7 @@ int main(int argc, char **argv) {
         if (host_model) apply_model(dist.data() + q * n2, p.n_ind, p.evol_model, p.n_threads);
         if (p.verbose >= 2) fprintf(stderr, "> Printing distance matrix\n");
         write_matrix(out_fh, labels, dist.data() + q * n2, p.n_ind, p.n_threads);
-        if (tree_fh) write_tree(tree_fh, ctx, p.nni_bme, dist.data() + q * n2, labels, &trees);
+        if (tree_fh) tb.add(dist.data() + q * n2);
       }
       rep += k - 1;
       continue;
@@ -842,10 +870,13 @@ int main(int argc, char **argv) {
     if (host_model) apply_model(dist.data(), p.n_ind, p.evol_model, p.n_threads);
     if (p.verbose >= 2) fprintf(stderr, "> Printing distance matrix\n");
     write_matrix(out_fh, labels, dist.data(), p.n_ind, p.n_threads);
-    if (tree_fh) write_tree(tree_fh, ctx, p.nni_bme, dist.data(), labels, &trees);
+    if (tree_fh) tb.add(dist.data());
   }
   fclose(out_fh);
-  if (tree_fh) fclose(tree_fh);
+  if (tree_fh) {
+    tb.flush();
+    fclose(tree_fh);
+  }
   if (tree_fh && p.n_boot_rep > 0) write_support(p.tree, trees);
   stamp("all matrices written");
   if (p.verbose >= 1) fprintf(stderr, "==> Freeing memory...\n");

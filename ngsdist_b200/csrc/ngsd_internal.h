@@ -6,6 +6,10 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <algorithm>
+#include <atomic>
+#include <string>
+#include <thread>
 #include <vector>
 
 #include "../../include/ngsdist_b200.h"
@@ -240,10 +244,41 @@ cudaError_t ngsd_launch_epilogue_int(ngsd_ctx *ctx, uint32_t n_splits, uint64_t 
 // ---- N4 trees (nj.cu, bme.cu) ----
 // join t merged the subtrees in slots i < j with limb lengths li, lj; the new node takes slot i, slot j retires
 struct NjJoin { uint32_t i, j; double li, lj; };
-// the neighbour-joining loop on the device, on a working copy of dist_host, or of the device matrix dist_dev when
-// dist_host == NULL: the n - 3 joins, the three slots left (in increasing order) and their distances d(a,b), d(a,c),
-// d(b,c).  NGSD_ERR_ARG for a non-finite matrix.
-int ngsd_nj_joins(ngsd_ctx *ctx, const double *dist_host, const double *dist_dev, std::vector<NjJoin> *joins, uint64_t rem[3], double d3[3]);
+// the three slots left after the joins (in increasing order) and their distances d(a,b), d(a,c), d(b,c)
+struct NjLast { uint32_t rem[3], pad; double d3[3]; };
+// the neighbour-joining results of one chunk of matrices
+struct NjBatch {
+  uint32_t n = 0, count = 0;
+  std::vector<NjJoin> joins;    // [count][n - 2]: the n - 3 joins of every matrix
+  std::vector<NjLast> last;     // [count]
+  std::vector<int> bad;         // [count]: the matrix holds non-finite values (no tree)
+};
+// Trees of n_mat matrices on ctx's GPU (nj.cu), in chunks sized from the free device memory: dist_host [n_mat][n][n], or
+// the single device matrix dist_dev.  out[k], n_nni[k] and status[k] (NGSD_ERR_ARG: non-finite, out[k] empty) per matrix.
+// method: NGSD_TREE_NJ / NGSD_TREE_BME.  ngsd_nj_tree, ngsd_bme_tree and ngsd_trees_batch all run through it.
+int ngsd_trees_run(ngsd_ctx *ctx, const double *dist_host, const double *dist_dev, uint64_t n_mat, int method, const char *const *labels,
+                   std::string *out, uint64_t *n_nni, int32_t *status);
+// BME refinement of the NJ trees of one chunk (bme.cu): D the chunk's input matrices (device, stride dstride), R NJ's
+// working copies, reused for the prefix sums (n (n + 1) doubles each, stride rstride); skips the matrices nj marks bad
+int ngsd_bme_chunk(ngsd_ctx *ctx, const double *D, uint64_t dstride, double *R, uint64_t rstride, const NjBatch &nj, const char *const *labels,
+                   std::string *out, uint64_t *n_nni);
+uint64_t ngsd_bme_bytes(uint64_t n);   // device bytes of one matrix in ngsd_bme_chunk besides D and R
+
+// fn(0) .. fn(count - 1) on up to one host thread per core (inline for a single item); every item is independent
+template <typename F>
+void ngsd_parallel_for(uint64_t count, F fn) {
+  const uint64_t T = std::min<uint64_t>({count, (uint64_t) std::max(1u, std::thread::hardware_concurrency()), 64});
+  if (T <= 1) {
+    for (uint64_t k = 0; k < count; k++) fn(k);
+    return;
+  }
+  std::atomic<uint64_t> next{0};
+  auto work = [&]() { for (uint64_t k; (k = next.fetch_add(1)) < count;) fn(k); };
+  std::vector<std::thread> th;
+  for (uint64_t t = 1; t < T; t++) th.emplace_back(work);
+  work();
+  for (auto &x : th) x.join();
+}
 
 // ---- multi-GPU (comm.cu) ----
 extern "C" int ngsd_frontend_resolve(ngsd_ctx *ctx);      // api.cu: knife-edge triples -> host libm -> k_patch
@@ -260,3 +295,5 @@ int ngsd_group_distances(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n
 int ngsd_group_distances_batch(ngsd_ctx *ctx, const uint32_t *block_counts, uint64_t n_rep, uint64_t n_blocks, uint64_t block_size, double *out);
 int ngsd_group_get_posteriors(ngsd_ctx *ctx, double *P_host, uint8_t *miss_host);
 int ngsd_group_get_timing(ngsd_ctx *ctx, ngsd_timing *t);
+int ngsd_group_trees(ngsd_ctx *ctx, const double *dist_host, uint64_t n_mat, int method, const char *const *labels, std::string *out,
+                     uint64_t *n_nni, int32_t *status);   // contiguous slices of the batch, one per GPU, through ngsd_trees_run

@@ -16,9 +16,16 @@
 // (one block: best row, limb lengths, the O(n) update of row / column u and of the row sums, the join record).  The host
 // replays the n - 3 join records into Newick once at the end.  Sum over joins of the active m^2 entries = n^3 / 3 reads:
 // 21 GB at n = 2 000 (4 ms of HBM time; launch-bound at ~8 us per join), 21 TB at n = 20 000.
+//
+// Batches (ngsd_trees_batch; ngsd_nj_tree and ngsd_bme_tree are batches of one): every kernel takes its matrix from
+// blockIdx.y and each matrix has its own working copy, row sums, active flags, node count, row minima, join records and
+// `bad` flag, so one loop of n - 3 steps builds the trees of a whole chunk of matrices with the launches of one tree.
+// The arithmetic, block sizes and tie rules of every matrix are those of a single tree, so every tree is byte-identical
+// to the one the matrix gives alone.  A chunk is as many matrices as fit in the free device memory at call time.
 #include <math.h>
 #include <string.h>
 
+#include <algorithm>
 #include <string>
 #include <unordered_map>
 #include <vector>
@@ -27,9 +34,12 @@
 
 namespace {
 
-__global__ void __launch_bounds__(256) k_nj_rowsum(const double *__restrict__ D, uint64_t n, double *__restrict__ r, int *__restrict__ bad) {
+__global__ void __launch_bounds__(256) k_nj_rowsum(const double *__restrict__ W, uint64_t ws, uint64_t n, double *__restrict__ r_all,
+                                                   int *__restrict__ bad) {
   __shared__ double red[256];
   const uint64_t i = blockIdx.x;
+  const double *__restrict__ D = W + blockIdx.y * ws;
+  double *__restrict__ r = r_all + blockIdx.y * n;
   double s = 0;
   int nf = 0;
   for (uint64_t k = threadIdx.x; k < n; k += 256) {
@@ -43,16 +53,24 @@ __global__ void __launch_bounds__(256) k_nj_rowsum(const double *__restrict__ D,
     __syncthreads();
   }
   if (threadIdx.x == 0) r[i] = red[0];
-  if (nf) atomicOr(bad, 1);
+  if (nf) atomicOr(bad + blockIdx.y, 1);
 }
 
 // (Q, j) of the best partner j > i of row i; rows that are retired or have no partner report +inf
-__global__ void __launch_bounds__(256) k_nj_rowmin(const double *__restrict__ D, const double *__restrict__ r, const uint8_t *__restrict__ active,
-                                                   uint64_t n, const uint32_t *__restrict__ m_ptr, double *__restrict__ rowq, uint32_t *__restrict__ rowj) {
+__global__ void __launch_bounds__(256, 6) k_nj_rowmin(const double *__restrict__ W, uint64_t ws, const double *__restrict__ r_all,
+                                                   const uint8_t *__restrict__ active_all, uint64_t n, const uint32_t *__restrict__ m_all,
+                                                   double *__restrict__ rowq_all, uint32_t *__restrict__ rowj_all) {
   __shared__ double sq[256];
   __shared__ uint32_t sj[256];
   const uint64_t i = blockIdx.x;
-  const uint32_t m = *m_ptr;
+  const double *__restrict__ D = W + blockIdx.y * ws;
+  const double *__restrict__ r = r_all + blockIdx.y * n;
+  const uint8_t *__restrict__ active = active_all + blockIdx.y * n;
+  if (!active[i]) {                                            // a retired row: no partner, and no block reduction to wait for
+    if (threadIdx.x == 0) { rowq_all[blockIdx.y * n + i] = INFINITY; rowj_all[blockIdx.y * n + i] = 0xFFFFFFFFu; }
+    return;
+  }
+  const uint32_t m = m_all[blockIdx.y];
   const double mm2 = (double) (m - 2);
   double best = INFINITY;
   uint32_t bj = 0xFFFFFFFFu;
@@ -65,7 +83,7 @@ __global__ void __launch_bounds__(256) k_nj_rowmin(const double *__restrict__ D,
     for (uint64_t k = threadIdx.x; k < i; k += 256) f |= active[k];
     skip_row = __syncthreads_or(f) != 0;
   }
-  if (active[i] && !skip_row) {
+  if (!skip_row) {
     const double ri = r[i];
     for (uint64_t j = i + 1 + threadIdx.x; j < n; j += 256) {
       if (!active[j]) continue;
@@ -84,16 +102,22 @@ __global__ void __launch_bounds__(256) k_nj_rowmin(const double *__restrict__ D,
     }
     __syncthreads();
   }
-  if (threadIdx.x == 0) { rowq[i] = sq[0]; rowj[i] = sj[0]; }
+  if (threadIdx.x == 0) { rowq_all[blockIdx.y * n + i] = sq[0]; rowj_all[blockIdx.y * n + i] = sj[0]; }
 }
 
-__global__ void __launch_bounds__(1024) k_nj_join(double *__restrict__ D, double *__restrict__ r, uint8_t *__restrict__ active, uint64_t n,
-                                                  uint32_t *__restrict__ m_ptr, const double *__restrict__ rowq, const uint32_t *__restrict__ rowj,
-                                                  NjJoin *__restrict__ joins, uint32_t step) {
+// one block per matrix (blockIdx.x)
+__global__ void __launch_bounds__(1024) k_nj_join(double *__restrict__ W, uint64_t ws, double *__restrict__ r_all, uint8_t *__restrict__ active_all,
+                                                  uint64_t n, uint32_t *__restrict__ m_all, const double *__restrict__ rowq_all,
+                                                  const uint32_t *__restrict__ rowj_all, NjJoin *__restrict__ joins_all, uint32_t step) {
   __shared__ double sq[1024];
   __shared__ uint32_t si[1024];
   __shared__ double sred[1024];
   __shared__ uint32_t pick[2];
+  double *__restrict__ D = W + blockIdx.x * ws;
+  double *__restrict__ r = r_all + blockIdx.x * n;
+  uint8_t *__restrict__ active = active_all + blockIdx.x * n;
+  const double *__restrict__ rowq = rowq_all + blockIdx.x * n;
+  const uint32_t *__restrict__ rowj = rowj_all + blockIdx.x * n;
   double best = INFINITY;
   uint32_t bi = 0xFFFFFFFFu;
   for (uint64_t i = threadIdx.x; i < n; i += 1024) {
@@ -115,7 +139,7 @@ __global__ void __launch_bounds__(1024) k_nj_join(double *__restrict__ D, double
   __syncthreads();
   const uint64_t i = pick[0], j = pick[1];
   if (i == 0xFFFFFFFFu || j == 0xFFFFFFFFu) return;           // (non-finite input: reported by the caller)
-  const uint32_t m = *m_ptr;
+  const uint32_t m = m_all[blockIdx.x];
   const double dij = D[i * n + j], ri = r[i], rj = r[j];
   double ru = 0;
   for (uint64_t k = threadIdx.x; k < n; k += 1024) {
@@ -135,11 +159,77 @@ __global__ void __launch_bounds__(1024) k_nj_join(double *__restrict__ D, double
   }
   if (threadIdx.x == 0) {
     const double li = dij / 2 + (ri - rj) / (2 * (double) (m - 2));
-    joins[step] = {(uint32_t) i, (uint32_t) j, li, dij - li};
+    joins_all[blockIdx.x * (n - 2) + step] = {(uint32_t) i, (uint32_t) j, li, dij - li};
     r[i] = sred[0];
     active[j] = 0;
-    *m_ptr = m - 1;
+    m_all[blockIdx.x] = m - 1;
   }
+}
+
+// one warp per matrix: the three slots left (in increasing order) and their distances
+__global__ void __launch_bounds__(32) k_nj_last(const double *__restrict__ W, uint64_t ws, const uint8_t *__restrict__ active_all, uint64_t n,
+                                                NjLast *__restrict__ last) {
+  const double *__restrict__ D = W + blockIdx.x * ws;
+  const uint8_t *__restrict__ active = active_all + blockIdx.x * n;
+  uint32_t a = 0, b = 0, c = 0, found = 0;
+  for (uint64_t base = 0; base < n && found < 3; base += 32) {
+    const uint64_t k = base + threadIdx.x;
+    uint32_t bits = __ballot_sync(0xFFFFFFFFu, k < n && active[k]);
+    for (; bits && found < 3; bits &= bits - 1, found++) {
+      const uint32_t x = (uint32_t) base + __ffs(bits) - 1;
+      if (found == 0) a = x; else if (found == 1) b = x; else c = x;
+    }
+  }
+  if (threadIdx.x == 0) last[blockIdx.x] = {{a, b, c}, 0, {D[a * n + b], D[a * n + c], D[b * n + c]}};
+}
+
+struct NjBuffers {
+  double *r = nullptr, *rowq = nullptr;
+  uint32_t *rowj = nullptr, *m = nullptr;
+  uint8_t *active = nullptr;
+  NjJoin *joins = nullptr;
+  NjLast *last = nullptr;
+  int *bad = nullptr;
+  ~NjBuffers() { cudaFree(r); cudaFree(rowq); cudaFree(rowj); cudaFree(m); cudaFree(active); cudaFree(joins); cudaFree(last); cudaFree(bad); }
+};
+
+// device bytes of one matrix besides its working copy (NjBuffers)
+uint64_t nj_bytes(uint64_t n) { return n * (2 * sizeof(double) + sizeof(uint32_t) + 1) + (n - 2) * sizeof(NjJoin) + sizeof(NjLast) + 8; }
+
+// the join loop over `count` working copies (device, stride ws), each overwritten: one launch per kernel and step serves them all
+int nj_chunk(ngsd_ctx *ctx, double *W, uint64_t ws, uint32_t count, NjBatch *out) {
+  const uint64_t n = ctx->n_ind;
+  cudaStream_t st = ctx->stream;
+  NjBuffers b;
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.r, count * n * sizeof(double)));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.rowq, count * n * sizeof(double)));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.rowj, count * n * sizeof(uint32_t)));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.m, count * sizeof(uint32_t)));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.active, count * n));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.joins, count * (n - 2) * sizeof(NjJoin)));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.last, count * sizeof(NjLast)));
+  NGSD_CUDA(ctx, cudaMalloc((void **) &b.bad, count * sizeof(int)));
+  const std::vector<uint32_t> m0(count, (uint32_t) n);
+  NGSD_CUDA(ctx, cudaMemcpyAsync(b.m, m0.data(), count * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+  NGSD_CUDA(ctx, cudaMemsetAsync(b.active, 1, count * n, st));
+  NGSD_CUDA(ctx, cudaMemsetAsync(b.bad, 0, count * sizeof(int), st));
+  k_nj_rowsum<<<dim3((unsigned) n, count), 256, 0, st>>>(W, ws, n, b.r, b.bad);
+  for (uint32_t step = 0; step + 3 < n + 0u; step++) {          // n - 3 joins: three nodes are left
+    k_nj_rowmin<<<dim3((unsigned) n, count), 256, 0, st>>>(W, ws, b.r, b.active, n, b.m, b.rowq, b.rowj);
+    k_nj_join<<<count, 1024, 0, st>>>(W, ws, b.r, b.active, n, b.m, b.rowq, b.rowj, b.joins, step);
+  }
+  k_nj_last<<<count, 32, 0, st>>>(W, ws, b.active, n, b.last);
+  NGSD_CUDA(ctx, cudaGetLastError());
+  out->n = (uint32_t) n;
+  out->count = count;
+  out->joins.resize(count * (n - 2));
+  out->last.resize(count);
+  out->bad.resize(count);
+  NGSD_CUDA(ctx, cudaMemcpyAsync(out->joins.data(), b.joins, count * (n - 2) * sizeof(NjJoin), cudaMemcpyDeviceToHost, st));
+  NGSD_CUDA(ctx, cudaMemcpyAsync(out->last.data(), b.last, count * sizeof(NjLast), cudaMemcpyDeviceToHost, st));
+  NGSD_CUDA(ctx, cudaMemcpyAsync(out->bad.data(), b.bad, count * sizeof(int), cudaMemcpyDeviceToHost, st));
+  NGSD_CUDA(ctx, cudaStreamSynchronize(st));
+  return NGSD_OK;
 }
 
 void append_len(std::string &s, double v) {
@@ -148,105 +238,139 @@ void append_len(std::string &s, double v) {
   s += b;
 }
 
+// replay the joins of matrix k: the subtree living in every slot, as Newick text
+std::string nj_newick(const NjBatch &nj, uint32_t k, const char *const *labels) {
+  const uint32_t n = nj.n;
+  std::vector<std::string> sub(n);
+  for (uint64_t i = 0; i < n; i++) sub[i] = labels && labels[i] ? std::string(labels[i]) : "Ind_" + std::to_string(i);
+  for (const NjJoin *jn = nj.joins.data() + (uint64_t) k * (n - 2), *e = jn + (n - 3); jn != e; jn++) {
+    std::string s = "(" + sub[jn->i];
+    append_len(s, jn->li);
+    s += "," + sub[jn->j];
+    append_len(s, jn->lj);
+    s += ")";
+    sub[jn->i].swap(s);
+    sub[jn->j].clear();
+  }
+  const NjLast &l = nj.last[k];
+  const double *d3 = l.d3;                                      // d(a,b), d(a,c), d(b,c)
+  const double la = (d3[0] + d3[1] - d3[2]) / 2, lb = (d3[0] + d3[2] - d3[1]) / 2, lc = (d3[1] + d3[2] - d3[0]) / 2;
+  std::string out = "(" + sub[l.rem[0]];
+  append_len(out, la);
+  out += "," + sub[l.rem[1]];
+  append_len(out, lb);
+  out += "," + sub[l.rem[2]];
+  append_len(out, lc);
+  out += ");";
+  return out;
+}
+
+// one tree through the batch driver: ngsd_nj_tree and ngsd_bme_tree
+int one_tree(ngsd_ctx *ctx, const double *dist_host, int method, const char *const *labels, char *newick, uint64_t newick_cap,
+             uint64_t *newick_len, uint64_t *n_nni) {
+  if (!ctx || !newick_len) return NGSD_ERR_ARG;
+  if (!ctx->kids.empty()) ctx = ctx->kids[0];
+  if (ctx->n_ind < 3) { ngsd_set_error(ctx, "a tree needs at least 3 individuals"); return NGSD_ERR_ARG; }
+  if (!dist_host && !ctx->d_out) { ngsd_set_error(ctx, "no distance matrix yet: call ngsd_distances first or pass one"); return NGSD_ERR_STATE; }
+  std::string out;
+  uint64_t k = 0;
+  int32_t status = NGSD_OK;
+  if (int rc = ngsd_trees_run(ctx, dist_host, dist_host ? nullptr : ctx->d_out, 1, method, labels, &out, &k, &status)) return rc;
+  if (status) { ngsd_set_error(ctx, "the distance matrix holds non-finite values (pairs without shared sites?): no tree"); return status; }
+  if (n_nni) *n_nni = k;
+  *newick_len = out.size();
+  if (!newick || newick_cap < out.size() + 1) { ngsd_set_error(ctx, "newick buffer too small: %llu bytes needed", (unsigned long long) out.size() + 1); return NGSD_ERR_ARG; }
+  memcpy(newick, out.c_str(), out.size() + 1);
+  return NGSD_OK;
+}
+
 }  // namespace
 
-// the join loop, shared by ngsd_nj_tree and ngsd_bme_tree (bme.cu)
-int ngsd_nj_joins(ngsd_ctx *ctx, const double *dist_host, const double *dist_dev, std::vector<NjJoin> *joins, uint64_t rem[3], double d3[3]) {
-  const uint64_t n = ctx->n_ind;
+int ngsd_trees_run(ngsd_ctx *ctx, const double *dist_host, const double *dist_dev, uint64_t n_mat, int method, const char *const *labels,
+                   std::string *out, uint64_t *n_nni, int32_t *status) {
+  const uint64_t n = ctx->n_ind, n2 = n * n;
+  const bool bme = method == NGSD_TREE_BME;
   NGSD_CUDA(ctx, cudaSetDevice(ctx->device));
-  double *D = nullptr, *r = nullptr, *rowq = nullptr;
-  uint32_t *rowj = nullptr, *m_dev = nullptr;
-  uint8_t *active = nullptr;
-  NjJoin *jdev = nullptr;
-  int *bad = nullptr;
-  auto release = [&]() { cudaFree(D); cudaFree(r); cudaFree(rowq); cudaFree(rowj); cudaFree(m_dev); cudaFree(active); cudaFree(jdev); cudaFree(bad); };
-#define NJ_CUDA(call)                                                                                   \
-  do {                                                                                                  \
-    cudaError_t e_ = (call);                                                                            \
-    if (e_ != cudaSuccess) {                                                                            \
-      ngsd_set_error(ctx, "CUDA error: %s (%s:%d: %s)", cudaGetErrorString(e_), __FILE__, __LINE__, #call); \
-      release();                                                                                        \
-      return NGSD_ERR_CUDA;                                                                             \
-    }                                                                                                   \
-  } while (0)
-  NJ_CUDA(cudaMalloc((void **) &D, n * n * sizeof(double)));
-  NJ_CUDA(cudaMalloc((void **) &r, n * sizeof(double)));
-  NJ_CUDA(cudaMalloc((void **) &rowq, n * sizeof(double)));
-  NJ_CUDA(cudaMalloc((void **) &rowj, n * sizeof(uint32_t)));
-  NJ_CUDA(cudaMalloc((void **) &m_dev, sizeof(uint32_t)));
-  NJ_CUDA(cudaMalloc((void **) &active, n));
-  NJ_CUDA(cudaMalloc((void **) &jdev, (n - 2) * sizeof(NjJoin)));
-  NJ_CUDA(cudaMalloc((void **) &bad, sizeof(int)));
+  // BME reuses NJ's working copy for its n (n + 1) prefix sums, and keeps the input matrix (a host matrix is uploaded once)
+  const uint64_t ws = bme ? n * (n + 1) : n2;
+  const bool upload_d = bme && dist_host;
+  const uint64_t per = ws * sizeof(double) + (upload_d ? n2 * sizeof(double) : 0) + nj_bytes(n) + (bme ? ngsd_bme_bytes(n) : 0);
+  size_t free_b = 0, total_b = 0;
+  NGSD_CUDA(ctx, cudaMemGetInfo(&free_b, &total_b));
+  const uint64_t reserve = 256ull << 20;                       // allocation granularity and whatever else the device needs meanwhile
+  const uint64_t fit = free_b > reserve ? (free_b - reserve) / per : 0;
+  const uint32_t C = (uint32_t) std::max<uint64_t>(1, std::min<uint64_t>({fit, n_mat, 65535}));   // (65535: gridDim.y)
+  struct Chunk {
+    double *W = nullptr, *D = nullptr;
+    ~Chunk() { cudaFree(W); cudaFree(D); }
+  } c;
+  NGSD_CUDA(ctx, cudaMalloc((void **) &c.W, C * ws * sizeof(double)));
+  if (upload_d) NGSD_CUDA(ctx, cudaMalloc((void **) &c.D, C * n2 * sizeof(double)));
   cudaStream_t st = ctx->stream;
-  if (dist_host) NJ_CUDA(cudaMemcpyAsync(D, dist_host, n * n * sizeof(double), cudaMemcpyHostToDevice, st));
-  else NJ_CUDA(cudaMemcpyAsync(D, dist_dev, n * n * sizeof(double), cudaMemcpyDeviceToDevice, st));
-  const uint32_t m0 = (uint32_t) n;
-  NJ_CUDA(cudaMemcpyAsync(m_dev, &m0, sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-  NJ_CUDA(cudaMemsetAsync(active, 1, n, st));
-  NJ_CUDA(cudaMemsetAsync(bad, 0, sizeof(int), st));
-  k_nj_rowsum<<<(unsigned) n, 256, 0, st>>>(D, n, r, bad);
-  for (uint32_t step = 0; step + 3 < n + 0u; step++) {          // n - 3 joins: three nodes are left
-    k_nj_rowmin<<<(unsigned) n, 256, 0, st>>>(D, r, active, n, m_dev, rowq, rowj);
-    k_nj_join<<<1, 1024, 0, st>>>(D, r, active, n, m_dev, rowq, rowj, jdev, step);
+  for (uint64_t c0 = 0; c0 < n_mat; c0 += C) {
+    const uint32_t cnt = (uint32_t) std::min<uint64_t>(C, n_mat - c0);
+    const double *src = dist_host ? dist_host + c0 * n2 : dist_dev;   // (a device matrix comes alone)
+    if (upload_d) NGSD_CUDA(ctx, cudaMemcpyAsync(c.D, src, cnt * n2 * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (dist_host && !bme) {
+      NGSD_CUDA(ctx, cudaMemcpyAsync(c.W, src, cnt * n2 * sizeof(double), cudaMemcpyHostToDevice, st));
+    } else {
+      const double *D = upload_d ? c.D : dist_dev;
+      for (uint32_t k = 0; k < cnt; k++)
+        NGSD_CUDA(ctx, cudaMemcpyAsync(c.W + k * ws, D + k * n2, n2 * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    }
+    NjBatch nj;
+    if (int rc = nj_chunk(ctx, c.W, ws, cnt, &nj)) return rc;
+    for (uint32_t k = 0; k < cnt; k++) {
+      status[c0 + k] = nj.bad[k] ? NGSD_ERR_ARG : NGSD_OK;
+      n_nni[c0 + k] = 0;
+      out[c0 + k].clear();
+    }
+    if (bme) {
+      if (int rc = ngsd_bme_chunk(ctx, upload_d ? c.D : dist_dev, n2, c.W, ws, nj, labels, out + c0, n_nni + c0)) return rc;
+    } else {
+      ngsd_parallel_for(cnt, [&](uint64_t k) { if (!nj.bad[k]) out[c0 + k] = nj_newick(nj, (uint32_t) k, labels); });
+    }
   }
-  NJ_CUDA(cudaGetLastError());
-  std::vector<NjJoin> &hj = *joins;
-  hj.resize(n - 3);
-  std::vector<uint8_t> hact(n);
-  int hbad = 0;
-  if (n > 3) NJ_CUDA(cudaMemcpyAsync(hj.data(), jdev, (n - 3) * sizeof(NjJoin), cudaMemcpyDeviceToHost, st));
-  NJ_CUDA(cudaMemcpyAsync(hact.data(), active, n, cudaMemcpyDeviceToHost, st));
-  NJ_CUDA(cudaMemcpyAsync(&hbad, bad, sizeof(int), cudaMemcpyDeviceToHost, st));
-  NJ_CUDA(cudaStreamSynchronize(st));
-  if (hbad) { release(); ngsd_set_error(ctx, "the distance matrix holds non-finite values (pairs without shared sites?): no tree"); return NGSD_ERR_ARG; }
-  uint64_t nr = 0;
-  for (uint64_t k = 0; k < n && nr < 3; k++)
-    if (hact[k]) rem[nr++] = k;
-  d3[0] = d3[1] = d3[2] = 0;
-  NJ_CUDA(cudaMemcpyAsync(&d3[0], D + rem[0] * n + rem[1], sizeof(double), cudaMemcpyDeviceToHost, st));
-  NJ_CUDA(cudaMemcpyAsync(&d3[1], D + rem[0] * n + rem[2], sizeof(double), cudaMemcpyDeviceToHost, st));
-  NJ_CUDA(cudaMemcpyAsync(&d3[2], D + rem[1] * n + rem[2], sizeof(double), cudaMemcpyDeviceToHost, st));
-  NJ_CUDA(cudaStreamSynchronize(st));
-  release();
-#undef NJ_CUDA
+  return NGSD_OK;
+}
+
+extern "C" int ngsd_trees_batch(ngsd_ctx *ctx, const double *dist_host, uint64_t n_mat, int32_t method, const char *const *labels, char *newicks,
+                                uint64_t cap, uint64_t *offsets, uint64_t *n_nni, int32_t *status) {
+  if (!ctx) return NGSD_ERR_ARG;
+  if (n_mat == 0) {
+    if (offsets) offsets[0] = 0;
+    return NGSD_OK;
+  }
+  if (!dist_host) { ngsd_set_error(ctx, "no distance matrices: dist_host is NULL"); return NGSD_ERR_ARG; }
+  if (!offsets || !status) { ngsd_set_error(ctx, "offsets and status are required"); return NGSD_ERR_ARG; }
+  if (method != NGSD_TREE_NJ && method != NGSD_TREE_BME) { ngsd_set_error(ctx, "unknown tree method %d (NGSD_TREE_NJ or NGSD_TREE_BME)", (int) method); return NGSD_ERR_ARG; }
+  const uint64_t n = (ctx->kids.empty() ? ctx : ctx->kids[0])->n_ind;
+  if (n < 3) { ngsd_set_error(ctx, "a tree needs at least 3 individuals"); return NGSD_ERR_ARG; }
+  std::vector<std::string> out(n_mat);
+  std::vector<uint64_t> nni(n_mat, 0);
+  const int rc = ctx->kids.empty() ? ngsd_trees_run(ctx, dist_host, nullptr, n_mat, method, labels, out.data(), nni.data(), status)
+                                   : ngsd_group_trees(ctx, dist_host, n_mat, method, labels, out.data(), nni.data(), status);
+  if (rc) return rc;
+  uint64_t pos = 0;
+  for (uint64_t k = 0; k < n_mat; k++) {
+    offsets[k] = pos;
+    pos += out[k].size() + 1;
+  }
+  offsets[n_mat] = pos;
+  if (n_nni) memcpy(n_nni, nni.data(), n_mat * sizeof(uint64_t));
+  if (!newicks || cap < pos) { ngsd_set_error(ctx, "newick buffer too small: %llu bytes needed", (unsigned long long) pos); return NGSD_ERR_ARG; }
+  for (uint64_t k = 0; k < n_mat; k++) memcpy(newicks + offsets[k], out[k].c_str(), out[k].size() + 1);
   return NGSD_OK;
 }
 
 extern "C" int ngsd_nj_tree(ngsd_ctx *ctx, const double *dist_host, const char *const *labels, char *newick, uint64_t newick_cap,
                             uint64_t *newick_len) {
-  if (!ctx || !newick_len) return NGSD_ERR_ARG;
-  if (!ctx->kids.empty()) ctx = ctx->kids[0];
-  const uint64_t n = ctx->n_ind;
-  if (n < 3) { ngsd_set_error(ctx, "a tree needs at least 3 individuals"); return NGSD_ERR_ARG; }
-  if (!dist_host && !ctx->d_out) { ngsd_set_error(ctx, "no distance matrix yet: call ngsd_distances first or pass one"); return NGSD_ERR_STATE; }
-  std::vector<NjJoin> hj;
-  uint64_t rem[3];
-  double d3[3];                                                 // d(a,b), d(a,c), d(b,c)
-  if (int rc = ngsd_nj_joins(ctx, dist_host, ctx->d_out, &hj, rem, d3)) return rc;
-  // replay the joins: the subtree living in every slot, as Newick text
-  std::vector<std::string> sub(n);
-  for (uint64_t k = 0; k < n; k++) sub[k] = labels && labels[k] ? std::string(labels[k]) : "Ind_" + std::to_string(k);
-  for (const NjJoin &jn : hj) {
-    std::string s = "(" + sub[jn.i];
-    append_len(s, jn.li);
-    s += "," + sub[jn.j];
-    append_len(s, jn.lj);
-    s += ")";
-    sub[jn.i].swap(s);
-    sub[jn.j].clear();
-  }
-  const double la = (d3[0] + d3[1] - d3[2]) / 2, lb = (d3[0] + d3[2] - d3[1]) / 2, lc = (d3[1] + d3[2] - d3[0]) / 2;
-  std::string out = "(" + sub[rem[0]];
-  append_len(out, la);
-  out += "," + sub[rem[1]];
-  append_len(out, lb);
-  out += "," + sub[rem[2]];
-  append_len(out, lc);
-  out += ");";
-  *newick_len = out.size();
-  if (!newick || newick_cap < out.size() + 1) { ngsd_set_error(ctx, "newick buffer too small: %llu bytes needed", (unsigned long long) out.size() + 1); return NGSD_ERR_ARG; }
-  memcpy(newick, out.c_str(), out.size() + 1);
-  return NGSD_OK;
+  return one_tree(ctx, dist_host, NGSD_TREE_NJ, labels, newick, newick_cap, newick_len, nullptr);
+}
+
+extern "C" int ngsd_bme_tree(ngsd_ctx *ctx, const double *dist_host, const char *const *labels, char *newick, uint64_t newick_cap,
+                             uint64_t *newick_len, uint64_t *n_nni) {
+  return one_tree(ctx, dist_host, NGSD_TREE_BME, labels, newick, newick_cap, newick_len, n_nni);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
