@@ -204,6 +204,37 @@ void ngsd_default_cfg(ngsd_cfg *cfg) {
 
 const char *ngsd_last_error(const ngsd_ctx *ctx) { return ctx ? ctx->err : g_create_err; }
 
+// Coefficients of the pdel two-plane form (ngsd_internal.h) for score S (S[g1][g2] = score[3*g1 + g2], g1 the row
+// individual's genotype), in double with Cramer's rule so that dyadic scores give exact coefficients:
+//   V = Z^T S Z,  r = V^-1 Z^T S c,  l = V^-T Z^T S^T c,  kappa = c^T S c - l^T V r     (c = (0,0,1)).
+// Taken only when every coefficient is finite, max(|l|, |r|) <= 4 and |kappa| <= 4 max|S|: that keeps the per-site
+// terms within a small multiple of the three-plane ones and rejects singular V (--avg_nuc_dist: S has rank 1 on the
+// zero-sum plane), near-singular and non-finite scores, which keep the three planes.
+static bool pdel2_coefficients(const double *score, double l[2], double r[2], double V[4], double *kappa) {
+  auto S = [&](int a, int b) { return score[3 * a + b]; };
+  // S Z: columns S e_g - S e_2 (g = 0, 1); then Z^T (S Z): rows e_g - e_2
+  double SZ[3][2];
+  for (int a = 0; a < 3; a++)
+    for (int g = 0; g < 2; g++) SZ[a][g] = S(a, g) - S(a, 2);
+  for (int f = 0; f < 2; f++)
+    for (int g = 0; g < 2; g++) V[f * 2 + g] = SZ[f][g] - SZ[2][g];
+  const double bR[2] = {S(0, 2) - S(2, 2), S(1, 2) - S(2, 2)};   // Z^T S c
+  const double bL[2] = {S(2, 0) - S(2, 2), S(2, 1) - S(2, 2)};   // Z^T S^T c
+  const double det = V[0] * V[3] - V[1] * V[2];
+  r[0] = (V[3] * bR[0] - V[1] * bR[1]) / det;
+  r[1] = (V[0] * bR[1] - V[2] * bR[0]) / det;
+  l[0] = (V[3] * bL[0] - V[2] * bL[1]) / det;
+  l[1] = (V[0] * bL[1] - V[1] * bL[0]) / det;
+  *kappa = S(2, 2) - (l[0] * (V[0] * r[0] + V[1] * r[1]) + l[1] * (V[2] * r[0] + V[3] * r[1]));
+  double smax = 0;
+  for (int k = 0; k < 9; k++) smax = std::max(smax, fabs(score[k]));
+  const double vals[9] = {l[0], l[1], r[0], r[1], V[0], V[1], V[2], V[3], *kappa};
+  for (double v : vals)
+    if (!std::isfinite(v)) return false;
+  const double shift = std::max(std::max(fabs(l[0]), fabs(l[1])), std::max(fabs(r[0]), fabs(r[1])));
+  return shift <= 4.0 && fabs(*kappa) <= 4.0 * smax;
+}
+
 int ngsd_create(const ngsd_cfg *cfg, ngsd_ctx **out) {
   if (!cfg || !out) { ngsd_set_error(nullptr, "null argument"); return NGSD_ERR_ARG; }
   *out = nullptr;
@@ -303,7 +334,16 @@ int ngsd_create(const ngsd_cfg *cfg, ngsd_ctx **out) {
     CREATE_CUDA(dev_alloc(&ctx->codes, ctx->RB * ctx->NW * 512));
     CREATE_CUDA(dev_alloc(&ctx->codes4, ctx->RB * ctx->NW * 1024));
   }
-  const uint64_t plane = ctx->int_path ? 0 : ctx->RB * ctx->NC * NGSD_TILE_DOUBLES;
+  // --pairwise_del on the FP64 path: two planes with the mask term folded into the shared-site count (ngsd_internal.h),
+  // for contractions of at least NGSD_PDEL2_MIN_PAIR_SITES pair-sites per matrix
+  const double pair_sites = (double) cfg->n_ind * (double) (cfg->n_ind - 1) / 2 * (double) cfg->n_sites;
+  ctx->pdel2 = cfg->indep_geno && cfg->pairwise_del && !ctx->int_path && !(cfg->reserved & 1) && pair_sites >= (double) NGSD_PDEL2_MIN_PAIR_SITES &&
+               pdel2_coefficients(cfg->score, ctx->pd_l, ctx->pd_r, ctx->pd_V, &ctx->pd_kappa);
+  if (ctx->pdel2) {
+    ctx->k4 = NGSD_K4_PD2;
+    ctx->tile_doubles = (uint64_t) NGSD_K4_PD2 * NGSD_K4_DOUBLES;
+  }
+  const uint64_t plane = ctx->int_path ? 0 : ctx->RB * ctx->NC * ctx->tile_doubles;
   CREATE_CUDA(dev_alloc(&ctx->Apack, plane));
   CREATE_CUDA(dev_alloc(&ctx->Bpack, plane));
   CREATE_CUDA(dev_alloc(&ctx->mask, ctx->RB * ctx->NW * 128));
@@ -1468,10 +1508,10 @@ static int distances_enqueue(ngsd_ctx *ctx, const uint32_t *block_counts, uint64
   job->count_timed = cnt_on_tc || run_k3;
   ctx->timing.launches = launches;
   ctx->timing.dist_ctas = plan.grid;
-  // DMMAs executed per K4 step: 256 per full tile, 136 per diagonal tile, 16 per real 8-column block of an edge tile
+  // DMMAs executed per K4 step (ctx->k4 steps per chunk): 256 per full tile, 136 per diagonal tile, 16 per real 8-column block of an edge tile
   const uint64_t dmma_step = (uint64_t) (ctx->n_tiles - ctx->n_diag_tiles - ctx->n_edge_tiles) * 256ull + (uint64_t) ctx->n_diag_tiles * 136ull +
                              (uint64_t) ctx->n_edge_tiles * 16ull * ngsd_edge_c8(ctx->n_ind);
-  ctx->timing.dist_dmma = (em_path || (use_cache && !build_cache)) ? 0 : (uint64_t) plan.n_chunks * NGSD_K4_PER_CHUNK * dmma_step;
+  ctx->timing.dist_dmma = (em_path || (use_cache && !build_cache)) ? 0 : (uint64_t) plan.n_chunks * ctx->k4 * dmma_step;
   ctx->timing.active_sites = active_sites;
   ctx->timing.block_cache = use_cache ? (build_cache ? 1 : 2) : 0;
   if (use_cache) {

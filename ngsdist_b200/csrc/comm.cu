@@ -205,8 +205,8 @@ void site_range_segments(ngsd_ctx *c, uint64_t s0, uint64_t s1, bool last, std::
   const uint64_t c0 = s0 / (uint64_t) c->sc, c1 = last ? c->NC : s1 / (uint64_t) c->sc;
   for (uint64_t rb = 0; rb < c->RB; rb++) {
     if (!c->int_path && c1 > c0) {
-      out.push_back({(char *) (c->Apack + (rb * c->NC + c0) * NGSD_TILE_DOUBLES), (c1 - c0) * NGSD_TILE_BYTES});
-      out.push_back({(char *) (c->Bpack + (rb * c->NC + c0) * NGSD_TILE_DOUBLES), (c1 - c0) * NGSD_TILE_BYTES});
+      out.push_back({(char *) (c->Apack + (rb * c->NC + c0) * c->tile_doubles), (c1 - c0) * c->tile_doubles * sizeof(double)});
+      out.push_back({(char *) (c->Bpack + (rb * c->NC + c0) * c->tile_doubles), (c1 - c0) * c->tile_doubles * sizeof(double)});
     }
     if (rb == 0 && w1 > w0) out.push_back({(char *) (c->d_blank + w0), (w1 - w0) * sizeof(uint64_t)});
     if (w1 > w0) {

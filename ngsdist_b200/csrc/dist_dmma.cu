@@ -5,7 +5,9 @@
 //
 // Structure (one persistent CTA per SM):
 //   warp 8        producer: one elected lane stages (A tile, B tile[, 8 weights]) of one 8-site chunk per pipeline
-//                 step with cp.async.bulk (TMA bulk copy, SASS UBLKCP) completing on an mbarrier; 4 stages x 48 KiB.
+//                 step with cp.async.bulk (TMA bulk copy, SASS UBLKCP) completing on an mbarrier; 4 stages x 48 KiB
+//                 (three planes, K4 = 6 k4-groups per chunk) or 4 stages x 32 KiB (pdel two-plane mode, K4 = 4; a
+//                 6-stage ring measured the same at C3 on a B200).
 //   warps 0..7    consumers, 2 (M) x 4 (N): each owns a 64 x 32 sub-tile = 8 x 4 DMMA accumulators (128 registers);
 //                 fragments come straight from the packed layout with conflict-free 256-byte LDS.64.
 //                 Diagonal tiles (upper triangle only) and edge tiles (real columns only) have their own warp layouts.
@@ -19,11 +21,18 @@
 
 namespace {
 
-constexpr int kStages = 4;
 constexpr int kConsumerWarps = 8;
 constexpr int kThreads = (kConsumerWarps + 1) * 32;
-constexpr int kStageBytes = 2 * NGSD_TILE_BYTES + 128;  // A + B + up to 12 per-site weights
-constexpr size_t kSmemBytes = (size_t) kStages * kStageBytes + 2 * kStages * sizeof(uint64_t) + kStages * 2 * sizeof(uint32_t) + 128;
+
+// Pipeline geometry for K4 k4-groups per chunk (6: three planes or the 12-site two-plane layout; 4: pdel two-plane mode)
+template <int K4>
+struct Ring {
+  static constexpr int kTileDoubles = K4 * NGSD_K4_DOUBLES;
+  static constexpr int kTileBytes = kTileDoubles * 8;
+  static constexpr int kStages = 4;
+  static constexpr int kStageBytes = 2 * kTileBytes + 128;   // A + B + up to 12 per-site weights
+  static constexpr size_t kSmemBytes = (size_t) kStages * kStageBytes + 2 * kStages * sizeof(uint64_t) + kStages * 2 * sizeof(uint32_t) + 128;
+};
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t) __cvta_generic_to_shared(p); }
 
@@ -97,10 +106,10 @@ __device__ __forceinline__ void step_full(double (&acc)[64], const double *As, c
 // balanced): acc[0..31] = row W, columns 0..15; acc[32..63] = row 15-W.  Specialised per warp at compile time:
 // predicated-off DMMAs still cost issue slots on the FP64 tensor pipe, so each warp runs straight-line code with
 // exactly its 17 DMMA + (18 - W) LDS.64 per K4 step.
-template <int W, int PLANES>
+template <int W, int PLANES, int K4>
 __device__ __forceinline__ void chunk_diag(double (&acc)[64], const double *As, const double *Bs, const double (&wv)[3]) {
 #pragma unroll
-  for (int k4 = 0; k4 < NGSD_K4_PER_CHUNK; k4++) {
+  for (int k4 = 0; k4 < K4; k4++) {
     const double *Ak = As + k4 * 512, *Bk = Bs + k4 * 512;
     const double w = wv[PLANES == 3 ? (k4 & 1) : (k4 % 3)];
     const double a0 = Ak[W * 32], a1 = Ak[(15 - W) * 32];
@@ -127,10 +136,10 @@ __device__ __forceinline__ void store_diag(const double (&acc)[64], double2 *dst
 // LDS.64 per K4 step on every warp (the full-tile layout would leave the padding columns on SMSPs 2 and 3 and keep them
 // the busiest).  acc[0 .. 2*C8) = row W, acc[2*C8 .. 4*C8) = row W + 8.  Each 8x8 block takes the same fragments, the
 // same weight product and the same DMMA sequence as in step_full, so its sums are bit-identical.
-template <int C8, int PLANES>
+template <int C8, int PLANES, int K4>
 __device__ __forceinline__ void chunk_edge(double (&acc)[64], const double *As, const double *Bs, const double (&wv)[3]) {
 #pragma unroll
-  for (int k4 = 0; k4 < NGSD_K4_PER_CHUNK; k4++) {
+  for (int k4 = 0; k4 < K4; k4++) {
     const double *Ak = As + k4 * 512, *Bk = Bs + k4 * 512;
     const double w = wv[PLANES == 3 ? (k4 & 1) : (k4 % 3)];
     const double a0 = Ak[0], a1 = Ak[8 * 32];
@@ -156,16 +165,19 @@ __device__ __forceinline__ void store_edge(const double (&acc)[64], double2 *til
 }
 
 // PLANES = 3: chunk of 8 sites, k4-group = g*2 + h;  PLANES = 2: chunk of 12 sites, k4-group = g*3 + h (ngsd_internal.h).
-// The only place the two differ inside the kernel is which per-site weight a k4-group takes.
-template <bool WEIGHTED, int PLANES>
+// The only place the two differ inside the kernel is which per-site weight a k4-group takes.  K4 = k4-groups per chunk:
+// 6, or 4 in pdel two-plane mode (8-site chunks, PLANES = 3 weight indexing, g = 0..1).
+template <bool WEIGHTED, int PLANES, int K4>
 __global__ void __launch_bounds__(kThreads, 1) k_dist_dmma(DistArgs a) {
+  constexpr int kStages = Ring<K4>::kStages, kStageBytes = Ring<K4>::kStageBytes, kTileBytes = Ring<K4>::kTileBytes;
+  constexpr int kTileDoubles = Ring<K4>::kTileDoubles;
   extern __shared__ __align__(128) unsigned char smem[];
   uint64_t *full = reinterpret_cast<uint64_t *>(smem + (size_t) kStages * kStageBytes);
   uint64_t *empty = full + kStages;
   uint32_t *meta = reinterpret_cast<uint32_t *>(empty + kStages);   // [kStages][2] = {unit, flags}
   auto stageA = [&](int s) { return reinterpret_cast<double *>(smem + (size_t) s * kStageBytes); };
-  auto stageB = [&](int s) { return reinterpret_cast<double *>(smem + (size_t) s * kStageBytes + NGSD_TILE_BYTES); };
-  auto stageW = [&](int s) { return reinterpret_cast<double *>(smem + (size_t) s * kStageBytes + 2 * NGSD_TILE_BYTES); };
+  auto stageB = [&](int s) { return reinterpret_cast<double *>(smem + (size_t) s * kStageBytes + kTileBytes); };
+  auto stageW = [&](int s) { return reinterpret_cast<double *>(smem + (size_t) s * kStageBytes + 2 * kTileBytes); };
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (threadIdx.x == 0) {
@@ -186,8 +198,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_dmma(DistArgs a) {
         const uint32_t q = u / a.n_tiles, t = u - q * a.n_tiles;
         const ngsd_tile tl = a.tiles[t];
         const uint32_t c0 = a.split_begin[q], c1 = a.split_begin[q + 1];
-        const double *Ab = a.Apack + (uint64_t) tl.ti * a.NC * NGSD_TILE_DOUBLES;
-        const double *Bb = a.Bpack + (uint64_t) tl.tj * a.NC * NGSD_TILE_DOUBLES;
+        const double *Ab = a.Apack + (uint64_t) tl.ti * a.NC * kTileDoubles;
+        const double *Bb = a.Bpack + (uint64_t) tl.tj * a.NC * kTileDoubles;
         const uint32_t fl = tl.ti == tl.tj ? kDiag : (tl.tj == a.edge_tj ? kEdge : 0u);
         for (uint32_t c = c0; c < c1; c++) {
           const uint64_t chunk = a.chunk_ids ? a.chunk_ids[c] : c;
@@ -195,9 +207,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_dmma(DistArgs a) {
           meta[stage * 2] = u;
           meta[stage * 2 + 1] = fl | (c == c0 ? kFirst : 0u) | (c + 1 == c1 ? kLast : 0u);
           constexpr int kSites = PLANES == 3 ? NGSD_SC : NGSD_SC2;
-          mbar_expect_tx(&full[stage], 2 * NGSD_TILE_BYTES + (WEIGHTED ? kSites * 8 : 0));
-          bulk_g2s(stageA(stage), Ab + chunk * NGSD_TILE_DOUBLES, NGSD_TILE_BYTES, &full[stage]);
-          bulk_g2s(stageB(stage), Bb + chunk * NGSD_TILE_DOUBLES, NGSD_TILE_BYTES, &full[stage]);
+          mbar_expect_tx(&full[stage], 2 * kTileBytes + (WEIGHTED ? kSites * 8 : 0));
+          bulk_g2s(stageA(stage), Ab + chunk * kTileDoubles, kTileBytes, &full[stage]);
+          bulk_g2s(stageB(stage), Bb + chunk * kTileDoubles, kTileBytes, &full[stage]);
           if (WEIGHTED) bulk_g2s(stageW(stage), a.weights + chunk * kSites, kSites * 8, &full[stage]);
           if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
@@ -232,28 +244,28 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_dmma(DistArgs a) {
     if (fl & kDiag) {
       const double *As = stageA(stage) + lane, *Bs = stageB(stage) + lane;
       switch (warp) {       // warp-uniform: no divergence
-        case 0: chunk_diag<0, PLANES>(acc, As, Bs, wv); break;
-        case 1: chunk_diag<1, PLANES>(acc, As, Bs, wv); break;
-        case 2: chunk_diag<2, PLANES>(acc, As, Bs, wv); break;
-        case 3: chunk_diag<3, PLANES>(acc, As, Bs, wv); break;
-        case 4: chunk_diag<4, PLANES>(acc, As, Bs, wv); break;
-        case 5: chunk_diag<5, PLANES>(acc, As, Bs, wv); break;
-        case 6: chunk_diag<6, PLANES>(acc, As, Bs, wv); break;
-        default: chunk_diag<7, PLANES>(acc, As, Bs, wv); break;
+        case 0: chunk_diag<0, PLANES, K4>(acc, As, Bs, wv); break;
+        case 1: chunk_diag<1, PLANES, K4>(acc, As, Bs, wv); break;
+        case 2: chunk_diag<2, PLANES, K4>(acc, As, Bs, wv); break;
+        case 3: chunk_diag<3, PLANES, K4>(acc, As, Bs, wv); break;
+        case 4: chunk_diag<4, PLANES, K4>(acc, As, Bs, wv); break;
+        case 5: chunk_diag<5, PLANES, K4>(acc, As, Bs, wv); break;
+        case 6: chunk_diag<6, PLANES, K4>(acc, As, Bs, wv); break;
+        default: chunk_diag<7, PLANES, K4>(acc, As, Bs, wv); break;
       }
     } else if (fl & kEdge) {
       const double *As = stageA(stage) + warp * 32 + lane, *Bs = stageB(stage) + lane;
       switch (a.edge_c8) {  // kernel-uniform
-#define NGSD_EDGE_CASE(C) case C: chunk_edge<C, PLANES>(acc, As, Bs, wv); break;
+#define NGSD_EDGE_CASE(C) case C: chunk_edge<C, PLANES, K4>(acc, As, Bs, wv); break;
         NGSD_EDGE_CASE(1) NGSD_EDGE_CASE(2) NGSD_EDGE_CASE(3) NGSD_EDGE_CASE(4) NGSD_EDGE_CASE(5)
         NGSD_EDGE_CASE(6) NGSD_EDGE_CASE(7) NGSD_EDGE_CASE(8) NGSD_EDGE_CASE(9) NGSD_EDGE_CASE(10)
-        NGSD_EDGE_CASE(11) NGSD_EDGE_CASE(12) NGSD_EDGE_CASE(13) NGSD_EDGE_CASE(14) default: chunk_edge<15, PLANES>(acc, As, Bs, wv); break;
+        NGSD_EDGE_CASE(11) NGSD_EDGE_CASE(12) NGSD_EDGE_CASE(13) NGSD_EDGE_CASE(14) default: chunk_edge<15, PLANES, K4>(acc, As, Bs, wv); break;
 #undef NGSD_EDGE_CASE
       }
     } else {
       const double *As = stageA(stage) + (wm * 8) * 32 + lane, *Bs = stageB(stage) + (wn * 4) * 32 + lane;
 #pragma unroll
-      for (int k4 = 0; k4 < NGSD_K4_PER_CHUNK; k4++) step_full(acc, As + k4 * 512, Bs + k4 * 512, wv[PLANES == 3 ? (k4 & 1) : (k4 % 3)]);
+      for (int k4 = 0; k4 < K4; k4++) step_full(acc, As + k4 * 512, Bs + k4 * 512, wv[PLANES == 3 ? (k4 & 1) : (k4 % 3)]);
     }
     __syncwarp();
     if (lane == 0) mbar_arrive(&empty[stage]);
@@ -314,14 +326,19 @@ __global__ void k_dmma_peak(double *out, int iters) {
 
 }  // namespace
 
-size_t ngsd_dist_smem_bytes() { return kSmemBytes; }
+size_t ngsd_dist_smem_bytes() { return std::max(Ring<NGSD_K4_3>::kSmemBytes, Ring<NGSD_K4_PD2>::kSmemBytes); }
 
 cudaError_t ngsd_launch_dist_dmma(ngsd_ctx *ctx, const ngsd_dist_plan &p) {
   static bool attr_set[64] = {};
   if (!attr_set[ctx->device & 63]) {
-    const void *fns[3] = {(const void *) k_dist_dmma<false, 3>, (const void *) k_dist_dmma<true, 3>, (const void *) k_dist_dmma<true, 2>};
-    for (const void *f : fns) {
-      cudaError_t e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) kSmemBytes);
+    const void *fns[5] = {(const void *) k_dist_dmma<false, 3, NGSD_K4_3>, (const void *) k_dist_dmma<true, 3, NGSD_K4_3>,
+                          (const void *) k_dist_dmma<true, 2, NGSD_K4_3>, (const void *) k_dist_dmma<false, 3, NGSD_K4_PD2>,
+                          (const void *) k_dist_dmma<true, 3, NGSD_K4_PD2>};
+    const size_t smem[5] = {Ring<NGSD_K4_3>::kSmemBytes, Ring<NGSD_K4_3>::kSmemBytes, Ring<NGSD_K4_3>::kSmemBytes,
+                            Ring<NGSD_K4_PD2>::kSmemBytes, Ring<NGSD_K4_PD2>::kSmemBytes};
+    for (int k = 0; k < 5; k++) {
+      const void *f = fns[k];
+      cudaError_t e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem[k]);
       if (e != cudaSuccess) return e;
       e = cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
       if (e != cudaSuccess) return e;
@@ -346,13 +363,20 @@ cudaError_t ngsd_launch_dist_dmma(ngsd_ctx *ctx, const ngsd_dist_plan &p) {
   a.edge_c8 = c8;
   cudaError_t e = cudaMemsetAsync(ctx->d_sched, 0, sizeof(uint32_t), ctx->stream);
   if (e != cudaSuccess) return e;
-  if (p.weighted && !p.uniform_scale) {
-    if (ctx->planes == 3)
-      k_dist_dmma<true, 3><<<p.grid, kThreads, kSmemBytes, ctx->stream>>>(a);
+  constexpr size_t smem3 = Ring<NGSD_K4_3>::kSmemBytes, smem2 = Ring<NGSD_K4_PD2>::kSmemBytes;
+  const bool per_site = p.weighted && !p.uniform_scale;
+  if (ctx->pdel2) {
+    if (per_site)
+      k_dist_dmma<true, 3, NGSD_K4_PD2><<<p.grid, kThreads, smem2, ctx->stream>>>(a);
     else
-      k_dist_dmma<true, 2><<<p.grid, kThreads, kSmemBytes, ctx->stream>>>(a);
+      k_dist_dmma<false, 3, NGSD_K4_PD2><<<p.grid, kThreads, smem2, ctx->stream>>>(a);
+  } else if (per_site) {
+    if (ctx->planes == 3)
+      k_dist_dmma<true, 3, NGSD_K4_3><<<p.grid, kThreads, smem3, ctx->stream>>>(a);
+    else
+      k_dist_dmma<true, 2, NGSD_K4_3><<<p.grid, kThreads, smem3, ctx->stream>>>(a);
   } else {
-    k_dist_dmma<false, 3><<<p.grid, kThreads, kSmemBytes, ctx->stream>>>(a);   // unweighted: plane count is irrelevant
+    k_dist_dmma<false, 3, NGSD_K4_3><<<p.grid, kThreads, smem3, ctx->stream>>>(a);   // unweighted: plane count is irrelevant
   }
   return cudaGetLastError();
 }

@@ -284,7 +284,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_dist_em3(EmArgs a) {
     for (int h = 0; h < 6; h++) {
       const int seg = h * 2 + (tid >> 8);
       const uint64_t gi0 = (uint64_t) (seg < 6 ? ti : tj) * kEdge;
-      const double *src = a.Apack + ((gi0 >> 7) * a.NC + chunk) * NGSD_TILE_DOUBLES + (seg % 6) * 512 + ((gi0 & 127) >> 3) * 32;
+      const double *src = a.Apack + ((gi0 >> 7) * a.NC + chunk) * (NGSD_K4_3 * NGSD_K4_DOUBLES) + (seg % 6) * 512 + ((gi0 & 127) >> 3) * 32;
       raw[seg * 256 + (tid & 255)] = src[tid & 255];
     }
     if (WEIGHTED && tid < NGSD_SC) wgt[tid] = a.weights[chunk * NGSD_SC + tid];

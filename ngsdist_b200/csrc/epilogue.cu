@@ -14,6 +14,7 @@ struct EpiArgs {
   const uint32_t *cnt_cache;  // per-block counts [n_splits][n_tiles][4][64][64] (bootstrap block cache) or nullptr
   const double *cvec;         // [n_pad] 2-plane mode: weighted row sums of the B_2 plane, added for column j; or nullptr
   const double *fix;          // [n_ind][n_ind] 2-plane mode: correction for row triples that do not sum to one; or nullptr
+  double kappa;               // pdel two-plane mode: num += kappa * cnt (the mask term of ngsd_internal.h); else 0
   double *out, *num;          // [n_ind][n_ind]
   uint64_t *cntout;
   uint64_t n_ind, n_pad, const_cnt, tot_sites;
@@ -84,6 +85,7 @@ __global__ void __launch_bounds__(256) k_epilogue(EpiArgs a) {
         if (w != 0.0) cnt += (uint64_t) w * (uint64_t) pc[(uint64_t) q2 * cstride];
       }
     }
+    if (a.kappa != 0.0) num += a.kappa * (double) cnt;   // the weighted shared-site count, before the tot_sites override
     if (a.num) a.num[i * a.n_ind + j] = a.num[j * a.n_ind + i] = num;
     if (a.cntout) a.cntout[i * a.n_ind + j] = a.cntout[j * a.n_ind + i] = cnt;
     if (a.tot_sites > 0) cnt = a.tot_sites;
@@ -279,6 +281,7 @@ cudaError_t ngsd_launch_epilogue(ngsd_ctx *ctx, const ngsd_epilogue_args &e) {
   a.cnt_cache = e.use_cnt ? ctx->cur_cnt_cache : nullptr;
   a.cvec = ctx->planes == 2 ? ctx->d_cvec : nullptr;
   a.fix = (ctx->planes == 2 && ctx->def_rows) ? ctx->d_fix : nullptr;
+  a.kappa = ctx->pdel2 ? ctx->pd_kappa : 0.0;         // pdel2 implies --pairwise_del: cnt is the real count
   a.out = ctx->d_out;
   a.num = ctx->d_num;
   a.cntout = ctx->d_cntout;

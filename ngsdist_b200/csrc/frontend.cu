@@ -7,8 +7,9 @@
 //   shared/gen_func.cpp:862-868                         miss_data predicate (EPSILON = 1e-5)
 // and writes what gen_dist (ngsDist.cpp:325-404) will contract: A = p, B = score.p in DMMA fragment order.
 //
-// HBM-bound by design: 24 B read + 48 B written per individual-site; one thread owns 4 consecutive sites of one
-// individual so that every global store is a full 32-byte sector and a warp stores 1 KiB contiguous per plane.
+// HBM-bound by design: 24 B read + 48 B written per individual-site (32 B in pdel two-plane mode); one thread owns 4
+// consecutive sites of one individual so that every global store is a full 32-byte sector and a warp stores 1 KiB
+// contiguous per plane.
 #include <algorithm>
 
 #include "ngsd_internal.h"
@@ -18,6 +19,8 @@ namespace {
 constexpr double kNegInfClamp = -1e15;               // "INF" of shared/gen_func.hpp:15
 constexpr double kEps = 1e-5;                        // EPSILON, shared/gen_func.hpp:16
 constexpr double kThird = 0x1.5555555555555p-2;      // exp(log(1/3)) as glibc evaluates it (SURVEY §8a H3)
+constexpr uint64_t kTile3 = NGSD_K4_3 * NGSD_K4_DOUBLES;     // doubles per operand tile: three planes / planes == 2
+constexpr uint64_t kTilePd2 = NGSD_K4_PD2 * NGSD_K4_DOUBLES; // pdel two-plane mode
 
 // One 32-byte sector per instruction (sm_100 has 256-bit global stores: STG.E.ENL2.256); p must be 32-byte aligned.
 __device__ __forceinline__ void st256(double *p, double a, double b, double c, double d) {
@@ -30,6 +33,8 @@ struct FrontCfg {
   int call_geno;
   int pairwise_del;
   int planes;        // 3, or 2 (sum-to-one reduction, see ngsd_internal.h)
+  int pdel2;         // pdel two-plane mode (planes == 3 chunks, 2 planes; ngsd_internal.h)
+  double pl[2], pr[2], pV[4];   // its shifts l, r and V (row-major)
   int int_path;      // called genotypes: write 2-bit codes for dist_umma.cu instead of FP64 planes
   double N_thresh, call_thresh;
   double score[9];
@@ -249,6 +254,19 @@ __device__ __forceinline__ bool miss_data(const double p[3]) {      // gen_func.
   return fabs(p[0] - p[1]) < kEps && fabs(p[1] - p[2]) < kEps;
 }
 
+// Pdel two-plane operands of one individual-site: A = m (p0 + l0, p1 + l1), B = m V (p0 + r0, p1 + r1).  A present
+// triple with a non-finite component poisons both coordinates (the form drops p2, and with it a NaN in p2 alone): its
+// row and column turn NaN, as in the three-plane contraction.
+__device__ __forceinline__ void pdel2_operands(const FrontCfg &c, const double p[3], bool present, double a[2], double b[2]) {
+  if (!present) { a[0] = a[1] = b[0] = b[1] = 0.0; return; }
+  double q0 = p[0] + c.pl[0], q1 = p[1] + c.pl[1], t0 = p[0] + c.pr[0], t1 = p[1] + c.pr[1];
+  if (!(isfinite(p[0]) && isfinite(p[1]) && isfinite(p[2]))) q0 = q1 = t0 = t1 = NAN;
+  a[0] = q0;
+  a[1] = q1;
+  b[0] = c.pV[0] * t0 + c.pV[1] * t1;
+  b[1] = c.pV[2] * t0 + c.pV[3] * t1;
+}
+
 // grid (n_pad/32, ceil(n/64)); block (32 individuals, 16 site groups of 4) = one 64-site mask word per individual.
 // EXACT = the reference's log-space sequence (needed by call_geno's comparisons); otherwise the fast path above.
 template <bool EXACT>
@@ -315,36 +333,52 @@ __global__ void __launch_bounds__(512, EXACT ? 1 : 2) k_frontend(FrontCfg c, con
   // packed stores: 32 bytes per plane per operand; B = score . p evaluated in the reference's g2 order (ngsDist.cpp:351-353)
   const uint64_t rb = i >> 7, r = i & 127;
   const uint64_t sgrp = site0 / 4 + (uint64_t) blockIdx.y * 16 + ty;     // global 4-site group
-  double Bv[3][4];
-#pragma unroll
-  for (int g = 0; g < 3; g++)
-#pragma unroll
-    for (int q = 0; q < 4; q++) {
-      double b = c.score[3 * g + 0] * A[q][0];
-      b += c.score[3 * g + 1] * A[q][1];
-      b += c.score[3 * g + 2] * A[q][2];
-      Bv[g][q] = b;
-    }
-  if (c.planes == 3) {
+  if (c.pdel2) {
+    // pdel two-plane: chunk of 8 sites, k4-group = g*2 + h, g = 0..1 (no C plane, no deficit list: a triple that does not
+    // sum to one -- all-zero, blank -- is missing under --pairwise_del)
     const uint64_t chunk = sgrp >> 1, h = sgrp & 1;
-    const uint64_t base = (rb * NC + chunk) * NGSD_TILE_DOUBLES + (r >> 3) * 32 + (r & 7) * 4;
+    const uint64_t base = (rb * NC + chunk) * kTilePd2 + (r >> 3) * 32 + (r & 7) * 4;
+    double Av[4][2], Bw[4][2];
 #pragma unroll
-    for (int g = 0; g < 3; g++) {
-      const uint64_t o = base + (uint64_t) (g * 2 + h) * (16 * 32);
-      st256(Apack + o, A[0][g], A[1][g], A[2][g], A[3][g]);
-      st256(Bpack + o, Bv[g][0], Bv[g][1], Bv[g][2], Bv[g][3]);
-    }
-  } else {
-    // two planes: A = (p0, p1), B = (B0 - B2, B1 - B2), C = B2; chunk of 12 sites, k4-group = g*3 + h
-    const uint64_t chunk = sgrp / 3, h = sgrp % 3;
-    const uint64_t base = (rb * NC + chunk) * NGSD_TILE_DOUBLES + (r >> 3) * 32 + (r & 7) * 4;
+    for (int q = 0; q < 4; q++) pdel2_operands(c, A[q], (bits >> q) & 1u, Av[q], Bw[q]);
 #pragma unroll
     for (int g = 0; g < 2; g++) {
-      const uint64_t o = base + (uint64_t) (g * 3 + h) * (16 * 32);
-      st256(Apack + o, A[0][g], A[1][g], A[2][g], A[3][g]);
-      st256(Bpack + o, Bv[g][0] - Bv[2][0], Bv[g][1] - Bv[2][1], Bv[g][2] - Bv[2][2], Bv[g][3] - Bv[2][3]);
+      const uint64_t o = base + (uint64_t) (g * 2 + h) * NGSD_K4_DOUBLES;
+      st256(Apack + o, Av[0][g], Av[1][g], Av[2][g], Av[3][g]);
+      st256(Bpack + o, Bw[0][g], Bw[1][g], Bw[2][g], Bw[3][g]);
     }
-    st256(Cplane + (word * ldc + i) * 64 + ty * 4, Bv[2][0], Bv[2][1], Bv[2][2], Bv[2][3]);   // [word][n_pad][64]: a site range is contiguous (all-gather)
+  } else {
+    double Bv[3][4];
+#pragma unroll
+    for (int g = 0; g < 3; g++)
+#pragma unroll
+      for (int q = 0; q < 4; q++) {
+        double b = c.score[3 * g + 0] * A[q][0];
+        b += c.score[3 * g + 1] * A[q][1];
+        b += c.score[3 * g + 2] * A[q][2];
+        Bv[g][q] = b;
+      }
+    if (c.planes == 3) {
+      const uint64_t chunk = sgrp >> 1, h = sgrp & 1;
+      const uint64_t base = (rb * NC + chunk) * kTile3 + (r >> 3) * 32 + (r & 7) * 4;
+#pragma unroll
+      for (int g = 0; g < 3; g++) {
+        const uint64_t o = base + (uint64_t) (g * 2 + h) * (16 * 32);
+        st256(Apack + o, A[0][g], A[1][g], A[2][g], A[3][g]);
+        st256(Bpack + o, Bv[g][0], Bv[g][1], Bv[g][2], Bv[g][3]);
+      }
+    } else {
+      // two planes: A = (p0, p1), B = (B0 - B2, B1 - B2), C = B2; chunk of 12 sites, k4-group = g*3 + h
+      const uint64_t chunk = sgrp / 3, h = sgrp % 3;
+      const uint64_t base = (rb * NC + chunk) * kTile3 + (r >> 3) * 32 + (r & 7) * 4;
+#pragma unroll
+      for (int g = 0; g < 2; g++) {
+        const uint64_t o = base + (uint64_t) (g * 3 + h) * (16 * 32);
+        st256(Apack + o, A[0][g], A[1][g], A[2][g], A[3][g]);
+        st256(Bpack + o, Bv[g][0] - Bv[2][0], Bv[g][1] - Bv[2][1], Bv[g][2] - Bv[2][2], Bv[g][3] - Bv[2][3]);
+      }
+      st256(Cplane + (word * ldc + i) * 64 + ty * 4, Bv[2][0], Bv[2][1], Bv[2][2], Bv[2][3]);   // [word][n_pad][64]: a site range is contiguous (all-gather)
+    }
   }
 
   nib[ty][tx] = bits;
@@ -363,7 +397,7 @@ __global__ void __launch_bounds__(512, EXACT ? 1 : 2) k_frontend(FrontCfg c, con
 // memory in every thread of the caller.)  Returns the code, + 4 when a NaN was found on the binary path.
 __device__ __noinline__ unsigned called_code_exact(int kind, int in_log, double N_thresh, double call_thresh, double x0, double x1, double x2) {
   FrontCfg c;
-  c.kind = kind; c.in_log = in_log; c.call_geno = 1; c.pairwise_del = 0; c.planes = 3; c.int_path = 1;
+  c.kind = kind; c.in_log = in_log; c.call_geno = 1; c.pairwise_del = 0; c.planes = 3; c.pdel2 = 0; c.int_path = 1;
   c.N_thresh = N_thresh; c.call_thresh = call_thresh;
   double p[3];
   bool knife;
@@ -540,28 +574,34 @@ __global__ void __launch_bounds__(512, 4) k_codes_from_int8(const int8_t *__rest
 
 // Inspection: packed A planes + mask -> [ind][site][3] / [ind][site]
 __global__ void k_unpack(const double *__restrict__ Apack, const uint32_t *__restrict__ codes, const uint64_t *__restrict__ mask,
-                         uint64_t n_ind, uint64_t n_sites, uint64_t NC, uint64_t NW, int planes, double *__restrict__ P,
-                         uint8_t *__restrict__ miss) {
+                         uint64_t n_ind, uint64_t n_sites, uint64_t NC, uint64_t NW, int planes, int pdel2, double l0, double l1,
+                         double *__restrict__ P, uint8_t *__restrict__ miss) {
   const uint64_t idx = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= n_ind * n_sites) return;
   const uint64_t i = idx / n_sites, s = idx % n_sites;
   const uint64_t rb = i >> 7, r = i & 127, sgrp = s >> 2, q = s & 3;
+  const bool present = (mask[(rb * NW + (s >> 6)) * 128 + r] >> (s & 63)) & 1;
   if (P) {
     if (codes) {
       const unsigned code = (codes[((rb * NW + (s >> 6)) * 4 + ((s >> 4) & 3)) * 128 + r] >> (2 * (s & 15))) & 3u;
       for (unsigned g = 0; g < 3; g++) P[idx * 3 + g] = code == 3u ? kThird : (code == g ? 1.0 : 0.0);
+    } else if (pdel2) {     // A = m (p0 + l0, p1 + l1): missing individual-sites read as zero, as in the three planes
+      const uint64_t chunk = sgrp >> 1, h = sgrp & 1;
+      const uint64_t base = (rb * NC + chunk) * kTilePd2 + (r >> 3) * 32 + (r & 7) * 4 + q;
+      const double p0 = present ? Apack[base + h * 512] - l0 : 0.0, p1 = present ? Apack[base + (2 + h) * 512] - l1 : 0.0;
+      P[idx * 3 + 0] = p0; P[idx * 3 + 1] = p1; P[idx * 3 + 2] = present ? 1.0 - p0 - p1 : 0.0;
     } else if (planes == 3) {
       const uint64_t chunk = sgrp >> 1, h = sgrp & 1;
-      const uint64_t base = (rb * NC + chunk) * NGSD_TILE_DOUBLES + (r >> 3) * 32 + (r & 7) * 4 + q;
+      const uint64_t base = (rb * NC + chunk) * kTile3 + (r >> 3) * 32 + (r & 7) * 4 + q;
       for (int g = 0; g < 3; g++) P[idx * 3 + g] = Apack[base + (uint64_t) (g * 2 + h) * 512];
     } else {
       const uint64_t chunk = sgrp / 3, h = sgrp % 3;
-      const uint64_t base = (rb * NC + chunk) * NGSD_TILE_DOUBLES + (r >> 3) * 32 + (r & 7) * 4 + q;
+      const uint64_t base = (rb * NC + chunk) * kTile3 + (r >> 3) * 32 + (r & 7) * 4 + q;
       const double p0 = Apack[base + (uint64_t) (0 * 3 + h) * 512], p1 = Apack[base + (uint64_t) (1 * 3 + h) * 512];
       P[idx * 3 + 0] = p0; P[idx * 3 + 1] = p1; P[idx * 3 + 2] = 1.0 - p0 - p1;   // the identity the 2-plane mode relies on
     }
   }
-  if (miss) miss[idx] = !((mask[(rb * NW + (s >> 6)) * 128 + r] >> (s & 63)) & 1);
+  if (miss) miss[idx] = !present;
 }
 
 // ngsd_push_packed_genotypes: 2-bit fields, four individuals per byte -> the int8 codes of read_data.cpp:88-95 that
@@ -603,6 +643,12 @@ __global__ void k_synth(double *__restrict__ raw, uint64_t seed, uint64_t thr, i
 
 }  // namespace
 
+static void set_pdel2(FrontCfg &c, const ngsd_ctx *ctx) {
+  c.pdel2 = ctx->pdel2 ? 1 : 0;
+  for (int k = 0; k < 2; k++) { c.pl[k] = ctx->pd_l[k]; c.pr[k] = ctx->pd_r[k]; }
+  for (int k = 0; k < 4; k++) c.pV[k] = ctx->pd_V[k];
+}
+
 cudaError_t ngsd_launch_frontend(ngsd_ctx *ctx, const ngsd_frontend_args &a) {
   FrontCfg c;
   c.kind = ctx->cfg.input_kind;
@@ -610,6 +656,7 @@ cudaError_t ngsd_launch_frontend(ngsd_ctx *ctx, const ngsd_frontend_args &a) {
   c.call_geno = ctx->cfg.call_geno;
   c.pairwise_del = ctx->cfg.pairwise_del;
   c.planes = ctx->planes;
+  set_pdel2(c, ctx);
   c.int_path = ctx->int_path ? 1 : 0;
   c.N_thresh = ctx->cfg.N_thresh;
   c.call_thresh = ctx->cfg.call_thresh;
@@ -669,6 +716,18 @@ __global__ void k_patch(FrontCfg c, const ngsd_deferred *__restrict__ list, unsi
   }
   double p[3] = {d.x[0], d.x[1], d.x[2]};
   if (c.pairwise_del && !present) p[0] = p[1] = p[2] = 0;
+  const uint64_t sgrp = s >> 2, q = s & 3;
+  if (c.pdel2) {
+    double a[2], b[2];
+    pdel2_operands(c, p, present, a, b);
+    const uint64_t base = (rb * NC + (sgrp >> 1)) * kTilePd2 + (r >> 3) * 32 + (r & 7) * 4 + q;
+    for (int g = 0; g < 2; g++) {
+      const uint64_t o = base + (uint64_t) (g * 2 + (sgrp & 1)) * 512;
+      Apack[o] = a[g];
+      Bpack[o] = b[g];
+    }
+    return;
+  }
   double B[3];
 #pragma unroll
   for (int g = 0; g < 3; g++) {
@@ -677,16 +736,15 @@ __global__ void k_patch(FrontCfg c, const ngsd_deferred *__restrict__ list, unsi
     b += c.score[3 * g + 2] * p[2];
     B[g] = b;
   }
-  const uint64_t sgrp = s >> 2, q = s & 3;
   if (c.planes == 3) {
-    const uint64_t base = (rb * NC + (sgrp >> 1)) * NGSD_TILE_DOUBLES + (r >> 3) * 32 + (r & 7) * 4 + q;
+    const uint64_t base = (rb * NC + (sgrp >> 1)) * kTile3 + (r >> 3) * 32 + (r & 7) * 4 + q;
     for (int g = 0; g < 3; g++) {
       const uint64_t o = base + (uint64_t) (g * 2 + (sgrp & 1)) * 512;
       Apack[o] = p[g];
       Bpack[o] = B[g];
     }
   } else {
-    const uint64_t base = (rb * NC + sgrp / 3) * NGSD_TILE_DOUBLES + (r >> 3) * 32 + (r & 7) * 4 + q;
+    const uint64_t base = (rb * NC + sgrp / 3) * kTile3 + (r >> 3) * 32 + (r & 7) * 4 + q;
     for (int g = 0; g < 2; g++) {
       const uint64_t o = base + (uint64_t) (g * 3 + sgrp % 3) * 512;
       Apack[o] = p[g];
@@ -704,6 +762,7 @@ cudaError_t ngsd_launch_patch(ngsd_ctx *ctx, const ngsd_deferred *list_dev, unsi
   memset(&c, 0, sizeof(c));
   c.pairwise_del = ctx->cfg.pairwise_del;
   c.planes = ctx->planes;
+  set_pdel2(c, ctx);
   c.int_path = ctx->int_path ? 1 : 0;
   for (int k = 0; k < 9; k++) c.score[k] = ctx->cfg.score[k];
   k_patch<<<(n + 127) / 128, 128, 0, ctx->stream>>>(c, list_dev, n, ctx->n_pad, ctx->NC, ctx->NW, ctx->Apack, ctx->Bpack, ctx->Cplane, ctx->codes,
@@ -747,7 +806,8 @@ cudaError_t ngsd_launch_unpack_2bit(ngsd_ctx *ctx, const uint8_t *packed_dev, ui
 cudaError_t ngsd_launch_unpack(ngsd_ctx *ctx, double *P_dev, uint8_t *miss_dev) {
   const uint64_t tot = ctx->n_ind * ctx->n_sites;
   k_unpack<<<(unsigned) ((tot + 255) / 256), 256, 0, ctx->stream>>>(ctx->Apack, ctx->codes, ctx->mask, ctx->n_ind, ctx->n_sites, ctx->NC,
-                                                                    ctx->NW, ctx->planes, P_dev, miss_dev);
+                                                                    ctx->NW, ctx->planes, ctx->pdel2 ? 1 : 0, ctx->pd_l[0], ctx->pd_l[1],
+                                                                    P_dev, miss_dev);
   return cudaGetLastError();
 }
 

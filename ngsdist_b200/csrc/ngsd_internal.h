@@ -19,7 +19,8 @@
 //
 //   row block  : 128 individuals           (n_pad = ceil(n_ind/128)*128, RB = n_pad/128)
 //   site chunk : 8 sites                   (NC = ceil(n_sites/8))
-//   one (row block, chunk) tile of an operand = 6 k4-groups x 16 row-groups x 32 doubles = 24 KiB, contiguous:
+//   one (row block, chunk) tile of an operand = 6 k4-groups x 16 row-groups x 32 doubles = 24 KiB, contiguous
+//   (ngsd_ctx::k4 / tile_doubles: 4 k4-groups = 16 KiB in pdel two-plane mode, below):
 //       k4-group  kg = g*2 + h     genotype plane g in 0..2, half h in 0..1 (sites chunk*8 + h*4 .. +3)
 //       row-group r8               8 consecutive individuals
 //       32 doubles in DMMA.8x8x4 fragment order: lane = (ind&7)*4 + (site&3)
@@ -33,14 +34,28 @@
 //   A planes = (p_0, p_1), B planes = (B_0 - B_2, B_1 - B_2), chunk = 12 sites (k4-group = g*3 + h, h = 0..2: the tile
 //   stays 6 k4-groups = 24 KiB), plus the plane C[ind][site] = B_2 whose (weighted) row sums c_j are added in the epilogue.
 //   One third fewer DMMAs and 8 bytes less per individual-site; exact for one-hot posteriors, ~1e-16 absolute otherwise.
+//
+// Pdel two-plane mode (ngsd_ctx::pdel2; indep_geno && pairwise_del, FP64 path, well-conditioned score).  With Z the
+// zero-sum directions [[1,0],[0,1],[-1,-1]], V = Z^T S Z and the shifts l, r (api.cu pdel2_coefficients), a present
+// triple p (sum one) and a missing one (zero) satisfy  p_i^T S p_j = q_i^T V q_j + kappa * m_i m_j  exactly, so
+//   A planes = m (p_0 + l_0, p_1 + l_1), B planes = m V (p_0 + r_0, p_1 + r_1)        (m = presence bit)
+// and the epilogue adds kappa * cnt(i, j) (the exact shared-site count of --pairwise_del).  Chunks stay 8 sites with
+// k4-group kg = g*2 + h, g = 0..1: the three-plane layout without its third plane, 4 k4-groups = 16 KiB per tile.
+// One third fewer DMMAs and 16 bytes less per individual-site; exact for one-hot posteriors and dyadic coefficients
+// (default score), ~1e-16 absolute per site otherwise.
 // ---------------------------------------------------------------------------------------------
 constexpr int NGSD_TILE = 128;                 // individuals per row block / CTA tile edge
-constexpr int NGSD_SC = 8;                     // sites per chunk (= one pipeline stage), 3-plane mode
+constexpr int NGSD_SC = 8;                     // sites per chunk (= one pipeline stage), 3-plane and pdel two-plane modes
 constexpr int NGSD_SC2 = 12;                   // sites per chunk, 2-plane mode
 constexpr int NGSD_SC_MAX = 12;
-constexpr int NGSD_K4_PER_CHUNK = 6;           // 3 planes x 2 halves
-constexpr int NGSD_TILE_DOUBLES = NGSD_K4_PER_CHUNK * 16 * 32;   // 3072 doubles = 24 KiB
-constexpr int NGSD_TILE_BYTES = NGSD_TILE_DOUBLES * 8;
+constexpr int NGSD_K4_DOUBLES = 16 * 32;       // one k4-group of a tile: 16 row-groups x 32 doubles = 4 KiB
+constexpr int NGSD_K4_3 = 6;                   // k4-groups per chunk: 3 planes x 2 halves (also 2 planes x 3 thirds, planes == 2)
+constexpr int NGSD_K4_PD2 = 4;                 // k4-groups per chunk in pdel two-plane mode: 2 planes x 2 halves
+// Pdel two-plane mode is taken for matrices of at least 2^30 pair-sites (n_ind (n_ind - 1) / 2 * n_sites).  Below that a
+// three-plane contraction takes under 0.2 ms on a B200 and launch, count pass and epilogue set the matrix time, so the
+// exact three-plane form is kept: per-site products without the shifted cancellation of the two-plane form, exact
+// ngsd_get_posteriors, and the same sums as the three-plane contraction for every small data set.
+constexpr uint64_t NGSD_PDEL2_MIN_PAIR_SITES = 1ull << 30;
 constexpr int NGSD_TILE_ELEMS = NGSD_TILE * NGSD_TILE;           // accumulator elements per tile
 
 struct ngsd_tile { uint16_t ti, tj; };
@@ -75,10 +90,15 @@ struct ngsd_ctx {
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   uint64_t n_ind = 0, n_pad = 0, RB = 0, n_sites = 0, NC = 0, NW = 0;
   int planes = 3, sc = NGSD_SC;                // operand planes per site (3, or 2 with the sum-to-one reduction) / sites per chunk
+  // pdel two-plane mode (see above): planes stays 3 (8-site chunks, no C plane), k4 = 4
+  bool pdel2 = false;
+  double pd_l[2] = {0, 0}, pd_r[2] = {0, 0}, pd_V[4] = {0, 0, 0, 0}, pd_kappa = 0;   // V row-major
+  int k4 = NGSD_K4_3;                          // k4-groups per chunk
+  uint64_t tile_doubles = NGSD_K4_3 * NGSD_K4_DOUBLES;   // doubles per (row block, chunk) tile of Apack / Bpack
   double *Cplane = nullptr;                    // [NW][n_pad][64] B_2 plane (2-plane mode); ldc = n_pad
   uint64_t ldc = 0;
   double *d_cvec = nullptr;                    // [n_pad] weighted row sums of Cplane for the current matrix
-  double *Apack = nullptr, *Bpack = nullptr;   // [RB][NC][3072]
+  double *Apack = nullptr, *Bpack = nullptr;   // [RB][NC][tile_doubles]
   uint64_t *mask = nullptr;                    // [RB][NW][128] presence bits (1 = data present)
   // called-genotype integer path (dist_umma.cu): 2-bit codes instead of FP64 planes
   bool int_path = false;
